@@ -24,6 +24,8 @@ kernels or NCCL all-gather + reduce kernel): total work is fixed, so scaling = "
 
 `--impl reference` times only that CPU path (rank 0), same metric and the same `config` object (job_config); what an
 arm did on that config (search path, exchange, pipelining, rescans) is printed beside it under `run`.
+`--dump-outputs DIR` writes the ids and scores of the last timed search of each batch size as .npy files.  Every input is
+generated from a fixed seed, so the same arguments give the same files and two builds can be compared output for output.
 Clocks and throttle reasons are sampled through NVML during the timed regions; a region that saw hw_slowdown,
 hw_thermal_slowdown or sw_thermal_slowdown is rejected and measured once more (`clocks.remeasured_after`); sw_power_cap
 is kept and reported.
@@ -42,6 +44,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark may run from a read-only tree: no __pycache__ next to the sources
 
 METRIC = "exact top-k queries/sec at 10Mx768"
 SEED_CORPUS, SEED_QUERY = 1234, 1235
@@ -66,7 +69,34 @@ def parse_args():
                     help="rows of the CPU baseline sample (0 = the whole corpus when MemAvailable >= 1.3 x rows*dim*4, else 2M rows, extrapolated)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extra-regimes", action="store_true", help="skip the clustered-corpus and ingest legs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the ids (as float64) and scores (float32) of the last timed search of "
+                         "each batch size as DIR/<name>.npy, at most 64 MB in all (a fixed sample of queries beyond that)")
+    a = ap.parse_args()
+    if a.steps < 1 or a.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return a
+
+
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(d, results):
+    """results: (name, ids [nq, k] int64, scores [nq, k] fp32) per timed batch size.  ids are written as float64 (exact)
+    so that every file is floating point; queries beyond the byte budget are sampled with a fixed seed, and the sampled
+    query positions are written as <name>_queries.npy."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    per = DUMP_BYTES // max(1, len(results)) - 3 * 1024          # 3 files, npy headers included
+    for name, ids, scores in results:
+        nq, k = ids.shape
+        keep = max(1, per // (12 * k + 8))                          # float64 id + float32 score per hit, float64 query position
+        if nq > keep:
+            rows = np.sort(np.random.default_rng(0).choice(nq, keep, replace=False))
+            ids, scores = ids[rows], scores[rows]
+            np.save(os.path.join(d, f"{name}_queries.npy"), rows.astype(np.float64))
+        np.save(os.path.join(d, f"{name}_ids.npy"), ids.astype(np.float64))
+        np.save(os.path.join(d, f"{name}_scores.npy"), scores.astype(np.float32))
 
 
 def workload_name(a):
@@ -217,7 +247,7 @@ def cpu_corpus(a, rows):
     return out
 
 
-def cpu_baseline(a, budget_s: float, steps: int | None = None):
+def cpu_baseline(a, budget_s: float, steps: int | None = None, warmup: int = 1):
     import numpy as np
     import torch
     from oracle import c_oracle, fast_cpu
@@ -235,11 +265,12 @@ def cpu_baseline(a, budget_s: float, steps: int | None = None):
     stored = cpu_corpus(a, rows)
     t_gen = time.perf_counter() - t_gen
     q = c_oracle.synth_rows(SEED_QUERY, 0, nq * 4, a.dim)
-    fast_cpu.fast_topk(stored, q[:nq], a.k)          # warm-up
+    for i in range(warmup):
+        fast_cpu.fast_topk(stored, q[(i % 4) * nq:(i % 4 + 1) * nq], a.k)
     times, t_end, i = [], time.perf_counter() + budget_s, 0
     while (steps is None and time.perf_counter() < t_end) or (steps is not None and i < steps):
         t0 = time.perf_counter()
-        fast_cpu.fast_topk(stored, q[(i % 4) * nq:(i % 4 + 1) * nq], a.k)
+        last = fast_cpu.fast_topk(stored, q[(i % 4) * nq:(i % 4 + 1) * nq], a.k)
         times.append(time.perf_counter() - t0)
         i += 1
         if steps is None and i >= 400:
@@ -252,7 +283,7 @@ def cpu_baseline(a, budget_s: float, steps: int | None = None):
               f", {len(times)} calls, median")
     return {"value": qps, "unit": "queries/s", "cores": torch.get_num_threads(), "kind": "port", "sample": sample,
             "extrapolated": extrapolated, "rows_timed": rows, "corpus_build_s": round(t_gen, 1),
-            "ms_per_call_on_sample": per_call * 1e3}, len(times), per_call
+            "ms_per_call_on_sample": per_call * 1e3}, last
 
 
 def job_config(a, world):
@@ -266,8 +297,10 @@ def run_reference(a):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    # every step is one search of the batch over the corpus; at most 60 calls are timed so that the run ends within minutes
-    base, n, per_call = cpu_baseline(a, budget_s=0.0, steps=min(a.steps + a.warmup, 60))
+    # every step is one search of the batch (at most 64 of its queries) over the corpus
+    base, (ids, scores) = cpu_baseline(a, budget_s=0.0, steps=a.steps, warmup=a.warmup)
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, [(f"batch_{a.batch}", ids, scores)])
     line = {
         "impl": "reference", "metric": METRIC, "value": base["value"], "unit": "queries/s", "n_gpus": a.gpus,
         "steps": a.steps, "warmup": a.warmup, "ms_per_step": a.batch / base["value"] * 1e3,
@@ -370,10 +403,11 @@ def run_ours(a):
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         ev0.record()
         for i in range(steps):
-            searcher.search(q_dev[i % nbatches], a.k)
+            last = searcher.search(q_dev[i % nbatches], a.k)
         ev1.record()
         barrier()
         ms = torch.tensor([ev0.elapsed_time(ev1)], dtype=torch.float64, device=dev)
+        last = (last[0].cpu().numpy(), last[1].cpu().numpy()) if a.dump_outputs else None
         # roofline: the same K steps once more with the library's event pair around every launch of the dominant kernel
         # (serialised by those events: per-launch durations, not throughput)
         idx.profile(True)
@@ -434,7 +468,7 @@ def run_ours(a):
             "e2e": {"value": batch * steps / (e2e_ms * 1e-3), "unit": "queries/s", "ms_per_step": e2e_ms / steps,
                     "h2d_bytes_per_step": batch * a.dim * 4, "d2h_bytes_per_step": batch * a.k * 12},
             "gpu_launches": launches_per_step * steps, "roofline": roof,
-            "queries_rescanned_last_step": st["queries_rescanned"],
+            "queries_rescanned_last_step": st["queries_rescanned"], "last_step_outputs": last,
             "search_path": {0: "scan + finalize", 1: "tensor-core sweep, multi-kernel", 2: "large k", 3: "one kernel (sweep_fused)"}.get(st["path"]),
             "exchange": None if world == 1 else ("in-kernel peer stores (ragfin_search_sharded)" if fused_sharded else
                                                  "peer-memory push / merge kernels" if searcher.exchange is not None else "nccl all-gather + reduce kernel"),
@@ -555,7 +589,8 @@ def run_ours(a):
         n_dev, n_host = 2_000_000, 500_000
         per_row = 4 * a.dim + esize * ld
         out = {"bytes_per_row": per_row, "kernel": "ingest_vec_kernel" if a.dim % 4 == 0 and ld <= 1024 else "ingest_kernel"}
-        src = torch.randn((n_dev, a.dim), dtype=torch.float32, device=dev)
+        src = torch.randn((n_dev, a.dim), dtype=torch.float32, device=dev,
+                          generator=torch.Generator(device=dev).manual_seed(SEED_CORPUS + 1))
         tmp = ragfin_b200.Index(a.dim, a.dtype, capacity=3 * n_dev, device=local)
         tmp.add(src)                                    # warm-up (first launch, clocks)
         tmp.profile(True)
@@ -572,7 +607,7 @@ def run_ours(a):
                          "wall_ms_through_the_api": wall * 1e3}
         tmp.close()
         del src
-        hsrc = torch.randn((n_host, a.dim), dtype=torch.float32).pin_memory()
+        hsrc = torch.randn((n_host, a.dim), dtype=torch.float32, generator=torch.Generator().manual_seed(SEED_CORPUS + 2)).pin_memory()
         tmp = ragfin_b200.Index(a.dim, a.dtype, capacity=2 * n_host, device=local)
         tmp.add(hsrc.numpy())
         torch.cuda.synchronize()
@@ -667,10 +702,17 @@ def run_ours(a):
 
     main = measure_checked(a.batch, a.steps, a.warmup)
     main["parity_check"] = parity_check(a.batch)
+    last = main.pop("last_step_outputs")
+    outputs = [(f"batch_{a.batch}",) + last] if last else []
     other = None
     if a.also_batch and a.also_batch != a.batch:
         other = measure_checked(a.also_batch, max(5, a.steps // 10), a.warmup)
         other["parity_check"] = parity_check(a.also_batch)
+        last = other.pop("last_step_outputs")
+        if last:
+            outputs.append((f"batch_{a.also_batch}",) + last)
+    if a.dump_outputs and rank == 0:   # every rank holds the same merged result
+        dump_outputs(a.dump_outputs, outputs)
     def side_leg(fn, *args):
         """The side regimes must not cost the headline line: on one GPU a failure is reported in place of the leg's figures
         (with several ranks it propagates - a rank that skipped a leg would leave the others waiting in its collectives)."""

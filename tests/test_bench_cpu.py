@@ -47,6 +47,51 @@ def test_reference_arm_line_and_shared_config():
     assert set(d["config"]) == {"workload", "rows", "dim", "k", "batch", "parallelism", "l2"}
 
 
+def test_reference_arm_times_steps_calls_and_dumps_the_last(tmp_path):
+    """--steps 2 --warmup 1 times exactly two calls; --dump-outputs writes what the last of them returned."""
+    import numpy as np
+    from oracle import c_oracle
+    r = _run(["--impl", "reference", "--dump-outputs", str(tmp_path)])
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads([ln for ln in r.stdout.splitlines() if ln.startswith("{")][-1])
+    assert ", 2 calls, median" in d["cpu_baseline"]["sample"]
+    ids, sc = np.load(tmp_path / "batch_1_ids.npy"), np.load(tmp_path / "batch_1_scores.npy")
+    assert ids.dtype == np.float64 and sc.dtype == np.float32 and ids.shape == sc.shape == (1, 7)
+    bench = _bench_module()
+    x = c_oracle.normalize_rows(c_oracle.synth_rows(bench.SEED_CORPUS, 0, 30000, 96), "f32")
+    q = c_oracle.synth_rows(bench.SEED_QUERY, 0, 4, 96)[1:2]        # step 1 of 0..1 searches query batch 1
+    want_ids, want_sc = c_oracle.cosine_topk(q, x, 7)
+    assert np.array_equal(ids, want_ids.astype(np.float64))
+    assert np.allclose(sc, want_sc, rtol=1e-5, atol=1e-7)
+
+
+def test_dump_outputs_samples_queries_within_the_budget(tmp_path):
+    import numpy as np
+    bench = _bench_module()
+    rng = np.random.default_rng(3)
+    big_ids = rng.integers(0, 10_000_000, size=(40_000, 200), dtype=np.int64)       # 96 MB as written
+    big_sc = rng.random((40_000, 200), dtype=np.float32)
+    small_ids, small_sc = big_ids[:4, :10].copy(), big_sc[:4, :10].copy()
+    bench.dump_outputs(str(tmp_path), [("batch_4", small_ids, small_sc), ("batch_40000", big_ids, big_sc)])
+    assert sum(p.stat().st_size for p in tmp_path.iterdir()) <= 64_000_000
+    assert not (tmp_path / "batch_4_queries.npy").exists()
+    assert np.array_equal(np.load(tmp_path / "batch_4_ids.npy"), small_ids.astype(np.float64))
+    assert np.array_equal(np.load(tmp_path / "batch_4_scores.npy"), small_sc)
+    rows = np.load(tmp_path / "batch_40000_queries.npy")
+    assert rows.dtype == np.float64 and 0 < len(rows) < 40_000 and (np.diff(rows) > 0).all()
+    rows = rows.astype(np.int64)
+    assert np.array_equal(np.load(tmp_path / "batch_40000_ids.npy"), big_ids[rows].astype(np.float64))
+    assert np.array_equal(np.load(tmp_path / "batch_40000_scores.npy"), big_sc[rows])
+    again = tmp_path / "again"
+    bench.dump_outputs(str(again), [("batch_4", small_ids, small_sc), ("batch_40000", big_ids, big_sc)])
+    assert np.array_equal(np.load(again / "batch_40000_queries.npy"), rows.astype(np.float64))   # the same sample every run
+
+
+def test_steps_below_one_is_refused():
+    r = _run(["--impl", "reference", "--steps", "0"])
+    assert r.returncode != 0 and "--steps" in r.stderr
+
+
 def test_reference_arm_runs_on_rank_0_only():
     r = _run(["--impl", "reference", "--gpus", "2"], env={"RANK": "1", "LOCAL_RANK": "1", "WORLD_SIZE": "2"})
     assert r.returncode == 0 and r.stdout.strip() == ""

@@ -64,11 +64,3 @@ def test_directory_loader_matches_the_bundle(bundle, tmp_path):
             with open(tmp_path / quarter / name, "w") as f:
                 json.dump(doc, f)
     assert chunker.build_corpus(str(tmp_path)) == chunker.build_corpus_from_bundle(bundle)
-
-
-@pytest.mark.skipif(not os.path.isdir("/root/reference/extract_data"), reason="reference tree not mounted")
-def test_fixtures_are_the_reference_files():
-    built = chunker.build_corpus("/root/reference/extract_data")
-    with open("/root/reference/FinRag_knowledge_graph/chunks.json") as f:
-        ref = {c["id"]: c["text"] for c in json.load(f)}
-    assert {c["id"]: c["text"] for c in built} == ref

@@ -219,7 +219,9 @@ def _worker_fused_agreement(rank, world, port, out):
         dist.destroy_process_group()
 
 
-def test_one_kernel_path_is_taken_only_when_every_rank_can():
+def test_one_kernel_path_is_taken_only_when_every_rank_can(monkeypatch):
+    # the stand-ins are host code: a rank that saw a GPU would stage its queries there (search_host, fused_ok)
+    monkeypatch.setenv("CUDA_VISIBLE_DEVICES", "")
     world = 2
     ctx = mp.get_context("spawn")
     out = ctx.Manager().dict()
