@@ -35,7 +35,8 @@ extern "C" {
 
 typedef struct ragfin ragfin_t;
 
-enum { RAGFIN_F32 = 0, RAGFIN_BF16 = 1, RAGFIN_F16 = 2 };
+/* RAGFIN_F32_F16: fp32 rows plus an fp16 copy of them (see ragfin_create). */
+enum { RAGFIN_F32 = 0, RAGFIN_BF16 = 1, RAGFIN_F16 = 2, RAGFIN_F32_F16 = 3 };
 
 enum {
     RAGFIN_OK = 0,
@@ -46,12 +47,17 @@ enum {
 };
 
 /* ABI version of this header; bumped on any signature change. */
-#define RAGFIN_ABI_VERSION 3
+#define RAGFIN_ABI_VERSION 4
 int ragfin_abi_version(void);
 
 /* Create an empty collection of `dim`-wide embeddings stored as `dtype` on CUDA device
  * `device`, with room for `capacity_rows` rows (HBM is reserved up front: one contiguous
  * row-major [capacity, ld] matrix, ld = dim rounded up to 8).
+ * dtype RAGFIN_F32_F16 holds two matrices: the fp32 rows exactly as RAGFIN_F32 stores them, and an fp16 copy
+ * [capacity, ld] (each element RNE-rounded from the stored fp32 value: bit for bit what RAGFIN_F16 stores for the same
+ * input).  The tensor-core sweeps stream the copy (16-bit bytes, kind::f16); every exact step - rescore, exact tiers,
+ * small-batch scan - reads the fp32 rows, so results are bit-identical to a RAGFIN_F32 collection.  Cost: 6 bytes per
+ * element (46.1 GB at 10M x 768, against 30.7 GB for fp32), which is why it is opt-in.
  * Replaces: Collection(name, CollectionSchema([... FieldSchema("embedding", FLOAT_VECTOR,
  * dim=384) ...])) + create_index(COSINE)  - "chunking_storing (1).py":14-29. */
 int ragfin_create(ragfin_t** out, int32_t dim, int32_t dtype, int64_t capacity_rows, int32_t device);
@@ -166,8 +172,11 @@ int ragfin_search_sharded_host(ragfin_t* h, ragfin_exchange_t* x, const float* q
 void ragfin_exchange_destroy(ragfin_exchange_t* x);
 
 /* Copy rows row0..row0+n of the STORED matrix, raw storage bytes [n, ld], to host memory
- * (test hook for ingest parity).  *ld_out receives the row stride in elements. */
+ * (test hook for ingest parity).  *ld_out receives the row stride in elements.  RAGFIN_F32_F16: the fp32 rows. */
 int ragfin_read_rows(ragfin_t* h, int64_t row0, int64_t n, void* out_host, int32_t* ld_out);
+/* Same for the rows the tensor-core sweeps read: the fp16 copy on a RAGFIN_F32_F16 handle ([n, ld] fp16), the stored
+ * rows otherwise (test hook). */
+int ragfin_read_sweep_rows(ragfin_t* h, int64_t row0, int64_t n, void* out_host, int32_t* ld_out);
 
 /* Counters of the most recent search on this handle: kernel launches issued, queries that
  * took the exact-rescan tier (certificate failed), which scoring path ran
@@ -190,7 +199,8 @@ int ragfin_profile_read(ragfin_t* h, double* total_ms, int32_t* launches);
 /* Persistence of the device-resident matrix (stands in for Milvus' flush()/load() durability,
  * "chunking_storing (1).py":395-396, retrieve.py:18-19).  File = 64-byte header {magic "RAGFINB2", version,
  * dim, ld, dtype, count, id_base} + the stored rows [count, ld] exactly as they sit in HBM, so a
- * reloaded collection returns bit-identical results without re-normalising.
+ * reloaded collection returns bit-identical results without re-normalising.  A RAGFIN_F32_F16 file has header dtype 3 and
+ * holds the fp32 rows only; ragfin_load rebuilds the fp16 copy from them on the device (same bits as at ingest).
  * ragfin_load creates a new handle on `device` with room for max(capacity_rows, count) rows. */
 int ragfin_save(ragfin_t* h, const char* path);
 int ragfin_load(ragfin_t** out, const char* path, int64_t capacity_rows, int32_t device);

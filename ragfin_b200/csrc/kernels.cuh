@@ -23,13 +23,17 @@ constexpr int kFinWarps = kFinThreads / kWarp;
 // SYNTH with topic_rows > 0: "templated corpus" generator - row r belongs to topic r / topic_rows and is
 //   centre(topic) + noise(r) * noise_scale     (noise_scale a power of two <= 1/2: the sum is exact in fp32),
 // i.e. contiguous runs of topic_rows near-duplicates (cosine ~0.98 to each other at scale 1/8), inserted in topic order.
+// DT = 3 (RAGFIN_F32_F16): the fp32 row exactly as DT = 0 stores it, and RNE_f16 of each stored value into dst16 - the
+// same bits DT = 2 stores for the same input, since both round the same fp32 y.
+template <int DT> using IngestT = typename Store<DT == 3 ? 0 : DT>::T;
 template <int DT, bool SYNTH>
 __global__ void __launch_bounds__(256) ingest_kernel(const float* __restrict__ src, uint64_t synth_key,
                                                      int64_t synth_row0, int dup_every, int zero_every,
                                                      int64_t n, int dim, int ld,
-                                                     typename Store<DT>::T* __restrict__ dst,
-                                                     int64_t topic_rows = 0, uint64_t topic_key = 0, float noise_scale = 0.f) {
-    typedef typename Store<DT>::T T;
+                                                     IngestT<DT>* __restrict__ dst,
+                                                     int64_t topic_rows = 0, uint64_t topic_key = 0, float noise_scale = 0.f,
+                                                     __half* __restrict__ dst16 = nullptr) {
+    typedef IngestT<DT> T;
     const int lane = threadIdx.x & 31;
     const int64_t gw = (int64_t)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     const int64_t nw = (int64_t)gridDim.x * (blockDim.x >> 5);
@@ -65,10 +69,11 @@ __global__ void __launch_bounds__(256) ingest_kernel(const float* __restrict__ s
         for (int i = lane * 2; i < ld; i += 2 * kWarp) {
             const float y0 = i < dim ? (float)((double)elem(i) * inv) : 0.0f;
             const float y1 = i + 1 < dim ? (float)((double)elem(i + 1) * inv) : 0.0f;
-            if (DT == 0) {
+            if (DT == 0 || DT == 3) {
                 *reinterpret_cast<float2*>(out + i) = make_float2(y0, y1);
+                if (DT == 3) *reinterpret_cast<__half2*>(dst16 + r * (int64_t)ld + i) = __halves2half2(__float2half_rn(y0), __float2half_rn(y1));
             } else {
-                T pr[2] = {Store<DT>::from_f32(y0), Store<DT>::from_f32(y1)};
+                T pr[2] = {Store<DT == 3 ? 0 : DT>::from_f32(y0), Store<DT == 3 ? 0 : DT>::from_f32(y1)};
                 *reinterpret_cast<uint32_t*>(out + i) = *reinterpret_cast<uint32_t*>(pr);
             }
         }
@@ -82,15 +87,15 @@ __global__ void __launch_bounds__(256) ingest_kernel(const float* __restrict__ s
 // is not the vector layout, so the warp transposes the row through its 128 NV * 16 bytes of shared memory (STS.128
 // in, conflict-free LDS.32 out); every lane then scales the elements it holds in registers and stores them with one
 // 64-bit (16-bit storage) or 128-bit (fp32 storage) store per vector.  Same bits as ingest_kernel.
-// Algorithmic HBM bytes per row: 4 * dim read + ld * sizeof(T) written.
+// Algorithmic HBM bytes per row: 4 * dim read + ld * sizeof(T) written (+ ld * 2 for the fp16 copy of DT = 3).
 // ---------------------------------------------------------------------------------
 constexpr int kIngestThreads = 256;
 constexpr int kIngestWarps = kIngestThreads / kWarp;
 
 template <int DT, int NV>
 __global__ void __launch_bounds__(kIngestThreads) ingest_vec_kernel(const float* __restrict__ src, int64_t n, int dim, int ld,
-                                                                      typename Store<DT>::T* __restrict__ dst) {
-    typedef typename Store<DT>::T T;
+                                                                      IngestT<DT>* __restrict__ dst, __half* __restrict__ dst16 = nullptr) {
+    typedef IngestT<DT> T;
     __shared__ __align__(16) float stage[kIngestWarps][NV * 128];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int64_t gw = (int64_t)blockIdx.x * kIngestWarps + warp;
@@ -125,14 +130,34 @@ __global__ void __launch_bounds__(kIngestThreads) ingest_vec_kernel(const float*
             if (vi < nvec_out) {                    // vectors in [nvec, nvec_out) are the zero padding of the stored row
                 const float y0 = (float)((double)v[j].x * inv), y1 = (float)((double)v[j].y * inv);
                 const float y2 = (float)((double)v[j].z * inv), y3 = (float)((double)v[j].w * inv);
-                if (DT == 0) {
+                if (DT == 0 || DT == 3) {
                     __stcs(reinterpret_cast<float4*>(out) + vi, make_float4(y0, y1, y2, y3));
+                    if (DT == 3) {
+                        const __half2 h01 = __halves2half2(__float2half_rn(y0), __float2half_rn(y1));
+                        const __half2 h23 = __halves2half2(__float2half_rn(y2), __float2half_rn(y3));
+                        __stcs(reinterpret_cast<uint2*>(dst16 + r * (int64_t)ld) + vi,
+                               make_uint2(*reinterpret_cast<const uint32_t*>(&h01), *reinterpret_cast<const uint32_t*>(&h23)));
+                    }
                 } else {
-                    T pr[4] = {Store<DT>::from_f32(y0), Store<DT>::from_f32(y1), Store<DT>::from_f32(y2), Store<DT>::from_f32(y3)};
+                    typedef Store<DT == 3 ? 0 : DT> S;
+                    T pr[4] = {S::from_f32(y0), S::from_f32(y1), S::from_f32(y2), S::from_f32(y3)};
                     __stcs(reinterpret_cast<uint2*>(out) + vi, *reinterpret_cast<uint2*>(pr));
                 }
             }
         }
+    }
+}
+
+// ---------------------------------------------------------------------------------
+// fp16 copy of stored fp32 rows (ragfin_load of a RAGFIN_F32_F16 file): dst[i] = RNE_f16(src[i]), 4 elements per thread
+// and step (128-bit loads, 64-bit stores) - the same bits the DT = 3 ingest stores.
+// ---------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256) cast_f16_kernel(const float4* __restrict__ src, uint2* __restrict__ dst, int64_t n4) {
+    for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n4; i += (int64_t)gridDim.x * blockDim.x) {
+        const float4 v = __ldcs(src + i);
+        const __half2 h01 = __halves2half2(__float2half_rn(v.x), __float2half_rn(v.y));
+        const __half2 h23 = __halves2half2(__float2half_rn(v.z), __float2half_rn(v.w));
+        __stcs(dst + i, make_uint2(*reinterpret_cast<const uint32_t*>(&h01), *reinterpret_cast<const uint32_t*>(&h23)));
     }
 }
 

@@ -60,7 +60,13 @@ struct ragfin {
     int dim = 0, ld = 0, dtype = 0, device = 0, num_sms = 0;
     int64_t capacity = 0, count = 0, id_base = 0;
     void* data = nullptr;  // [capacity, ld] storage, row-major, L2-normalised
-    bool is_view = false;  // ragfin_create_view: `data` belongs to another handle (read-only here, never freed here)
+    // The rows the tensor-core sweeps read: {data, dtype} on dtypes 0-2; on RAGFIN_F32_F16 (dtype = RAGFIN_F32 here, so every
+    // exact step keeps meaning "the fp32 rows") an fp16 copy [capacity, ld] of them, and eps_sweep bounds what reading the copy
+    // instead of the rows changes in a score (see eps_sweep_const).  Only the approximate passes read these three.
+    void* sweep_data = nullptr;
+    int sweep_dt = 0;
+    float eps_sweep = 0.f;
+    bool is_view = false;  // ragfin_create_view: `data` and `sweep_data` belong to another handle (read-only here, never freed here)
     std::mutex mu;
     // workspace (grow-only)
     Buf qhat, q16, eps_q, gtau, bmax, acnt, athr, allow, bk_scores, bk_state, bk_keys, bk_rows, cand, cand_e, flags, stage_q, stage_ids, stage_scores, add_stage;
@@ -116,6 +122,17 @@ static void prof_end(ragfin* h, cudaStream_t st) {
 }
 
 static size_t esize(int dtype) { return dtype == RAGFIN_F32 ? 4 : 2; }
+static bool has_copy(const ragfin* h) { return h->sweep_data != h->data; }
+// dtype as the caller named it (ragfin_create, the file header)
+static int public_dtype(const ragfin* h) { return has_copy(h) ? RAGFIN_F32_F16 : h->dtype; }
+
+// |q.x - q.x16| for the fp32 row x (|x|_2 <= 1 + 2^-20), its copy x16 = RNE_f16(x) and a normalised query (|q|_2 <= 1 + 2^-22):
+// per element |x_i - x16_i| <= 2^-11 |x_i| (fp16 normal range, half an ulp) or <= 2^-25 (subnormal range, half the spacing
+// 2^-24), so |x - x16|_2 <= 2^-11 |x|_2 + 2^-25 sqrt(ld) and |q.x - q.x16| <= |q|_2 |x - x16|_2.  Rounded up.
+static float eps_sweep_const(int ld) {
+    const double e = (1.0 + 2.384185791015625e-07) * (4.8828125e-04 * (1.0 + 9.5367431640625e-07) + 2.98023223876953125e-08 * sqrt((double)ld));
+    return nextafterf((float)e, INFINITY);
+}
 
 static int ensure(Buf& b, size_t bytes) {
     if (b.bytes >= bytes) return 0;
@@ -165,7 +182,7 @@ extern "C" int ragfin_create(ragfin_t** out, int32_t dim, int32_t dtype, int64_t
     if (!out) return fail(RAGFIN_EINVAL, "out is NULL");
     *out = nullptr;
     if (dim < 1 || dim > 65536) return fail(RAGFIN_EINVAL, "dim %d out of range [1, 65536]", dim);
-    if (dtype < 0 || dtype > 2) return fail(RAGFIN_EINVAL, "dtype %d is not 0 (f32), 1 (bf16) or 2 (f16)", dtype);
+    if (dtype < 0 || dtype > 3) return fail(RAGFIN_EINVAL, "dtype %d is not 0 (f32), 1 (bf16), 2 (f16) or 3 (f32 + f16 copy)", dtype);
     if (capacity_rows < 1 || capacity_rows >= (int64_t)0xFFFFFFFF)
         return fail(RAGFIN_EINVAL, "capacity_rows %lld out of range [1, 2^32-1)", (long long)capacity_rows);
     int ndev = 0;
@@ -187,20 +204,35 @@ extern "C" int ragfin_create(ragfin_t** out, int32_t dim, int32_t dtype, int64_t
     if (!h) return fail(RAGFIN_ENOMEM, "host allocation failed");
     h->dim = dim;
     h->ld = (dim + 7) / 8 * 8;
-    h->dtype = dtype;
+    h->dtype = dtype == RAGFIN_F32_F16 ? RAGFIN_F32 : dtype;
     h->device = device;
     h->num_sms = prop.multiProcessorCount;
     read_env_knobs(h);
     h->capacity = capacity_rows;
-    const size_t bytes = (size_t)capacity_rows * h->ld * esize(dtype);
+    const size_t bytes = (size_t)capacity_rows * h->ld * esize(h->dtype);
     e = cudaMalloc(&h->data, bytes);
     if (e != cudaSuccess) {
         (void)cudaGetLastError();
         delete h;
         return fail(RAGFIN_ENOMEM, "cudaMalloc of %zu bytes for the corpus failed: %s", bytes, cudaGetErrorString(e));
     }
+    h->sweep_data = h->data;
+    h->sweep_dt = h->dtype;
+    if (dtype == RAGFIN_F32_F16) {
+        const size_t bytes16 = (size_t)capacity_rows * h->ld * 2;
+        e = cudaMalloc(&h->sweep_data, bytes16);
+        if (e != cudaSuccess) {
+            (void)cudaGetLastError();
+            cudaFree(h->data);
+            delete h;
+            return fail(RAGFIN_ENOMEM, "cudaMalloc of %zu bytes for the fp16 copy failed: %s", bytes16, cudaGetErrorString(e));
+        }
+        h->sweep_dt = RAGFIN_F16;
+        h->eps_sweep = eps_sweep_const(h->ld);
+    }
     e = cudaEventCreateWithFlags(&h->last_done, cudaEventDisableTiming);
     if (e != cudaSuccess) {
+        if (has_copy(h)) cudaFree(h->sweep_data);
         cudaFree(h->data);
         delete h;
         return fail(RAGFIN_ECUDA, "cudaEventCreate failed: %s", cudaGetErrorString(e));
@@ -224,6 +256,7 @@ extern "C" int ragfin_create_view(ragfin_t* parent, ragfin_t** out) {
     h->dim = parent->dim; h->ld = parent->ld; h->dtype = parent->dtype; h->device = parent->device; h->num_sms = parent->num_sms;
     h->capacity = parent->count > 0 ? parent->count : 1; h->count = parent->count; h->id_base = parent->id_base;
     h->data = parent->data;
+    h->sweep_data = parent->sweep_data; h->sweep_dt = parent->sweep_dt; h->eps_sweep = parent->eps_sweep;
     h->is_view = true;
     h->gemm_min_nq = parent->gemm_min_nq; h->gemm_min_nq_large = parent->gemm_min_nq_large; h->gemm_cluster = parent->gemm_cluster;
     h->scan_variant = parent->scan_variant; h->use_append = parent->use_append; h->use_bound_pass = parent->use_bound_pass;
@@ -248,6 +281,7 @@ extern "C" void ragfin_destroy(ragfin_t* h) {
     Buf* bufs[] = {&h->qhat, &h->q16, &h->eps_q, &h->gtau, &h->bmax, &h->acnt, &h->athr, &h->allow, &h->bk_scores, &h->bk_state, &h->bk_keys, &h->bk_rows, &h->cand, &h->cand_e, &h->flags, &h->stage_q, &h->stage_ids, &h->stage_scores, &h->add_stage, &h->fctl, &h->fcand, &h->fqn, &h->fflags};
     for (Buf* b : bufs)
         if (b->p) cudaFree(b->p);
+    if (h->sweep_data && has_copy(h) && !h->is_view) cudaFree(h->sweep_data);
     if (h->data && !h->is_view) cudaFree(h->data);
     for (int b = 0; b < 2; ++b) {
         if (h->add_stage2[b].p) cudaFree(h->add_stage2[b].p);
@@ -287,12 +321,33 @@ extern "C" int ragfin_reserve(ragfin_t* h, int64_t capacity_rows) {
         (void)cudaGetLastError();
         return fail(RAGFIN_ENOMEM, "cudaMalloc of %zu bytes for the grown corpus failed: %s", (size_t)capacity_rows * rb, cudaGetErrorString(e));
     }
+    // the fp16 copy grows with the rows; both new buffers exist before either old one is touched, so a failed allocation
+    // leaves the handle as it was
+    const size_t rb16 = (size_t)h->ld * 2;
+    void* nd16 = nullptr;
+    if (has_copy(h)) {
+        e = cudaMalloc(&nd16, (size_t)capacity_rows * rb16);
+        if (e != cudaSuccess) {
+            (void)cudaGetLastError();
+            cudaFree(nd);
+            return fail(RAGFIN_ENOMEM, "cudaMalloc of %zu bytes for the grown fp16 copy failed: %s", (size_t)capacity_rows * rb16, cudaGetErrorString(e));
+        }
+    }
     if (h->count > 0) {
         e = cudaMemcpy(nd, h->data, (size_t)h->count * rb, cudaMemcpyDeviceToDevice);
-        if (e != cudaSuccess) { cudaFree(nd); (void)cudaGetLastError(); return fail(RAGFIN_ECUDA, "device copy failed: %s", cudaGetErrorString(e)); }
+        if (e == cudaSuccess && nd16) e = cudaMemcpyAsync(nd16, h->sweep_data, (size_t)h->count * rb16, cudaMemcpyDeviceToDevice, 0);
+        if (e == cudaSuccess && nd16) e = cudaStreamSynchronize(0);
+        if (e != cudaSuccess) {
+            cudaFree(nd);
+            if (nd16) cudaFree(nd16);
+            (void)cudaGetLastError();
+            return fail(RAGFIN_ECUDA, "device copy failed: %s", cudaGetErrorString(e));
+        }
     }
+    if (nd16) { CU_TRY(cudaFree(h->sweep_data)); h->sweep_data = nd16; }
     CU_TRY(cudaFree(h->data));
     h->data = nd;
+    if (!nd16) h->sweep_data = nd;
     h->capacity = capacity_rows;
     for (ragfin::MapSlot& m : h->map_cache) m = ragfin::MapSlot();   // tensor maps of the old matrix are stale
     return RAGFIN_OK;
@@ -309,10 +364,11 @@ extern "C" int ragfin_set_id_base(ragfin_t* h, int64_t id_base) {
 // ------------------------------------------------------------------------------
 // K1 launch
 // ------------------------------------------------------------------------------
+// dtype RAGFIN_F32_F16: fp32 rows into dst and their fp16 copy into dst16, one pass
 template <bool SYNTH>
 static int launch_ingest(int dtype, const float* src, uint64_t key, int64_t row0, int dup, int zero, int64_t n,
                          int dim, int ld, void* dst, int num_sms, cudaStream_t st,
-                         int64_t topic_rows = 0, uint64_t topic_key = 0, float noise_scale = 0.f) {
+                         int64_t topic_rows = 0, uint64_t topic_key = 0, float noise_scale = 0.f, void* dst16 = nullptr) {
     if (n == 0) return 0;
     const int threads = 256, wpb = threads / 32;
     int64_t blocks = (n + wpb - 1) / wpb;
@@ -328,7 +384,15 @@ static int launch_ingest(int dtype, const float* src, uint64_t key, int64_t row0
             case 6: ingest_vec_kernel<DT, 6><<<(int)blocks, kIngestThreads, 0, st>>>(src, n, dim, ld, (TT*)dst); break; \
             default: ingest_vec_kernel<DT, 8><<<(int)blocks, kIngestThreads, 0, st>>>(src, n, dim, ld, (TT*)dst); break; \
         }
-        if (dtype == 0) { RF_INGEST_VEC(0, float) } else if (dtype == 1) { RF_INGEST_VEC(1, __nv_bfloat16) } else { RF_INGEST_VEC(2, __half) }
+        if (dtype == 0) { RF_INGEST_VEC(0, float) } else if (dtype == 1) { RF_INGEST_VEC(1, __nv_bfloat16) } else if (dtype == 2) { RF_INGEST_VEC(2, __half) }
+        else {
+            switch (nv) {
+                case 2: ingest_vec_kernel<3, 2><<<(int)blocks, kIngestThreads, 0, st>>>(src, n, dim, ld, (float*)dst, (__half*)dst16); break;
+                case 4: ingest_vec_kernel<3, 4><<<(int)blocks, kIngestThreads, 0, st>>>(src, n, dim, ld, (float*)dst, (__half*)dst16); break;
+                case 6: ingest_vec_kernel<3, 6><<<(int)blocks, kIngestThreads, 0, st>>>(src, n, dim, ld, (float*)dst, (__half*)dst16); break;
+                default: ingest_vec_kernel<3, 8><<<(int)blocks, kIngestThreads, 0, st>>>(src, n, dim, ld, (float*)dst, (__half*)dst16); break;
+            }
+        }
 #undef RF_INGEST_VEC
         CU_TRY(cudaGetLastError());
         return 0;
@@ -338,7 +402,8 @@ static int launch_ingest(int dtype, const float* src, uint64_t key, int64_t row0
     switch (dtype) {
         case 0: ingest_kernel<0, SYNTH><<<(int)blocks, threads, 0, st>>>(src, key, row0, dup, zero, n, dim, ld, (float*)dst, topic_rows, topic_key, noise_scale); break;
         case 1: ingest_kernel<1, SYNTH><<<(int)blocks, threads, 0, st>>>(src, key, row0, dup, zero, n, dim, ld, (__nv_bfloat16*)dst, topic_rows, topic_key, noise_scale); break;
-        default: ingest_kernel<2, SYNTH><<<(int)blocks, threads, 0, st>>>(src, key, row0, dup, zero, n, dim, ld, (__half*)dst, topic_rows, topic_key, noise_scale); break;
+        case 2: ingest_kernel<2, SYNTH><<<(int)blocks, threads, 0, st>>>(src, key, row0, dup, zero, n, dim, ld, (__half*)dst, topic_rows, topic_key, noise_scale); break;
+        default: ingest_kernel<3, SYNTH><<<(int)blocks, threads, 0, st>>>(src, key, row0, dup, zero, n, dim, ld, (float*)dst, topic_rows, topic_key, noise_scale, (__half*)dst16); break;
     }
     CU_TRY(cudaGetLastError());
     return 0;
@@ -377,9 +442,10 @@ extern "C" int ragfin_add(ragfin_t* h, const float* rows, int64_t n, int32_t src
     int rc;
     if ((rc = wait_prev(h, st))) return rc;
     char* dst = (char*)h->data + (size_t)h->count * h->ld * esize(h->dtype);
+    char* dst16 = has_copy(h) ? (char*)h->sweep_data + (size_t)h->count * h->ld * 2 : nullptr;
     if (src_is_device) {
         prof_begin(h, st);
-        if ((rc = launch_ingest<false>(h->dtype, rows, 0, 0, 0, 0, n, h->dim, h->ld, dst, h->num_sms, st))) return rc;
+        if ((rc = launch_ingest<false>(public_dtype(h), rows, 0, 0, 0, 0, n, h->dim, h->ld, dst, h->num_sms, st, 0, 0, 0.f, dst16))) return rc;
         prof_end(h, st);
     } else {
         // Staged in slices through TWO device buffers so that a huge host matrix never needs a device copy of itself and
@@ -408,8 +474,9 @@ extern "C" int ragfin_add(ragfin_t* h, const float* rows, int64_t n, int32_t src
             CU_TRY(cudaEventRecord(h->stage_ready[b], h->copy_stream));
             CU_TRY(cudaStreamWaitEvent(st, h->stage_ready[b], 0));
             prof_begin(h, st);
-            if ((rc = launch_ingest<false>(h->dtype, (const float*)h->add_stage2[b].p, 0, 0, 0, 0, m, h->dim, h->ld,
-                                           dst + (size_t)r0 * h->ld * esize(h->dtype), h->num_sms, st)))
+            if ((rc = launch_ingest<false>(public_dtype(h), (const float*)h->add_stage2[b].p, 0, 0, 0, 0, m, h->dim, h->ld,
+                                           dst + (size_t)r0 * h->ld * esize(h->dtype), h->num_sms, st, 0, 0, 0.f,
+                                           dst16 ? dst16 + (size_t)r0 * h->ld * 2 : nullptr)))
                 return rc;
             prof_end(h, st);
             CU_TRY(cudaEventRecord(h->stage_free[b], st));
@@ -436,8 +503,9 @@ extern "C" int ragfin_add_synthetic(ragfin_t* h, uint64_t seed, int64_t row0, in
     int rc;
     if ((rc = wait_prev(h, st))) return rc;
     char* dst = (char*)h->data + (size_t)h->count * h->ld * esize(h->dtype);
-    if ((rc = launch_ingest<true>(h->dtype, nullptr, mix64(seed), row0, dup_every, zero_every, n, h->dim, h->ld, dst,
-                                  h->num_sms, st)))
+    char* dst16 = has_copy(h) ? (char*)h->sweep_data + (size_t)h->count * h->ld * 2 : nullptr;
+    if ((rc = launch_ingest<true>(public_dtype(h), nullptr, mix64(seed), row0, dup_every, zero_every, n, h->dim, h->ld, dst,
+                                  h->num_sms, st, 0, 0, 0.f, dst16)))
         return rc;
     h->count += n;
     return mark_done(h, st);
@@ -463,24 +531,36 @@ extern "C" int ragfin_add_synthetic_topics(ragfin_t* h, uint64_t seed, int64_t r
     int rc;
     if ((rc = wait_prev(h, st))) return rc;
     char* dst = (char*)h->data + (size_t)h->count * h->ld * esize(h->dtype);
-    if ((rc = launch_ingest<true>(h->dtype, nullptr, mix64(seed), row0, 0, 0, n, h->dim, h->ld, dst, h->num_sms, st, topic_rows,
-                                  mix64(seed + RAGFIN_TOPIC_SEED_OFFSET), ldexpf(1.0f, -noise_shift))))
+    char* dst16 = has_copy(h) ? (char*)h->sweep_data + (size_t)h->count * h->ld * 2 : nullptr;
+    if ((rc = launch_ingest<true>(public_dtype(h), nullptr, mix64(seed), row0, 0, 0, n, h->dim, h->ld, dst, h->num_sms, st, topic_rows,
+                                  mix64(seed + RAGFIN_TOPIC_SEED_OFFSET), ldexpf(1.0f, -noise_shift), dst16)))
         return rc;
     h->count += n;
     return mark_done(h, st);
 }
 
-extern "C" int ragfin_read_rows(ragfin_t* h, int64_t row0, int64_t n, void* out_host, int32_t* ld_out) {
+static int read_rows_of(ragfin* h, const void* base, int dtype, int64_t row0, int64_t n, void* out_host, int32_t* ld_out) {
     if (!h || !out_host) return fail(RAGFIN_EINVAL, "NULL argument");
-    std::lock_guard<std::mutex> lk(h->mu);
     if (row0 < 0 || n < 0 || row0 + n > h->count) return fail(RAGFIN_EINVAL, "rows [%lld, %lld) outside [0, %lld)",
                                                                (long long)row0, (long long)(row0 + n), (long long)h->count);
     DeviceGuard g(h->device);
     CU_TRY(cudaDeviceSynchronize());
-    const size_t rb = (size_t)h->ld * esize(h->dtype);
-    CU_TRY(cudaMemcpy(out_host, (char*)h->data + (size_t)row0 * rb, (size_t)n * rb, cudaMemcpyDeviceToHost));
+    const size_t rb = (size_t)h->ld * esize(dtype);
+    CU_TRY(cudaMemcpy(out_host, (const char*)base + (size_t)row0 * rb, (size_t)n * rb, cudaMemcpyDeviceToHost));
     if (ld_out) *ld_out = h->ld;
     return RAGFIN_OK;
+}
+
+extern "C" int ragfin_read_rows(ragfin_t* h, int64_t row0, int64_t n, void* out_host, int32_t* ld_out) {
+    if (!h) return fail(RAGFIN_EINVAL, "NULL argument");
+    std::lock_guard<std::mutex> lk(h->mu);
+    return read_rows_of(h, h->data, h->dtype, row0, n, out_host, ld_out);
+}
+
+extern "C" int ragfin_read_sweep_rows(ragfin_t* h, int64_t row0, int64_t n, void* out_host, int32_t* ld_out) {
+    if (!h) return fail(RAGFIN_EINVAL, "NULL argument");
+    std::lock_guard<std::mutex> lk(h->mu);
+    return read_rows_of(h, h->sweep_data, h->sweep_dt, row0, n, out_host, ld_out);
 }
 
 // ------------------------------------------------------------------------------
@@ -562,6 +642,19 @@ static float eps_fp32_accumulate(int ld) { return (float)((ld + 64) * 5.96046447
 
 static const size_t kHostStageQ = 64 << 10, kHostStageOut = 64 << 10;   // mapped staging of ragfin_search_host (small requests)
 static const size_t kHostStageFlag = 64;                                // ... + the completion word the one-kernel search sets
+
+// The mapped staging of the synchronous host calls.  Its completion word starts at 0 (host_seq counts from 1): pinned memory
+// freed by a destroyed handle can come back here still holding that handle's last sequence number, which would make the
+// first poll succeed before the kernel has written anything.
+static int alloc_hstage(ragfin* h) {
+    if (cudaHostAlloc(&h->hstage, kHostStageQ + kHostStageOut + kHostStageFlag, cudaHostAllocMapped) != cudaSuccess) {
+        (void)cudaGetLastError();
+        h->hstage = nullptr;
+        return fail(RAGFIN_ENOMEM, "pinned staging allocation failed");
+    }
+    memset((char*)h->hstage + kHostStageQ + kHostStageOut, 0, kHostStageFlag);
+    return 0;
+}
 static const int kMaxQueryBatch = 4096;  // queries per pass through the pipeline (bounds the workspace)
 
 // ------------------------------------------------------------------------------
@@ -691,6 +784,13 @@ static float eps_gemm_const(int dtype, int ld) {
     if (dtype == 0) e += 2.0 * 9.765625e-04 * 1.0625;                               // 2 * 2^-10
     return (float)e;
 }
+// |approximate score - exact score| beyond the query rounding term, for the rows the sweeps read: + eps_sweep when they are
+// the fp16 copy of fp32 rows (the exact score is the fp32 row's)
+static float eps_approx(const ragfin* h) {
+    const float e = eps_gemm_const(h->sweep_dt, h->ld);
+    if (h->eps_sweep == 0.f) return e;
+    return nextafterf((float)((double)e + (double)h->eps_sweep), INFINITY);
+}
 
 // TMA coordinates are signed 32-bit: shards of 2^31 rows or more stay on the scan path (int64 row arithmetic)
 static bool gemm_rows_ok(const ragfin* h) { return h->count > 0 && h->count < ((int64_t)1 << 31) - kGN; }
@@ -770,7 +870,7 @@ static int run_gemm(ragfin* h, int nb, int k, int kp, int* G, bool* appended, fl
     typedef void (*gemm_fn)(const CUtensorMap, const CUtensorMap, const GemmArgs);
 #define RF_PICK_MODE(KIND, CC) (mode == 0 ? gemm_topk_kernel<KIND, 0, CC> : mode == 1 ? gemm_topk_kernel<KIND, 1, CC> : mode == 2 ? gemm_topk_kernel<KIND, 2, CC> : gemm_topk_kernel<KIND, 3, CC>)
     auto pick = [&](int c, int mode) -> gemm_fn {
-        if (h->dtype == 0) return c == 4 ? RF_PICK_MODE(1, 4) : c == 2 ? RF_PICK_MODE(1, 2) : RF_PICK_MODE(1, 1);
+        if (h->sweep_dt == 0) return c == 4 ? RF_PICK_MODE(1, 4) : c == 2 ? RF_PICK_MODE(1, 2) : RF_PICK_MODE(1, 1);
         return c == 4 ? RF_PICK_MODE(0, 4) : c == 2 ? RF_PICK_MODE(0, 2) : RF_PICK_MODE(0, 1);
     };
 #undef RF_PICK_MODE
@@ -818,14 +918,14 @@ static int run_gemm(ragfin* h, int nb, int k, int kp, int* G, bool* appended, fl
     const float* qhat = (const float*)h->qhat.p;
     const void* a_base = qhat;
     if (prepped) {   // prep_queries_kernel already produced qhat, q16, eps_q and cleared gtau
-        if (h->dtype != 0) a_base = h->q16.p;
+        if (h->sweep_dt != 0) a_base = h->q16.p;
     } else if ((rc = ensure(h->eps_q, (size_t)nb * sizeof(float)))) {
         return rc;
-    } else if (h->dtype != 0) {
+    } else if (h->sweep_dt != 0) {
         if ((rc = ensure(h->q16, (size_t)nb_pad * h->ld * 2))) return rc;
         if (nb_pad > nb) CU_TRY(cudaMemsetAsync((char*)h->q16.p + (size_t)nb * h->ld * 2, 0, (size_t)(nb_pad - nb) * h->ld * 2, st));
         const int wpb = 8;
-        if (h->dtype == 1)
+        if (h->sweep_dt == 1)
             qconv_kernel<1><<<(nb + wpb - 1) / wpb, wpb * 32, 0, st>>>(qhat, nb, h->ld, (__nv_bfloat16*)h->q16.p, (float*)h->eps_q.p);
         else
             qconv_kernel<2><<<(nb + wpb - 1) / wpb, wpb * 32, 0, st>>>(qhat, nb, h->ld, (__half*)h->q16.p, (float*)h->eps_q.p);
@@ -836,8 +936,8 @@ static int run_gemm(ragfin* h, int nb, int k, int kp, int* G, bool* appended, fl
         CU_TRY(cudaMemsetAsync(h->eps_q.p, 0, (size_t)nb * sizeof(float), st));
     }
     CUtensorMap tmA, tmB;
-    if ((rc = cached_map(h, &tmA, h->dtype, a_base, nb_pad, h->ld, kGM))) return rc;
-    if ((rc = cached_map(h, &tmB, h->dtype, h->data, n, h->ld, kGN / C))) return rc;   // each CTA fetches 1/C of a tile
+    if ((rc = cached_map(h, &tmA, h->sweep_dt, a_base, nb_pad, h->ld, kGM))) return rc;
+    if ((rc = cached_map(h, &tmB, h->sweep_dt, h->sweep_data, n, h->ld, kGN / C))) return rc;   // each CTA fetches 1/C of a tile
     if (append) {
         if ((rc = ensure(h->cand, (size_t)nb * kAppendCap * sizeof(u64)))) return rc;
         if ((rc = ensure(h->acnt, (size_t)nb * sizeof(uint32_t)))) return rc;
@@ -846,8 +946,8 @@ static int run_gemm(ragfin* h, int nb, int k, int kp, int* G, bool* appended, fl
         if ((rc = ensure(h->cand, (size_t)nb * p.S * kp * sizeof(u64)))) return rc;
     }
     GemmArgs a;
-    a.idesc = make_idesc(h->dtype == 0 ? 2 : h->dtype == 1 ? 1 : 0);
-    a.k_elems = kGKBytes / (int)esize(h->dtype);
+    a.idesc = make_idesc(h->sweep_dt == 0 ? 2 : h->sweep_dt == 1 ? 1 : 0);
+    a.k_elems = kGKBytes / (int)esize(h->sweep_dt);
     a.num_kblocks = (h->ld + a.k_elems - 1) / a.k_elems;
     a.nq = nb;
     a.n_rows = n;
@@ -894,21 +994,21 @@ static int run_gemm(ragfin* h, int nb, int k, int kp, int* G, bool* appended, fl
         CU_TRY(cudaLaunchKernelEx(&cfg, bfn, tmA, tmB, b));
         RF_LAUNCH(bound_select_kernel, nb, 256, 0, st, (const float*)h->bmax.p, nblk, rank, append ? nullptr : (uint32_t*)h->gtau.p,
                                                  append ? (float*)h->athr.p : nullptr, append ? (uint32_t*)h->acnt.p : nullptr,
-                                                 eps_gemm_const(h->dtype, h->ld), (const float*)h->eps_q.p);
+                                                 eps_approx(h), (const float*)h->eps_q.p);
         CU_TRY(cudaGetLastError());
         h->stats.launches += 2;
     }
     if (append && (h->gemm_variant == 3 || h->gemm_variant == 0) && nb <= kRN && C == 1 && rows_stages(a.num_kblocks) >= 3) {
         // <= 16 queries, operand roles swapped (gemm_rows.cuh): corpus rows are the MMA's M, the queries its N = 16
         RowsArgs r;
-        r.idesc = make_idesc_n(h->dtype == 0 ? 2 : h->dtype == 1 ? 1 : 0, kRN);
+        r.idesc = make_idesc_n(h->sweep_dt == 0 ? 2 : h->sweep_dt == 1 ? 1 : 0, kRN);
         r.num_kblocks = a.num_kblocks; r.k_elems = a.k_elems; r.nq = nb; r.n_rows = n;
         r.S = p.S; r.rows_per_slice = p.rows_per_slice; r.stages = rows_stages(a.num_kblocks);
         r.cand = a.cand; r.thr = a.thr; r.cnt = a.cnt; r.cap = a.cap;
         CUtensorMap tmQ;
-        if ((rc = cached_map(h, &tmQ, h->dtype, a_base, nb_pad, h->ld, kRN))) return rc;
+        if ((rc = cached_map(h, &tmQ, h->sweep_dt, a_base, nb_pad, h->ld, kRN))) return rc;
         typedef void (*rows_fn)(const CUtensorMap, const CUtensorMap, const RowsArgs);
-        rows_fn rfn = h->dtype == 0 ? gemm_rows_kernel<1> : gemm_rows_kernel<0>;
+        rows_fn rfn = h->sweep_dt == 0 ? gemm_rows_kernel<1> : gemm_rows_kernel<0>;
         const size_t rsmem = rows_smem_bytes(r.num_kblocks, r.stages);
         if ((rc = set_dyn_smem(h->device, (const void*)rfn, rsmem))) return rc;
         prof_begin(h, st);
@@ -917,9 +1017,9 @@ static int run_gemm(ragfin* h, int nb, int k, int kp, int* G, bool* appended, fl
     } else if (want_pair && C == 2 && (append || dump)) {
         // gemm variant 4 (gemm_pair.cuh): one M = 256 MMA per cluster, each CTA holds half of the corpus tile
         GemmArgs pa = a;
-        pa.idesc = make_idesc_pair(h->dtype == 0 ? 2 : h->dtype == 1 ? 1 : 0);
+        pa.idesc = make_idesc_pair(h->sweep_dt == 0 ? 2 : h->sweep_dt == 1 ? 1 : 0);
         pa.stages = kPMaxStages;
-        gemm_fn pfn = h->dtype == 0 ? (dump ? gemm_pair_kernel<1, 1> : gemm_pair_kernel<1, 3>)
+        gemm_fn pfn = h->sweep_dt == 0 ? (dump ? gemm_pair_kernel<1, 1> : gemm_pair_kernel<1, 3>)
                                     : (dump ? gemm_pair_kernel<0, 1> : gemm_pair_kernel<0, 3>);
         const size_t psmem = pair_smem_bytes(pa.stages);
         if ((rc = set_dyn_smem(h->device, (const void*)pfn, psmem))) return rc;
@@ -1072,11 +1172,11 @@ struct FusedPlan {
 static FusedPlan plan_fused(const ragfin* h, int nb, int k) {
     FusedPlan best;
     if (nb < 1 || nb > (h->fused_max_nq < kFMaxQ ? h->fused_max_nq : kFMaxQ) || k > kFMaxK || (int64_t)nb * k > h->fused_max_nqk) return best;
-    const int es = (int)esize(h->dtype);
+    const int es = (int)esize(h->sweep_dt);
     const int k_elems = kGKBytes / es;
     const int nkb = (h->ld + k_elems - 1) / k_elems;
     const int pend = nb <= 16 ? 64 : 32;
-    const bool can_split = h->dtype != 0;
+    const bool can_split = h->sweep_dt != 0;
     // candidates in order of preference: split (tight error bound) first, then plain
     const int cols_split[3] = {16, 32, 64}, cols_plain[3] = {16, 32, 64};
     for (int pass = 0; pass < 2; ++pass) {
@@ -1142,12 +1242,13 @@ static int run_fused(ragfin* h, const float* q_dev, int nb, int k, int64_t n_eff
     h->fused_last = half;
     const GemmPlan p = plan_gemm(nb, n, h->num_sms, 32, 1);
     CUtensorMap tmB;
-    if ((rc = cached_map(h, &tmB, h->dtype, h->data, n, h->ld, kGN))) return rc;
+    if ((rc = cached_map(h, &tmB, h->sweep_dt, h->sweep_data, n, h->ld, kGN))) return rc;
     FusedArgs a;
-    a.idesc = make_idesc_n(h->dtype == 0 ? 2 : h->dtype == 1 ? 1 : 0, f.ncol);
-    a.k_elems = kGKBytes / (int)esize(h->dtype);
+    a.idesc = make_idesc_n(h->sweep_dt == 0 ? 2 : h->sweep_dt == 1 ? 1 : 0, f.ncol);
+    a.k_elems = kGKBytes / (int)esize(h->sweep_dt);
     a.num_kblocks = (h->ld + a.k_elems - 1) / a.k_elems;
     a.dt = h->dtype;
+    a.sdt = h->sweep_dt;
     a.nq = nb; a.dim = h->dim; a.ld = h->ld;
     a.n_rows = n;
     a.S = p.S; a.rows_per_slice = p.rows_per_slice;
@@ -1167,7 +1268,7 @@ static int run_fused(ragfin* h, const float* q_dev, int nb, int k, int64_t n_eff
     a.allow = h->cur_allow;
     a.cand = (u64*)((char*)h->fcand.p + half * cand_half); a.cap = f.cap;
     a.ctl = (FusedCtl*)h->fctl.p + half;
-    a.eps_const = eps_gemm_const(h->dtype, h->ld);
+    a.eps_const = eps_approx(h);
     a.id_base = h->id_base;
     a.out_ids = (long long*)out_ids; a.out_scores = out_scores;
     a.flags = (int*)h->fflags.p + half * (kFMaxQ + 1); a.flag_count = a.flags + kFMaxQ;
@@ -1176,7 +1277,7 @@ static int run_fused(ragfin* h, const float* q_dev, int nb, int k, int64_t n_eff
         a.xworld = x->world; a.xrank = x->rank; a.xstep = xstep; a.xrec_max = x->record_max;
         a.xpeer_area = x->d_peer_area; a.xpeer_qflag = x->d_peer_qflag;
     }
-    fused_fn fn = pick_fused(h->dtype, f.ncol, f.split);
+    fused_fn fn = pick_fused(h->sweep_dt, f.ncol, f.split);
     if ((rc = set_dyn_smem(h->device, (const void*)fn, f.smem))) return rc;
     h->fctl_dirty = true;          // until the launch is known to have been accepted
     cudaLaunchConfig_t cfg = {};
@@ -1263,7 +1364,7 @@ static int search_bigk_batched(ragfin* h, const float* q_dev, int nq, int k, int
     const int nbq = kGM;                                   // the sweep pads the query tile to 128 rows
     if ((rc = ensure(h->qhat, (size_t)nbq * h->ld * sizeof(float)))) return rc;
     if ((rc = ensure(h->eps_q, (size_t)nbq * sizeof(float))) || (rc = ensure(h->gtau, (size_t)nbq * sizeof(uint32_t)))) return rc;
-    if (h->dtype != 0 && (rc = ensure(h->q16, (size_t)nbq * h->ld * 2))) return rc;
+    if (h->sweep_dt != 0 && (rc = ensure(h->q16, (size_t)nbq * h->ld * 2))) return rc;
     if ((rc = ensure(h->flags, (size_t)(kMaxQueryBatch + 1) * sizeof(int)))) return rc;
     if ((rc = ensure(h->bk_scores, (size_t)kBigChunk * n * sizeof(float)))) return rc;
     if ((rc = ensure(h->bk_state, (size_t)nq * sizeof(BkState)))) return rc;
@@ -1275,12 +1376,12 @@ static int search_bigk_batched(ragfin* h, const float* q_dev, int nq, int k, int
     int* flag_count = (int*)h->flags.p + kMaxQueryBatch;
     CU_TRY(cudaMemsetAsync(states, 0, (size_t)nq * sizeof(BkState), st));
     const int blocks = h->num_sms * 8;
-    const float eps = eps_gemm_const(h->dtype, h->ld);
+    const float eps = eps_approx(h);
     for (int q0 = 0; q0 < nq; q0 += kBigChunk) {
         const int nb = nq - q0 < kBigChunk ? nq - q0 : kBigChunk;
         const int wpb = 8, pblocks = (nbq + wpb - 1) / wpb;
         const float* qsrc = q_dev + (size_t)q0 * h->dim;
-        switch (h->dtype) {
+        switch (h->sweep_dt) {
             case 0: prep_queries_kernel<0><<<pblocks, wpb * 32, 0, st>>>(qsrc, nb, nbq, h->dim, h->ld, qhat, nullptr, (float*)h->eps_q.p, flag_count, (uint32_t*)h->gtau.p); break;
             case 1: prep_queries_kernel<1><<<pblocks, wpb * 32, 0, st>>>(qsrc, nb, nbq, h->dim, h->ld, qhat, (__nv_bfloat16*)h->q16.p, (float*)h->eps_q.p, flag_count, (uint32_t*)h->gtau.p); break;
             default: prep_queries_kernel<2><<<pblocks, wpb * 32, 0, st>>>(qsrc, nb, nbq, h->dim, h->ld, qhat, (__half*)h->q16.p, (float*)h->eps_q.p, flag_count, (uint32_t*)h->gtau.p); break;
@@ -1368,10 +1469,10 @@ static int search_locked(ragfin* h, const float* q_dev, int nq, int k, int64_t* 
         const bool prepped = via_gemm && !(!ap && use_astat(h, kp));   // the 16-bit query copy is made here too
         {   // one launch: normalise + pad + [16-bit copy + eps_q] + counters (flags[q] itself is written by finalize for every q)
             if ((rc = ensure(h->eps_q, (size_t)nbq * sizeof(float))) || (rc = ensure(h->gtau, (size_t)nbq * sizeof(uint32_t)))) return rc;
-            if (prepped && h->dtype != 0 && (rc = ensure(h->q16, (size_t)nbq * h->ld * 2))) return rc;
+            if (prepped && h->sweep_dt != 0 && (rc = ensure(h->q16, (size_t)nbq * h->ld * 2))) return rc;
             const int wpb = 8, blocks = (nbq + wpb - 1) / wpb;
             const float* qsrc = q_dev + (size_t)q0 * h->dim;
-            switch (prepped ? h->dtype : 0) {
+            switch (prepped ? h->sweep_dt : 0) {
                 case 0: RF_LAUNCH(prep_queries_kernel<0>, blocks, wpb * 32, 0, st, qsrc, nb, nbq, h->dim, h->ld, qhat, nullptr, (float*)h->eps_q.p, flag_count, (uint32_t*)h->gtau.p); break;
                 case 1: RF_LAUNCH(prep_queries_kernel<1>, blocks, wpb * 32, 0, st, qsrc, nb, nbq, h->dim, h->ld, qhat, (__nv_bfloat16*)h->q16.p, (float*)h->eps_q.p, flag_count, (uint32_t*)h->gtau.p); break;
                 default: RF_LAUNCH(prep_queries_kernel<2>, blocks, wpb * 32, 0, st, qsrc, nb, nbq, h->dim, h->ld, qhat, (__half*)h->q16.p, (float*)h->eps_q.p, flag_count, (uint32_t*)h->gtau.p); break;
@@ -1391,7 +1492,7 @@ static int search_locked(ragfin* h, const float* q_dev, int nq, int k, int64_t* 
             h->stats.path = 1;
             sorted_lists = 0;
             scanned = true;
-            eps = eps_gemm_const(h->dtype, h->ld);
+            eps = eps_approx(h);
             eps_q = (const float*)h->eps_q.p;
         } else {
             // 2b. scan in groups of <= 4 queries.  Candidate layout [nb4][G][kp]; a group whose kernel
@@ -1508,7 +1609,7 @@ extern "C" int ragfin_save(ragfin_t* h, const char* path) {
     FileHeader hd;
     memset(&hd, 0, sizeof(hd));
     memcpy(hd.magic, "RAGFINB2", 8);
-    hd.version = 1; hd.dim = (uint32_t)h->dim; hd.ld = (uint32_t)h->ld; hd.dtype = (uint32_t)h->dtype;
+    hd.version = 1; hd.dim = (uint32_t)h->dim; hd.ld = (uint32_t)h->ld; hd.dtype = (uint32_t)public_dtype(h);   // rows: the fp32 ones
     hd.count = h->count; hd.id_base = h->id_base;
     int rc = 0;
     if (fwrite(&hd, sizeof(hd), 1, f) != 1) rc = fail(RAGFIN_EINVAL, "write to %s failed", path);
@@ -1532,7 +1633,7 @@ extern "C" int ragfin_load(ragfin_t** out, const char* path, int64_t capacity_ro
     FILE* f = fopen(path, "rb");
     if (!f) return fail(RAGFIN_EINVAL, "cannot open %s", path);
     FileHeader hd;
-    if (fread(&hd, sizeof(hd), 1, f) != 1 || memcmp(hd.magic, "RAGFINB2", 8) != 0 || hd.version != 1 || hd.dtype > 2 ||
+    if (fread(&hd, sizeof(hd), 1, f) != 1 || memcmp(hd.magic, "RAGFINB2", 8) != 0 || hd.version != 1 || hd.dtype > 3 ||
         hd.ld != (hd.dim + 7) / 8 * 8 || hd.count < 0) {
         fclose(f);
         return fail(RAGFIN_EINVAL, "%s is not a ragfin matrix file", path);
@@ -1553,6 +1654,14 @@ extern "C" int ragfin_load(ragfin_t** out, const char* path, int64_t capacity_ro
     }
     if (host) cudaFreeHost(host);
     fclose(f);
+    if (!rc && has_copy(h) && hd.count > 0) {   // the fp16 copy is not in the file: rebuilt from the fp32 rows (ld % 8 == 0)
+        const int64_t n4 = hd.count * h->ld / 4;
+        const int64_t cap_blocks = (int64_t)h->num_sms * 8, want = (n4 + 255) / 256;
+        cast_f16_kernel<<<(unsigned)(want < cap_blocks ? want : cap_blocks), 256>>>((const float4*)h->data, (uint2*)h->sweep_data, n4);
+        cudaError_t e = cudaGetLastError();
+        if (e == cudaSuccess) e = cudaDeviceSynchronize();
+        if (e != cudaSuccess) { (void)cudaGetLastError(); rc = fail(RAGFIN_ECUDA, "rebuilding the fp16 copy failed: %s", cudaGetErrorString(e)); }
+    }
     if (rc) { ragfin_destroy(h); return rc; }
     h->count = hd.count;
     h->id_base = hd.id_base;
@@ -1832,7 +1941,7 @@ extern "C" int ragfin_search_host(ragfin_t* h, const float* q_host, int32_t nq, 
         // small request: three copy-engine launches (~20 us) would cost more than the bytes; the kernels read the queries
         // from, and write the hits to, device-mapped pinned memory
         if (!h->hstage) {
-            if (cudaHostAlloc(&h->hstage, kHostStageQ + kHostStageOut + kHostStageFlag, cudaHostAllocMapped) != cudaSuccess) { (void)cudaGetLastError(); h->hstage = nullptr; }
+            (void)alloc_hstage(h);
         }
         void* dptr = nullptr;
         if (h->hstage && cudaHostGetDevicePointer(&dptr, h->hstage, 0) == cudaSuccess) {
@@ -2165,10 +2274,7 @@ extern "C" int ragfin_search_sharded_host(ragfin_t* h, ragfin_exchange_t* x, con
     if (nq > h->fused_max_nq || !fused_eligible(h, nq, k))
         return fail(RAGFIN_EUNSUPPORTED, "shape (nq = %d, k = %d) does not take the one-kernel search on this shard", nq, k);
     if ((size_t)nq * (((size_t)k * 12 + 15) / 16 * 16) > x->record_max) return fail(RAGFIN_EINVAL, "record exceeds the exchange's %zu bytes", x->record_max);
-    if (!h->hstage && cudaHostAlloc(&h->hstage, kHostStageQ + kHostStageOut + kHostStageFlag, cudaHostAllocMapped) != cudaSuccess) {
-        (void)cudaGetLastError(); h->hstage = nullptr;
-        return fail(RAGFIN_ENOMEM, "pinned staging allocation failed");
-    }
+    if (!h->hstage && (rc = alloc_hstage(h))) return rc;
     if ((rc = fused_host_call(h, x, q_host, nq, k, out_ids_host, out_scores_host, st))) return rc;
     // a finalizing CTA that waited 4 s for a peer's hits gives up and marks the query's empty slots with NaN scores
     for (size_t i = 0; i < (size_t)nq * k; ++i)

@@ -82,7 +82,9 @@ struct alignas(16) FusedInlineQ { float v[kFInlineFloats]; };   // 16-byte align
 struct FusedArgs {
     uint32_t idesc;             // M = 128, N = NCOL
     int num_kblocks, k_elems;   // k-blocks of 128 bytes; elements per k-block (64 for 16-bit storage, 32 for fp32)
-    int dt;                     // storage type of the corpus: 0 fp32, 1 bf16, 2 fp16
+    int dt;                     // type of `data`, the rows the exact rescore reads: 0 fp32, 1 bf16, 2 fp16
+    int sdt;                    // type of the rows tmB sweeps (the 16-bit query split follows it): = dt, except 2 on an fp32
+                                // collection with an fp16 copy (RAGFIN_F32_F16)
     int nq, dim, ld;
     long long n_rows;
     int S;                      // corpus slices
@@ -101,7 +103,7 @@ struct FusedArgs {
     u64* cand;                  // [nq][cap] append buffers
     int cap;
     FusedCtl* ctl;
-    float eps_const;            // accumulation allowance (+ tf32 truncation), see eps_gemm_const
+    float eps_const;            // accumulation allowance (+ tf32 truncation, + the fp16 copy's rounding), see eps_approx
     long long id_base;
     long long* out_ids;         // [nq][k]
     float* out_scores;          // [nq][k]
@@ -376,7 +378,7 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
                                 uint16_t hb[2], lb[2];
 #pragma unroll
                                 for (int t2 = 0; t2 < 2; ++t2) {
-                                    if (a.dt == 1) {
+                                    if (a.sdt == 1) {
                                         const __nv_bfloat16 hi = __float2bfloat16_rn(y[e + t2]);
                                         const float rest = y[e + t2] - __bfloat162float(hi);             // exact
                                         const __nv_bfloat16 lo = SPLIT ? __float2bfloat16_rn(rest) : __float2bfloat16_rn(0.f);
@@ -426,7 +428,7 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
                         } else {
                             // the lo row is 8 MMA columns further: same position inside the next 8-row group (+1024 bytes)
                             uint8_t* p_lo = p_hi + 1024;
-                            if (a.dt == 1) {
+                            if (a.sdt == 1) {
                                 const __nv_bfloat16 hi = __float2bfloat16_rn(y);
                                 const float rest = y - __bfloat162float(hi);        // exact
                                 const __nv_bfloat16 lo = SPLIT ? __float2bfloat16_rn(rest) : __float2bfloat16_rn(0.f);
@@ -452,8 +454,8 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
         {
             float eq = 0.f;
             if (KIND != 1) {
-                const float rel = a.dt == 1 ? (SPLIT ? 3.814697265625e-06f : 1.953125e-03f) : (SPLIT ? 5.9604644775390625e-08f : 2.44140625e-04f);
-                const float sub = a.dt == 1 ? 0.f : __fmul_ru(__fsqrt_ru((float)a.ld), 2.98023223876953125e-08f);
+                const float rel = a.sdt == 1 ? (SPLIT ? 3.814697265625e-06f : 1.953125e-03f) : (SPLIT ? 5.9604644775390625e-08f : 2.44140625e-04f);
+                const float sub = a.sdt == 1 ? 0.f : __fmul_ru(__fsqrt_ru((float)a.ld), 2.98023223876953125e-08f);
                 eq = __fmul_ru(__fadd_ru(rel, sub), 1.0078125f);
             }
             for (int j = tid; j < nq; j += kFThreads) eps_s[j] = __fadd_ru(a.eps_const, eq);

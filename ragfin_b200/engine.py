@@ -12,7 +12,10 @@ import numpy as np
 
 from . import _lib
 
-DTYPE_CODE = {"f32": 0, "fp32": 0, "float32": 0, "bf16": 1, "bfloat16": 1, "f16": 2, "fp16": 2, "float16": 2}
+# "f32+f16": fp32 rows (every exact step, so results equal "f32") plus an fp16 copy the tensor-core sweeps stream;
+# 6 bytes per element (include/ragfin.h, RAGFIN_F32_F16)
+DTYPE_CODE = {"f32": 0, "fp32": 0, "float32": 0, "bf16": 1, "bfloat16": 1, "f16": 2, "fp16": 2, "float16": 2, "f32+f16": 3}
+_DTYPE_NAME = ("f32", "bf16", "f16", "f32+f16")   # by header code
 MAX_TOPK = 16384  # Milvus' own limit on `limit`
 
 
@@ -89,7 +92,7 @@ class Index:
         with open(path, "rb") as f:
             hd = f.read(64)
         self.dim = int.from_bytes(hd[12:16], "little")
-        self.dtype = ("f32", "bf16", "f16")[int.from_bytes(hd[20:24], "little")]
+        self.dtype = _DTYPE_NAME[int.from_bytes(hd[20:24], "little")]
         self.capacity = max(int(capacity), int.from_bytes(hd[24:32], "little", signed=True), 1)
         return self
 
@@ -168,12 +171,21 @@ class Index:
         _lib.check(self._L.ragfin_add_synthetic_topics(self._h, seed, row0, n, topic_rows, noise_shift, None))
 
     def read_rows(self, row0: int, n: int) -> np.ndarray:
-        """Stored rows as fp32 values [n, dim] (test hook for ingest parity)."""
-        ld = (self.dim + 7) // 8 * 8
+        """Stored rows as fp32 values [n, dim] (test hook for ingest parity); the fp32 rows of an "f32+f16" index."""
         code = DTYPE_CODE[self.dtype]
+        return self._read(self._L.ragfin_read_rows, 0 if code == 3 else code, row0, n)
+
+    def read_sweep_rows(self, row0: int, n: int) -> np.ndarray:
+        """The rows the tensor-core sweeps read, as fp32 values [n, dim] (test hook): the fp16 copy of an "f32+f16" index,
+        the stored rows otherwise."""
+        code = DTYPE_CODE[self.dtype]
+        return self._read(self._L.ragfin_read_sweep_rows, 2 if code == 3 else code, row0, n)
+
+    def _read(self, fn, code: int, row0: int, n: int) -> np.ndarray:
+        ld = (self.dim + 7) // 8 * 8
         raw = np.empty((n, ld), dtype=np.float32 if code == 0 else np.uint16)
         ldo = ctypes.c_int32()
-        _lib.check(self._L.ragfin_read_rows(self._h, row0, n, raw.ctypes.data, ctypes.byref(ldo)))
+        _lib.check(fn(self._h, row0, n, raw.ctypes.data, ctypes.byref(ldo)))
         assert ldo.value == ld
         if code == 0:
             out = raw
