@@ -46,7 +46,9 @@ enum {
     RAGFIN_EUNSUPPORTED = -4
 };
 
-/* ABI version of this header; bumped on any signature change. */
+/* ABI version of this header; bumped on any signature change.  Version 4 also carries the row-deletion entry points
+ * (ragfin_delete, ragfin_live_count, ragfin_read_live_mask, ragfin_compact): they were added without changing any existing
+ * signature, so the version stays 4. */
 #define RAGFIN_ABI_VERSION 4
 int ragfin_abi_version(void);
 
@@ -85,6 +87,28 @@ int ragfin_add_synthetic_topics(ragfin_t* h, uint64_t seed, int64_t row0, int64_
 
 /* Number of rows held.  Replaces: Collection.num_entities - vector_rag_mcp/main.py:164. */
 int ragfin_count(const ragfin_t* h, int64_t* n);
+
+/* Row deletion.  ragfin_delete tombstones rows by the ids searches return (id_base + row): from then on no search entry point
+ * returns them, and searches keep the unfiltered kernel dispatch (the bound pass and the append-mode epilogues read the
+ * tombstone mask).  Duplicate ids and ids deleted before are allowed; *n_deleted_out (may be NULL) counts the rows this call
+ * deleted.  An id outside [id_base, id_base + count) fails the whole call with RAGFIN_EINVAL and changes nothing; a view
+ * returns RAGFIN_EUNSUPPORTED.  The call waits for the handle's searches in flight (the mask they read changes), under the
+ * same lock as ragfin_add.  Rows added later are live.  The handle keeps a host mirror of the mask; the device mask
+ * (capacity / 8 bytes) is allocated on the first delete, and a handle that never deletes allocates nothing for it.
+ * ragfin_count keeps counting the rows stored; ragfin_live_count returns stored minus tombstoned.
+ * ragfin_read_live_mask copies ceil(count / 32) words in the allow_bits layout (bit set = row live) - test hook.
+ * A filtered search on a handle with tombstones searches allow AND live; n_allowed still counts the caller's bits (the library
+ * counts what survives the AND itself: on the host for _filtered_host, with one extra stream synchronisation for the device
+ * mask of _filtered).  ragfin_search_sharded[_host] on a handle with tombstones returns RAGFIN_EUNSUPPORTED: compact first.
+ * ragfin_compact removes the tombstoned rows physically: survivors keep their order, new row r is the r-th live row (ids
+ * become id_base + new ordinal), the capacity is unchanged and the tombstones are cleared.  It builds the compacted matrix in a
+ * second allocation, so it needs a second copy of the matrix transiently (of both matrices on RAGFIN_F32_F16: 92 GB at
+ * 10M x 768), and synchronises the device.  RAGFIN_EUNSUPPORTED on a view or while views of the handle are live.
+ * Replaces: Collection.delete(expr) / upsert(data) / compact() of pymilvus 2.3. */
+int ragfin_delete(ragfin_t* h, const int64_t* ids_host, int64_t n, int64_t* n_deleted_out);
+int ragfin_live_count(const ragfin_t* h, int64_t* n);
+int ragfin_read_live_mask(ragfin_t* h, uint32_t* out_host);
+int ragfin_compact(ragfin_t* h);
 
 /* Grow the matrix to at least capacity_rows rows: a new device allocation and a device-to-device copy of the stored rows
  * (bits unchanged, nothing re-normalised, no host copy of the embeddings).  No-op when the capacity is already there.
@@ -198,7 +222,9 @@ int ragfin_profile_read(ragfin_t* h, double* total_ms, int32_t* launches);
 
 /* Persistence of the device-resident matrix (stands in for Milvus' flush()/load() durability,
  * "chunking_storing (1).py":395-396, retrieve.py:18-19).  File = 64-byte header {magic "RAGFINB2", version,
- * dim, ld, dtype, count, id_base} + the stored rows [count, ld] exactly as they sit in HBM, so a
+ * dim, ld, dtype, count, id_base} + the stored rows [count, ld] exactly as they sit in HBM.  A handle without tombstones
+ * writes version 1; with tombstones, version 2: the tombstone count (int64) in the header's first spare bytes (offset 40)
+ * and ceil(count / 32) live-mask words after the rows.  ragfin_load reads both versions.  So a
  * reloaded collection returns bit-identical results without re-normalising.  A RAGFIN_F32_F16 file has header dtype 3 and
  * holds the fp32 rows only; ragfin_load rebuilds the fp16 copy from them on the device (same bits as at ingest).
  * ragfin_load creates a new handle on `device` with room for max(capacity_rows, count) rows. */
@@ -255,7 +281,7 @@ int ragfin_set_fused(ragfin_t* h, int32_t enable, int64_t min_rows);
  * pipelined search may begin before the operation enqueued just ahead of it on the stream has completed, so its query buffer
  * must already hold the queries when the PREVIOUS search on this handle was enqueued (written by work ordered before that
  * search, or by the host).  Queries produced by a kernel enqueued between two searches need pipelining off.  Only a search
- * that directly follows this handle's own one-kernel search on the same stream is launched this way; after an add, a filter,
+ * that directly follows this handle's own one-kernel search on the same stream is launched this way; after an add, a delete, a filter,
  * another path or another stream the launch is an ordinary one.  Results are identical either way.
  * Replaces: nothing in the reference (its searches are sequential gRPC calls - vector_rag_mcp/main.py:51-57). */
 int ragfin_set_pipelined(ragfin_t* h, int32_t enable);
@@ -289,7 +315,9 @@ int ragfin_debug_plan(int32_t nq, int64_t n_rows, int32_t num_sms, int32_t k, in
  * view (or two views) may be in flight at once on different streams, so the latency-bound head and tail of one call
  * (query preparation, bound pass, finalize, exchange) overlap the neighbour's sweep.  Replaces nothing in the reference
  * (a Milvus querynode serves concurrent searches from one loaded segment the same way).  The view sees the rows present
- * when it is made, inherits the parent's tuning knobs, is read-only (ragfin_add returns RAGFIN_EUNSUPPORTED) and must
+ * when it is made (and the tombstones present then: it keeps its own copy of the mask), inherits the parent's tuning knobs,
+ * is read-only (ragfin_add, ragfin_delete and ragfin_compact return RAGFIN_EUNSUPPORTED), blocks ragfin_compact on its parent
+ * while it lives (ragfin_reserve of a parent with live views remains the caller's hazard) and must
  * be destroyed before its parent.  Measured (scripts/pipeline_check.py, profiles/r02): 1.25M-row shard, batch 1, three
  * handles on three streams: 0.284 ms per query against 0.327 ms on one handle. */
 int ragfin_create_view(ragfin_t* parent, ragfin_t** out);

@@ -410,6 +410,16 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                         for (int j = 0; j < 32; ++j)
                             if (c * 32 + j >= valid) v[j] = 0x7FC00000u;   // NaN: fails every >= test, ignored by fmaxf
                     }
+                    if (MODE == 2 && a.allow != nullptr && c * 32 < valid) {
+                        // bound pass over a masked corpus (tombstones): excluded rows must not raise a block maximum.  Tiles
+                        // start at multiples of kGN, so the chunk's 32 rows are exactly one mask word.
+                        const uint32_t w = __ldg(a.allow + ((trow + c * 32) >> 5));
+                        if (w != 0xFFFFFFFFu) {
+#pragma unroll
+                            for (int j = 0; j < 32; ++j)
+                                if (!((w >> j) & 1u)) v[j] = 0x7FC00000u;
+                        }
+                    }
                     // maxima of the four groups of 8 columns, then of the chunk: one compare in the common case
                     float gmx[4];
 #pragma unroll
@@ -429,9 +439,12 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 #pragma unroll
                                     for (int j = 0; j < 8; ++j) {
                                         const float sc = __uint_as_float(v[g * 8 + j]);
-                                        if (sc >= thr3) {   // one atomic per appended row (measured: reserving slots in blocks is no faster)
+                                        const long long row = trow + c * 32 + g * 8 + j;
+                                        // one atomic per appended row (measured: reserving slots in blocks is no faster); a
+                                        // masked (tombstoned) row never takes a slot
+                                        if (sc >= thr3 && (a.allow == nullptr || row_allowed(a.allow, row))) {
                                             const uint32_t pos = atomicAdd(cnt3, 1u);
-                                            if (pos < (uint32_t)a.cap) buf3[pos] = make_key(sc + 0.0f, (uint32_t)(trow + c * 32 + g * 8 + j));
+                                            if (pos < (uint32_t)a.cap) buf3[pos] = make_key(sc + 0.0f, (uint32_t)row);
                                         }
                                     }
                                 }

@@ -242,9 +242,10 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 #pragma unroll
                                 for (int j = 0; j < 8; ++j) {
                                     const float sc = __uint_as_float(v[g * 8 + j]);
-                                    if (sc >= thr3) {
+                                    const long long row = trow + c * 32 + g * 8 + j;
+                                    if (sc >= thr3 && (a.allow == nullptr || row_allowed(a.allow, row))) {   // tombstones never take a slot
                                         const uint32_t pos = atomicAdd(cnt3, 1u);
-                                        if (pos < (uint32_t)a.cap) buf3[pos] = make_key(sc + 0.0f, (uint32_t)(trow + c * 32 + g * 8 + j));
+                                        if (pos < (uint32_t)a.cap) buf3[pos] = make_key(sc + 0.0f, (uint32_t)row);
                                     }
                                 }
                             }

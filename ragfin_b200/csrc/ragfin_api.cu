@@ -20,6 +20,7 @@
 #include "sweep_fused.cuh"
 #include "scan_tma.cuh"
 #include "bigk.cuh"
+#include "tombstones.cuh"
 
 using namespace rfk;
 
@@ -75,8 +76,17 @@ struct ragfin {
     int gemm_cluster = 0;     // 0 = choose by batch size; 1, 2 or 4 = force
     bool allow_pipelined = false;          // ragfin_set_pipelined: consecutive one-kernel searches on one stream may overlap (see there)
     bool cur_pipelined = false;            // the search in flight came through an asynchronous entry point (ragfin_search)
-    const uint32_t* cur_allow = nullptr;   // scalar filter of the search in flight (device bitmask), else null
+    const uint32_t* cur_allow = nullptr;   // row mask of the search in flight (device bitmask: filter, tombstones or both), else null
     int64_t cur_allowed = 0;               // rows it allows
+    bool cur_user_filter = false;          // the caller passed a filter: filtered dispatch (no bound pass, no append mode)
+    // Tombstones (ragfin_delete).  live_host mirrors the device mask live_dev bit for bit: ceil(capacity / 32) words in the
+    // allow_bits layout, bit set = row live; rows at or past `count` are live (rows added later are).  Both stay empty until
+    // the first delete, and a handle with n_dead == 0 passes a null mask to every kernel.
+    std::vector<uint32_t> live_host;
+    uint32_t* live_dev = nullptr;
+    int64_t n_dead = 0;
+    ragfin* parent = nullptr;   // a view's owner (ragfin_create_view)
+    int n_views = 0;            // live views of this handle: compaction would move rows under them
     int scan_variant = 0;         // small-batch scan: 0 = automatic (= 1, measured faster), 1 = LDG kernel, 2 = TMA-fed ring
     bool use_append = true;       // tcgen05 path: append mode (threshold from the bound pass, no lists) when eligible
     bool use_bound_pass = true;   // tcgen05 path: sample pass that seeds the per-query thresholds (RAGFIN_NO_BOUND_PASS=1 disables)
@@ -122,6 +132,7 @@ static void prof_end(ragfin* h, cudaStream_t st) {
 }
 
 static size_t esize(int dtype) { return dtype == RAGFIN_F32 ? 4 : 2; }
+static size_t mask_words(int64_t rows) { return (size_t)((rows + 31) / 32); }
 static bool has_copy(const ragfin* h) { return h->sweep_data != h->data; }
 // dtype as the caller named it (ragfin_create, the file header)
 static int public_dtype(const ragfin* h) { return has_copy(h) ? RAGFIN_F32_F16 : h->dtype; }
@@ -270,6 +281,22 @@ extern "C" int ragfin_create_view(ragfin_t* parent, ragfin_t** out) {
         delete h;
         return fail(RAGFIN_ECUDA, "cudaEventCreate failed: %s", cudaGetErrorString(e));
     }
+    if (parent->n_dead > 0) {   // the view's own copy of the tombstones: rows deleted through the parent later stay visible here
+        const size_t words = mask_words(h->capacity);
+        h->live_host.assign(parent->live_host.begin(), parent->live_host.begin() + words);
+        e = cudaMalloc(&h->live_dev, words * sizeof(uint32_t));
+        if (e == cudaSuccess) e = cudaMemcpy(h->live_dev, parent->live_dev, words * sizeof(uint32_t), cudaMemcpyDeviceToDevice);
+        if (e != cudaSuccess) {
+            (void)cudaGetLastError();
+            if (h->live_dev) cudaFree(h->live_dev);
+            cudaEventDestroy(h->last_done);
+            delete h;
+            return fail(RAGFIN_ENOMEM, "copying the tombstone mask failed: %s", cudaGetErrorString(e));
+        }
+        h->n_dead = parent->n_dead;
+    }
+    h->parent = parent;
+    parent->n_views++;
     *out = h;
     return RAGFIN_OK;
 }
@@ -283,6 +310,11 @@ extern "C" void ragfin_destroy(ragfin_t* h) {
         if (b->p) cudaFree(b->p);
     if (h->sweep_data && has_copy(h) && !h->is_view) cudaFree(h->sweep_data);
     if (h->data && !h->is_view) cudaFree(h->data);
+    if (h->live_dev) cudaFree(h->live_dev);
+    if (h->parent) {
+        std::lock_guard<std::mutex> lk(h->parent->mu);
+        h->parent->n_views--;
+    }
     for (int b = 0; b < 2; ++b) {
         if (h->add_stage2[b].p) cudaFree(h->add_stage2[b].p);
         if (h->stage_ready[b]) cudaEventDestroy(h->stage_ready[b]);
@@ -300,6 +332,145 @@ extern "C" int ragfin_count(const ragfin_t* h, int64_t* n) {
     if (!h || !n) return fail(RAGFIN_EINVAL, "NULL argument");
     std::lock_guard<std::mutex> lk(const_cast<ragfin*>(h)->mu);   // count is written under the lock by ragfin_add
     *n = h->count;
+    return RAGFIN_OK;
+}
+
+extern "C" int ragfin_live_count(const ragfin_t* h, int64_t* n) {
+    if (!h || !n) return fail(RAGFIN_EINVAL, "NULL argument");
+    std::lock_guard<std::mutex> lk(const_cast<ragfin*>(h)->mu);
+    *n = h->count - h->n_dead;
+    return RAGFIN_OK;
+}
+
+// Tombstone rows by the ids searches return (id_base + row).  The host mirror decides what changes, so duplicates and rows
+// deleted before cost nothing; only the words that changed go to the device.  The device mask is read by searches still in
+// flight, so the call first waits for the handle's last operation (the completion event ragfin_add orders itself behind).
+extern "C" int ragfin_delete(ragfin_t* h, const int64_t* ids_host, int64_t n, int64_t* n_deleted_out) {
+    if (!h || n < 0 || (n > 0 && !ids_host)) return fail(RAGFIN_EINVAL, "bad argument");
+    std::lock_guard<std::mutex> lk(h->mu);
+    if (h->is_view) return fail(RAGFIN_EUNSUPPORTED, "a view is read-only: delete rows through the handle that owns the matrix");
+    for (int64_t i = 0; i < n; ++i)   // validate everything before anything changes
+        if (ids_host[i] < h->id_base || ids_host[i] - h->id_base >= h->count)
+            return fail(RAGFIN_EINVAL, "id %lld outside [%lld, %lld)", (long long)ids_host[i], (long long)h->id_base,
+                        (long long)(h->id_base + h->count));
+    if (n_deleted_out) *n_deleted_out = 0;
+    if (n == 0) return RAGFIN_OK;
+    DeviceGuard g(h->device);
+    if (h->have_pending) {   // a pipelined search never chains across a delete
+        CU_TRY(cudaEventRecord(h->last_done, h->pending_stream));
+        h->have_pending = false;
+    }
+    CU_TRY(cudaEventSynchronize(h->last_done));
+    const bool fresh = h->live_dev == nullptr;
+    if (fresh) {   // first delete: the mask covers the capacity, every row live
+        const size_t words = mask_words(h->capacity);
+        cudaError_t e = cudaMalloc(&h->live_dev, words * sizeof(uint32_t));
+        if (e != cudaSuccess) {
+            (void)cudaGetLastError();
+            h->live_dev = nullptr;
+            return fail(RAGFIN_ENOMEM, "cudaMalloc of the tombstone mask failed: %s", cudaGetErrorString(e));
+        }
+        h->live_host.assign(words, 0xFFFFFFFFu);
+    }
+    int64_t del = 0;
+    size_t w0 = fresh ? 0 : h->live_host.size(), w1 = fresh ? h->live_host.size() : 0;
+    for (int64_t i = 0; i < n; ++i) {
+        const int64_t r = ids_host[i] - h->id_base;
+        const size_t w = (size_t)(r >> 5);
+        const uint32_t bit = 1u << (r & 31);
+        if (!(h->live_host[w] & bit)) continue;
+        h->live_host[w] &= ~bit;
+        ++del;
+        if (w < w0) w0 = w;
+        if (w + 1 > w1) w1 = w + 1;
+    }
+    if (w1 > w0) CU_TRY(cudaMemcpy(h->live_dev + w0, h->live_host.data() + w0, (w1 - w0) * sizeof(uint32_t), cudaMemcpyHostToDevice));
+    h->n_dead += del;
+    if (n_deleted_out) *n_deleted_out = del;
+    return RAGFIN_OK;
+}
+
+// ceil(count / 32) words of the live mask as the kernels read it (the device copy; all ones without tombstones), bits at or
+// past `count` cleared.
+extern "C" int ragfin_read_live_mask(ragfin_t* h, uint32_t* out_host) {
+    if (!h || !out_host) return fail(RAGFIN_EINVAL, "NULL argument");
+    std::lock_guard<std::mutex> lk(h->mu);
+    const size_t words = mask_words(h->count);
+    if (words == 0) return RAGFIN_OK;
+    if (h->live_dev) {
+        DeviceGuard g(h->device);
+        CU_TRY(cudaDeviceSynchronize());
+        CU_TRY(cudaMemcpy(out_host, h->live_dev, words * sizeof(uint32_t), cudaMemcpyDeviceToHost));
+    } else {
+        for (size_t w = 0; w < words; ++w) out_host[w] = 0xFFFFFFFFu;
+    }
+    if (h->count & 31) out_host[words - 1] &= (1u << (h->count & 31)) - 1u;
+    return RAGFIN_OK;
+}
+
+// Physical removal of the tombstoned rows: survivors keep their order, live row r moves to the number of live rows before
+// it.  Into NEW allocations of the same capacity (the transient cost is a second copy of the matrix - of both on a
+// RAGFIN_F32_F16 handle), all made before anything is freed, so a failed allocation leaves the handle as it was.
+extern "C" int ragfin_compact(ragfin_t* h) {
+    if (!h) return fail(RAGFIN_EINVAL, "NULL handle");
+    std::lock_guard<std::mutex> lk(h->mu);
+    if (h->is_view) return fail(RAGFIN_EUNSUPPORTED, "a view is read-only");
+    if (h->n_views > 0) return fail(RAGFIN_EUNSUPPORTED, "%d view(s) of this collection are live: destroy them before compacting", h->n_views);
+    if (h->n_dead == 0) return RAGFIN_OK;
+    DeviceGuard g(h->device);
+    CU_TRY(cudaDeviceSynchronize());                 // no search may still be reading the old matrix
+    const size_t words = mask_words(h->count);
+    std::vector<uint32_t> off(words ? words : 1);    // exclusive prefix of the per-word live counts
+    uint32_t live = 0;
+    for (size_t w = 0; w < words; ++w) {
+        uint32_t v = h->live_host[w];
+        if (w + 1 == words && (h->count & 31)) v &= (1u << (h->count & 31)) - 1u;
+        off[w] = live;
+        live += (uint32_t)__builtin_popcount(v);
+    }
+    const size_t rb = (size_t)h->ld * esize(h->dtype), rb16 = (size_t)h->ld * 2;
+    void *nd = nullptr, *nd16 = nullptr, *doff = nullptr;
+    cudaError_t e = cudaMalloc(&nd, (size_t)h->capacity * rb);
+    if (e == cudaSuccess && has_copy(h)) e = cudaMalloc(&nd16, (size_t)h->capacity * rb16);
+    if (e == cudaSuccess) e = cudaMalloc(&doff, off.size() * sizeof(uint32_t));
+    if (e != cudaSuccess) {
+        (void)cudaGetLastError();
+        if (nd) cudaFree(nd);
+        if (nd16) cudaFree(nd16);
+        if (doff) cudaFree(doff);
+        return fail(RAGFIN_ENOMEM, "allocation for compaction failed (it needs a second copy of the matrix): %s", cudaGetErrorString(e));
+    }
+    e = cudaMemcpy(doff, off.data(), off.size() * sizeof(uint32_t), cudaMemcpyHostToDevice);
+    const int64_t want = (h->count + 7) / 8, cap_blocks = (int64_t)h->num_sms * 16;
+    const unsigned blocks = (unsigned)(want < cap_blocks ? (want > 0 ? want : 1) : cap_blocks);
+    prof_begin(h, 0);   // ragfin_profile: the gather kernels alone (the call also allocates and frees a matrix)
+    if (e == cudaSuccess) {
+        compact_rows_kernel<<<blocks, 256>>>((const uint4*)h->data, (uint4*)nd, (int)(rb / 16), h->count, h->live_dev, (const uint32_t*)doff);
+        e = cudaGetLastError();
+    }
+    if (e == cudaSuccess && nd16) {
+        compact_rows_kernel<<<blocks, 256>>>((const uint4*)h->sweep_data, (uint4*)nd16, (int)(rb16 / 16), h->count, h->live_dev, (const uint32_t*)doff);
+        e = cudaGetLastError();
+    }
+    prof_end(h, 0);
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    std::vector<uint32_t> ones(h->live_host.size(), 0xFFFFFFFFu);
+    if (e == cudaSuccess) e = cudaMemcpy(h->live_dev, ones.data(), ones.size() * sizeof(uint32_t), cudaMemcpyHostToDevice);
+    cudaFree(doff);
+    if (e != cudaSuccess) {
+        (void)cudaGetLastError();
+        cudaFree(nd);
+        if (nd16) cudaFree(nd16);
+        return fail(RAGFIN_ECUDA, "compaction failed: %s", cudaGetErrorString(e));
+    }
+    if (nd16) { CU_TRY(cudaFree(h->sweep_data)); h->sweep_data = nd16; }
+    CU_TRY(cudaFree(h->data));
+    h->data = nd;
+    if (!nd16) h->sweep_data = nd;
+    h->live_host.swap(ones);
+    h->count = live;
+    h->n_dead = 0;
+    for (ragfin::MapSlot& m : h->map_cache) m = ragfin::MapSlot();   // tensor maps of the old matrix are stale
     return RAGFIN_OK;
 }
 
@@ -333,6 +504,17 @@ extern "C" int ragfin_reserve(ragfin_t* h, int64_t capacity_rows) {
             return fail(RAGFIN_ENOMEM, "cudaMalloc of %zu bytes for the grown fp16 copy failed: %s", (size_t)capacity_rows * rb16, cudaGetErrorString(e));
         }
     }
+    uint32_t* nm = nullptr;   // the tombstone mask grows with the rows (new rows are live)
+    const size_t nwords = mask_words(capacity_rows);
+    if (h->live_dev) {
+        e = cudaMalloc(&nm, nwords * sizeof(uint32_t));
+        if (e != cudaSuccess) {
+            (void)cudaGetLastError();
+            cudaFree(nd);
+            if (nd16) cudaFree(nd16);
+            return fail(RAGFIN_ENOMEM, "cudaMalloc of the grown tombstone mask failed: %s", cudaGetErrorString(e));
+        }
+    }
     if (h->count > 0) {
         e = cudaMemcpy(nd, h->data, (size_t)h->count * rb, cudaMemcpyDeviceToDevice);
         if (e == cudaSuccess && nd16) e = cudaMemcpyAsync(nd16, h->sweep_data, (size_t)h->count * rb16, cudaMemcpyDeviceToDevice, 0);
@@ -340,9 +522,25 @@ extern "C" int ragfin_reserve(ragfin_t* h, int64_t capacity_rows) {
         if (e != cudaSuccess) {
             cudaFree(nd);
             if (nd16) cudaFree(nd16);
+            if (nm) cudaFree(nm);
             (void)cudaGetLastError();
             return fail(RAGFIN_ECUDA, "device copy failed: %s", cudaGetErrorString(e));
         }
+    }
+    if (nm) {
+        std::vector<uint32_t> grown(h->live_host);
+        grown.resize(nwords, 0xFFFFFFFFu);
+        e = cudaMemcpy(nm, grown.data(), nwords * sizeof(uint32_t), cudaMemcpyHostToDevice);
+        if (e != cudaSuccess) {
+            cudaFree(nd);
+            if (nd16) cudaFree(nd16);
+            cudaFree(nm);
+            (void)cudaGetLastError();
+            return fail(RAGFIN_ECUDA, "tombstone mask copy failed: %s", cudaGetErrorString(e));
+        }
+        CU_TRY(cudaFree(h->live_dev));
+        h->live_dev = nm;
+        h->live_host.swap(grown);
     }
     if (nd16) { CU_TRY(cudaFree(h->sweep_data)); h->sweep_data = nd16; }
     CU_TRY(cudaFree(h->data));
@@ -808,9 +1006,10 @@ static const int kAppendCap = 16384;   // append mode: keys one query may collec
 static const int kAppendMaxK = 256;    // largest k the append mode serves (tier 2, its overflow path, keeps 256 keys)
 
 // Append mode needs the bound pass (no scalar filter) and at least 4 k corpus tiles to draw 2 k sample blocks from.
+// Tombstones alone keep it: the bound pass and the append epilogues honour the mask (DESIGN.md, "Deleted rows").
 static bool append_eligible(const ragfin* h, int k) {
     const int64_t n_tiles = (h->count + kGN - 1) / kGN;
-    return h->use_bound_pass && h->use_append && h->cur_allow == nullptr && k <= kAppendMaxK && n_tiles >= 4 * (int64_t)k &&
+    return h->use_bound_pass && h->use_append && !h->cur_user_filter && k <= kAppendMaxK && n_tiles >= 4 * (int64_t)k &&
            h->count < ((int64_t)1 << 31) - kGN;
 }
 
@@ -876,10 +1075,10 @@ static int run_gemm(ragfin* h, int nb, int k, int kp, int* G, bool* appended, fl
 #undef RF_PICK_MODE
     // Sample ("bound") pass geometry.  nblk blocks of g sample tiles each, evenly strided over the corpus; the
     // rank-th largest block maximum bounds the rank-th best score from below.  Needs at least twice as many blocks
-    // as the rank and samples at most half of the corpus; skipped under a scalar filter (the maxima would count
-    // excluded rows) and for the dump hook.
+    // as the rank and samples at most half of the corpus; skipped under a scalar filter and for the dump hook.  Under
+    // tombstones alone it runs with the mask: excluded sample rows never raise a block maximum.
     const int64_t n_tiles = (n + kGN - 1) / kGN;
-    const bool can_bound = !dump && h->use_bound_pass && h->cur_allow == nullptr;
+    const bool can_bound = !dump && h->use_bound_pass && !h->cur_user_filter;
     const bool append = !dump && append_eligible(h, k);
     const bool bound = append || (can_bound && n_tiles >= 4 * (int64_t)kp);
     const int rank = append ? k : kp;
@@ -1004,7 +1203,7 @@ static int run_gemm(ragfin* h, int nb, int k, int kp, int* G, bool* appended, fl
         r.idesc = make_idesc_n(h->sweep_dt == 0 ? 2 : h->sweep_dt == 1 ? 1 : 0, kRN);
         r.num_kblocks = a.num_kblocks; r.k_elems = a.k_elems; r.nq = nb; r.n_rows = n;
         r.S = p.S; r.rows_per_slice = p.rows_per_slice; r.stages = rows_stages(a.num_kblocks);
-        r.cand = a.cand; r.thr = a.thr; r.cnt = a.cnt; r.cap = a.cap;
+        r.cand = a.cand; r.thr = a.thr; r.cnt = a.cnt; r.cap = a.cap; r.allow = a.allow;
         CUtensorMap tmQ;
         if ((rc = cached_map(h, &tmQ, h->sweep_dt, a_base, nb_pad, h->ld, kRN))) return rc;
         typedef void (*rows_fn)(const CUtensorMap, const CUtensorMap, const RowsArgs);
@@ -1609,8 +1808,9 @@ extern "C" int ragfin_save(ragfin_t* h, const char* path) {
     FileHeader hd;
     memset(&hd, 0, sizeof(hd));
     memcpy(hd.magic, "RAGFINB2", 8);
-    hd.version = 1; hd.dim = (uint32_t)h->dim; hd.ld = (uint32_t)h->ld; hd.dtype = (uint32_t)public_dtype(h);   // rows: the fp32 ones
+    hd.version = h->n_dead > 0 ? 2 : 1; hd.dim = (uint32_t)h->dim; hd.ld = (uint32_t)h->ld; hd.dtype = (uint32_t)public_dtype(h);   // rows: the fp32 ones
     hd.count = h->count; hd.id_base = h->id_base;
+    if (h->n_dead > 0) memcpy(hd.pad, &h->n_dead, sizeof(h->n_dead));   // version 2: tombstone count, then the live mask after the rows
     int rc = 0;
     if (fwrite(&hd, sizeof(hd), 1, f) != 1) rc = fail(RAGFIN_EINVAL, "write to %s failed", path);
     const size_t rb = (size_t)h->ld * esize(h->dtype);
@@ -1623,6 +1823,11 @@ extern "C" int ragfin_save(ragfin_t* h, const char* path) {
         if (fwrite(host, rb, (size_t)m, f) != (size_t)m) rc = fail(RAGFIN_EINVAL, "write to %s failed", path);
     }
     if (host) cudaFreeHost(host);
+    if (!rc && h->n_dead > 0) {
+        std::vector<uint32_t> m(h->live_host.begin(), h->live_host.begin() + mask_words(h->count));
+        if (h->count & 31) m.back() &= (1u << (h->count & 31)) - 1u;
+        if (fwrite(m.data(), sizeof(uint32_t), m.size(), f) != m.size()) rc = fail(RAGFIN_EINVAL, "write to %s failed", path);
+    }
     if (fclose(f) != 0 && !rc) rc = fail(RAGFIN_EINVAL, "close of %s failed", path);
     return rc;
 }
@@ -1633,7 +1838,7 @@ extern "C" int ragfin_load(ragfin_t** out, const char* path, int64_t capacity_ro
     FILE* f = fopen(path, "rb");
     if (!f) return fail(RAGFIN_EINVAL, "cannot open %s", path);
     FileHeader hd;
-    if (fread(&hd, sizeof(hd), 1, f) != 1 || memcmp(hd.magic, "RAGFINB2", 8) != 0 || hd.version != 1 || hd.dtype > 3 ||
+    if (fread(&hd, sizeof(hd), 1, f) != 1 || memcmp(hd.magic, "RAGFINB2", 8) != 0 || (hd.version != 1 && hd.version != 2) || hd.dtype > 3 ||
         hd.ld != (hd.dim + 7) / 8 * 8 || hd.count < 0) {
         fclose(f);
         return fail(RAGFIN_EINVAL, "%s is not a ragfin matrix file", path);
@@ -1653,6 +1858,25 @@ extern "C" int ragfin_load(ragfin_t** out, const char* path, int64_t capacity_ro
         if (cudaMemcpy((char*)h->data + (size_t)r0 * rb, host, (size_t)m * rb, cudaMemcpyHostToDevice) != cudaSuccess) { (void)cudaGetLastError(); rc = fail(RAGFIN_ECUDA, "device write failed"); }
     }
     if (host) cudaFreeHost(host);
+    int64_t n_dead = 0;
+    if (!rc && hd.version == 2) {   // tombstones: the live mask follows the rows
+        memcpy(&n_dead, hd.pad, sizeof(n_dead));
+        const size_t words = mask_words(hd.count), cap_words = mask_words(h->capacity);
+        std::vector<uint32_t> m(cap_words, 0xFFFFFFFFu);
+        int64_t live = 0;
+        if (fread(m.data(), sizeof(uint32_t), words, f) != words) rc = fail(RAGFIN_EINVAL, "%s is truncated", path);
+        for (size_t w = 0; !rc && w < words; ++w) {
+            if (w + 1 == words && (hd.count & 31)) m[w] |= ~((1u << (hd.count & 31)) - 1u);   // rows past count are live
+            live += __builtin_popcount(w + 1 == words && (hd.count & 31) ? m[w] & ((1u << (hd.count & 31)) - 1u) : m[w]);
+        }
+        if (!rc && (n_dead < 1 || live != hd.count - n_dead)) rc = fail(RAGFIN_EINVAL, "%s: the live mask does not match the tombstone count", path);
+        if (!rc) {
+            cudaError_t e = cudaMalloc(&h->live_dev, cap_words * sizeof(uint32_t));
+            if (e == cudaSuccess) e = cudaMemcpy(h->live_dev, m.data(), cap_words * sizeof(uint32_t), cudaMemcpyHostToDevice);
+            if (e != cudaSuccess) { (void)cudaGetLastError(); rc = fail(RAGFIN_ECUDA, "tombstone mask upload failed: %s", cudaGetErrorString(e)); }
+            h->live_host.swap(m);
+        }
+    }
     fclose(f);
     if (!rc && has_copy(h) && hd.count > 0) {   // the fp16 copy is not in the file: rebuilt from the fp32 rows (ld % 8 == 0)
         const int64_t n4 = hd.count * h->ld / 4;
@@ -1665,6 +1889,7 @@ extern "C" int ragfin_load(ragfin_t** out, const char* path, int64_t capacity_ro
     if (rc) { ragfin_destroy(h); return rc; }
     h->count = hd.count;
     h->id_base = hd.id_base;
+    h->n_dead = n_dead;
     *out = h;
     return RAGFIN_OK;
 }
@@ -1840,6 +2065,9 @@ extern "C" int ragfin_set_gemm_cluster(ragfin_t* h, int32_t cluster) {
     return RAGFIN_OK;
 }
 
+static int set_filter(ragfin* h, const uint32_t* allow_bits, int64_t n_allowed, int bits_on_device, cudaStream_t st);
+static void clear_filter(ragfin* h);
+
 extern "C" int ragfin_search(ragfin_t* h, const float* q, int32_t nq, int32_t k, int64_t* out_ids, float* out_scores,
                              void* stream) {
     if (!h) return fail(RAGFIN_EINVAL, "NULL handle");
@@ -1856,9 +2084,11 @@ extern "C" int ragfin_search(ragfin_t* h, const float* q, int32_t nq, int32_t k,
     const bool pipe = h->allow_pipelined && nq <= h->fused_max_nq && fused_eligible(h, nq, k);
     const bool chained = pipe && h->have_pending && st == h->pending_stream;
     if ((rc = wait_prev(h, st, pipe))) return rc;
+    if ((rc = set_filter(h, nullptr, 0, 1, st))) return rc;   // tombstones, if any
     h->cur_pipelined = chained;
     rc = search_locked(h, q, nq, k, out_ids, out_scores, st);
     h->cur_pipelined = false;
+    clear_filter(h);
     if (rc) return rc;
     return mark_done(h, st, pipe);
 }
@@ -1925,6 +2155,8 @@ static int fused_host_call(ragfin* h, ragfin_exchange* x, const float* q_host, i
     return 0;
 }
 
+static int search_host_locked(ragfin* h, const float* q_host, int nq, int k, int64_t* out_ids_host, float* out_scores_host,
+                              cudaStream_t st);
 extern "C" int ragfin_search_host(ragfin_t* h, const float* q_host, int32_t nq, int32_t k, int64_t* out_ids_host,
                                   float* out_scores_host) {
     if (!h) return fail(RAGFIN_EINVAL, "NULL handle");
@@ -1936,6 +2168,15 @@ extern "C" int ragfin_search_host(ragfin_t* h, const float* q_host, int32_t nq, 
     cudaStream_t st = 0;
     int rc;
     if ((rc = wait_prev(h, st))) return rc;
+    if ((rc = set_filter(h, nullptr, 0, 1, st))) return rc;   // tombstones, if any
+    rc = search_host_locked(h, q_host, nq, k, out_ids_host, out_scores_host, st);
+    clear_filter(h);
+    return rc;
+}
+
+static int search_host_locked(ragfin* h, const float* q_host, int nq, int k, int64_t* out_ids_host, float* out_scores_host,
+                              cudaStream_t st) {
+    int rc;
     const size_t qb = (size_t)nq * h->dim * sizeof(float), ib = (size_t)nq * k * sizeof(int64_t), sb = (size_t)nq * k * sizeof(float);
     if (qb <= kHostStageQ && ib + sb <= kHostStageOut) {
         // small request: three copy-engine launches (~20 us) would cost more than the bytes; the kernels read the queries
@@ -1972,18 +2213,66 @@ extern "C" int ragfin_search_host(ragfin_t* h, const float* q_host, int32_t nq, 
     return mark_done(h, st);
 }
 
-// Scalar-filtered search: bit r of allow_bits (ceil(count / 32) 32-bit words) set <=> row r may be returned.
+// The row mask of one search, installed before dispatch and cleared after it by every search entry point.
+//  - no filter, no tombstones: null (every row);
+//  - tombstones only: the live mask, with the UNFILTERED dispatch (bound pass and append mode honour the mask);
+//  - a filter (bit r of allow_bits, ceil(count / 32) 32-bit words, set <=> row r may be returned): the filtered dispatch,
+//    with the mask allow AND live when the handle has tombstones.  n_allowed counts the caller's bits; the rows left after
+//    the AND are counted here: on the host for a host mask, by mask_and_popc_kernel for a device mask (one stream
+//    synchronisation, only on handles with tombstones).
 static int set_filter(ragfin* h, const uint32_t* allow_bits, int64_t n_allowed, int bits_on_device, cudaStream_t st) {
-    if (!allow_bits) { h->cur_allow = nullptr; h->cur_allowed = 0; return 0; }
+    h->cur_user_filter = allow_bits != nullptr;
+    if (!allow_bits) {
+        h->cur_allow = h->n_dead > 0 ? h->live_dev : nullptr;
+        h->cur_allowed = h->n_dead > 0 ? h->count - h->n_dead : 0;
+        return 0;
+    }
     if (n_allowed < 0 || n_allowed > h->count) return fail(RAGFIN_EINVAL, "n_allowed %lld outside [0, %lld]", (long long)n_allowed, (long long)h->count);
-    if (bits_on_device) { h->cur_allow = allow_bits; h->cur_allowed = n_allowed; return 0; }
-    const size_t words = (size_t)((h->count + 31) / 32);
+    const size_t words = mask_words(h->count);
     int rc;
+    if (h->n_dead > 0 && bits_on_device) {
+        const size_t cnt_off = (words + 1) / 2 * 2 * sizeof(uint32_t);   // the 8-byte count after the words
+        if ((rc = ensure(h->allow, cnt_off + sizeof(unsigned long long)))) return rc;
+        unsigned long long* dcnt = (unsigned long long*)((char*)h->allow.p + cnt_off);
+        CU_TRY(cudaMemsetAsync(dcnt, 0, sizeof(*dcnt), st));
+        if (words > 0) {
+            const int64_t want = ((int64_t)words + 255) / 256, cap_blocks = (int64_t)h->num_sms * 4;
+            mask_and_popc_kernel<<<(unsigned)(want < cap_blocks ? want : cap_blocks), 256, 0, st>>>(allow_bits, h->live_dev, (uint32_t*)h->allow.p,
+                                                                                                 (int64_t)words, h->count, dcnt);
+            CU_TRY(cudaGetLastError());
+        }
+        unsigned long long live_allowed = 0;
+        CU_TRY(cudaMemcpyAsync(&live_allowed, dcnt, sizeof(live_allowed), cudaMemcpyDeviceToHost, st));
+        CU_TRY(cudaStreamSynchronize(st));
+        h->cur_allow = (const uint32_t*)h->allow.p;
+        h->cur_allowed = (int64_t)live_allowed;
+        return 0;
+    }
+    if (bits_on_device) { h->cur_allow = allow_bits; h->cur_allowed = n_allowed; return 0; }
     if ((rc = ensure(h->allow, (words ? words : 1) * sizeof(uint32_t)))) return rc;
-    CU_TRY(cudaMemcpyAsync(h->allow.p, allow_bits, words * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    if (h->n_dead > 0) {
+        std::vector<uint32_t> m(words);
+        int64_t live_allowed = 0;
+        for (size_t w = 0; w < words; ++w) {
+            uint32_t v = allow_bits[w] & h->live_host[w];
+            if (w + 1 == words && (h->count & 31)) v &= (1u << (h->count & 31)) - 1u;
+            m[w] = v;
+            live_allowed += __builtin_popcount(v);
+        }
+        CU_TRY(cudaMemcpyAsync(h->allow.p, m.data(), words * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaStreamSynchronize(st));   // `m` is pageable and local
+        h->cur_allowed = live_allowed;
+    } else {
+        CU_TRY(cudaMemcpyAsync(h->allow.p, allow_bits, words * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+        h->cur_allowed = n_allowed;
+    }
     h->cur_allow = (const uint32_t*)h->allow.p;
-    h->cur_allowed = n_allowed;
     return 0;
+}
+static void clear_filter(ragfin* h) {
+    h->cur_allow = nullptr;
+    h->cur_allowed = 0;
+    h->cur_user_filter = false;
 }
 
 extern "C" int ragfin_search_filtered(ragfin_t* h, const float* q, int32_t nq, int32_t k, const uint32_t* allow_bits_dev,
@@ -1999,7 +2288,7 @@ extern "C" int ragfin_search_filtered(ragfin_t* h, const float* q, int32_t nq, i
     if ((rc = wait_prev(h, st))) return rc;
     if ((rc = set_filter(h, allow_bits_dev, n_allowed, 1, st))) return rc;
     rc = search_locked(h, q, nq, k, out_ids, out_scores, st);
-    h->cur_allow = nullptr;
+    clear_filter(h);
     if (rc) return rc;
     return mark_done(h, st);
 }
@@ -2021,7 +2310,7 @@ extern "C" int ragfin_search_filtered_host(ragfin_t* h, const float* q_host, int
     if ((rc = set_filter(h, allow_bits_host, n_allowed, 0, st))) return rc;
     CU_TRY(cudaMemcpyAsync(h->stage_q.p, q_host, qb, cudaMemcpyHostToDevice, st));
     rc = search_locked(h, (const float*)h->stage_q.p, nq, k, (int64_t*)h->stage_ids.p, (float*)h->stage_scores.p, st);
-    h->cur_allow = nullptr;
+    clear_filter(h);
     if (rc) return rc;
     CU_TRY(cudaMemcpyAsync(out_ids_host, h->stage_ids.p, ib, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaMemcpyAsync(out_scores_host, h->stage_scores.p, sb, cudaMemcpyDeviceToHost, st));
@@ -2217,6 +2506,7 @@ static int sharded_locked(ragfin* h, ragfin_exchange* x, const float* q_dev, int
                           cudaStream_t st, bool pipelined) {
     if (!x->connected) return fail(RAGFIN_EINVAL, "exchange is not connected");
     if (x->device != h->device) return fail(RAGFIN_EINVAL, "exchange and collection live on different devices");
+    if (h->n_dead > 0) return fail(RAGFIN_EUNSUPPORTED, "sharded search over a shard with deleted rows: compact first");
     if (nq > kFMaxQ || !fused_eligible(h, nq, k))
         return fail(RAGFIN_EUNSUPPORTED, "shape (nq = %d, k = %d) does not take the one-kernel search on this shard", nq, k);
     const size_t record = (size_t)nq * (((size_t)k * 12 + 15) / 16 * 16);
@@ -2271,6 +2561,7 @@ extern "C" int ragfin_search_sharded_host(ragfin_t* h, ragfin_exchange_t* x, con
     const size_t qb = (size_t)nq * h->dim * sizeof(float), ib = (size_t)nq * k * sizeof(int64_t), sb = (size_t)nq * k * sizeof(float);
     if (qb > kHostStageQ || ib + sb > kHostStageOut) return fail(RAGFIN_EUNSUPPORTED, "request too large for the mapped staging");
     if (x->device != h->device) return fail(RAGFIN_EINVAL, "exchange and collection live on different devices");
+    if (h->n_dead > 0) return fail(RAGFIN_EUNSUPPORTED, "sharded search over a shard with deleted rows: compact first");
     if (nq > h->fused_max_nq || !fused_eligible(h, nq, k))
         return fail(RAGFIN_EUNSUPPORTED, "shape (nq = %d, k = %d) does not take the one-kernel search on this shard", nq, k);
     if ((size_t)nq * (((size_t)k * 12 + 15) / 16 * 16) > x->record_max) return fail(RAGFIN_EINVAL, "record exceeds the exchange's %zu bytes", x->record_max);

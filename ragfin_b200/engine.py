@@ -94,6 +94,7 @@ class Index:
         self.dim = int.from_bytes(hd[12:16], "little")
         self.dtype = _DTYPE_NAME[int.from_bytes(hd[20:24], "little")]
         self.capacity = max(int(capacity), int.from_bytes(hd[24:32], "little", signed=True), 1)
+        self._id_base = int.from_bytes(hd[32:40], "little", signed=True)
         return self
 
     def view(self) -> "Index":
@@ -104,6 +105,7 @@ class Index:
         v = Index.__new__(Index)
         v._L, v._h, v._parent = self._L, h, self
         v.dim, v.dtype, v.device, v.capacity = self.dim, self.dtype, self.device, max(len(self), 1)
+        v._id_base = getattr(self, "_id_base", 0)
         return v
 
     # -- lifecycle -------------------------------------------------------------------
@@ -126,6 +128,36 @@ class Index:
 
     num_entities = property(__len__)
 
+    # -- deletion --------------------------------------------------------------------
+    def delete(self, ids) -> int:
+        """Tombstone rows by the ids searches return; no search returns them afterwards.  Duplicates and rows deleted before
+        are allowed; returns the number of rows this call deleted.  An out-of-range id raises and deletes nothing."""
+        a = np.ascontiguousarray(np.asarray(ids, dtype=np.int64).reshape(-1))
+        n = ctypes.c_int64()
+        _lib.check(self._L.ragfin_delete(self._h, a.ctypes.data, a.size, ctypes.byref(n)))
+        return int(n.value)
+
+    @property
+    def live_count(self) -> int:
+        """Rows stored minus rows deleted (`len(self)` keeps counting the rows stored until `compact`)."""
+        n = ctypes.c_int64()
+        _lib.check(self._L.ragfin_live_count(self._h, ctypes.byref(n)))
+        return int(n.value)
+
+    def live_mask(self) -> np.ndarray:
+        """bool [len(self)]: True where the row is live (read from the device mask the kernels use)."""
+        n = len(self)
+        words = np.zeros(max((n + 31) // 32, 1), np.uint32)
+        _lib.check(self._L.ragfin_read_live_mask(self._h, words.ctypes.data))
+        return np.unpackbits(words.view(np.uint8), bitorder="little")[:n].astype(bool)
+
+    def compact(self) -> np.ndarray:
+        """Remove the deleted rows from the device matrix; survivors keep their order and row r becomes the r-th survivor.
+        Returns the surviving OLD ids in ascending order (new id i was old id out[i])."""
+        survivors = np.flatnonzero(self.live_mask()).astype(np.int64) + getattr(self, "_id_base", 0)
+        _lib.check(self._L.ragfin_compact(self._h))
+        return survivors
+
     def reserve(self, capacity: int) -> None:
         """Grow the device matrix to at least `capacity` rows (device-to-device copy of the stored rows, bits unchanged)."""
         _lib.check(self._L.ragfin_reserve(self._h, int(capacity)))
@@ -133,6 +165,7 @@ class Index:
 
     def set_id_base(self, base: int) -> None:
         _lib.check(self._L.ragfin_set_id_base(self._h, int(base)))
+        self._id_base = int(base)
 
     # -- ingest (K1) -----------------------------------------------------------------
     def add(self, rows, stream=None) -> None:

@@ -17,11 +17,14 @@ object the reference uses, so a maintainer switches with
   .search(data, anns_field, param, limit, output_fields=)   retrieve.py:28-34, vector_rag_mcp/main.py:51-57,
                                            "chunking_storing (1).py":411-417, graph_cons.py:275-281
   .query(expr, output_fields=, limit=)     test_vector.py:35-39, graph_cons.py:308-311
+  .delete(expr) / .upsert(data) / .compact()   keeping a corpus current: restated filings, re-cut chunks, withdrawn
+                                           documents (pymilvus 2.3 names; not called by the reference itself)
 
 Hits expose .id, .distance, .score, .entity.<field> and .entity.get(field) exactly as the
 call sites read them (retrieve.py:39-43, graph_cons.py:287-292).  Scalar columns live on the
 host; only the embedding column goes to the GPU.  Row id = insertion ordinal; equal scores
-resolve to the earlier-inserted row (SURVEY.md 8c).
+resolve to the earlier-inserted row (SURVEY.md 8c).  delete() tombstones rows (the engine's search never returns them);
+num_entities keeps counting them, as Milvus does, until compact() removes them and renumbers the survivors.
 
 The engine is exact: index_type / nlist / nprobe are accepted and ignored.
 """
@@ -145,7 +148,8 @@ class _Store:
         self.n_inserted = 0
         self.index = None
         self.metric: Optional[str] = None
-        self.pk_to_row: Dict[Any, int] = {}
+        self.pk_to_row: Dict[Any, int] = {}      # live rows only: a deleted row's key may be inserted again
+        self.dead: set = set()                    # tombstoned rows (mirrors the engine's live mask) until compact()
         # value -> ascending rows, per scalar field, built on the first filter over that field and kept current by
         # insert(): a filtered search costs the matching rows, not a pass over every row of the column
         self.scalar_index: Dict[str, Dict[Any, List[int]]] = {}
@@ -205,17 +209,22 @@ def save_collection(name: str, directory: str) -> None:
         st.flush()
         os.makedirs(directory, exist_ok=True)
         if st.index is not None:
-            st.index.save(os.path.join(directory, name + ".ragfin"))
+            st.index.save(os.path.join(directory, name + ".ragfin"))   # with deletions: a version-2 file carrying the live mask
         fields = [{"name": f.name, "dtype": int(f.dtype), "is_primary": f.is_primary, "params": f.params} for f in st.schema.fields]
         with open(os.path.join(directory, name + ".columns.json"), "w") as f:
             json.dump({"fields": fields, "description": st.schema.description, "columns": st.columns,
-                       "n": st.n_inserted, "storage_dtype": st.storage_dtype, "metric": st.metric}, f)
+                       "n": st.n_inserted, "storage_dtype": st.storage_dtype, "metric": st.metric,
+                       "deleted": sorted(st.dead)}, f)
 
 
-def load_collection(name: str, directory: str, device: int = 0, using: str = "default") -> "Collection":
-    """Re-open a saved collection without re-embedding or re-normalising (results are bit-identical)."""
+def load_collection(name: str, directory: str, device: int = 0, using: str = "default", index_loader=None) -> "Collection":
+    """Re-open a saved collection without re-embedding or re-normalising (results are bit-identical).  Deleted rows stay
+    deleted: the matrix file's live mask is checked against the rows recorded in columns.json.  `index_loader(path, capacity,
+    device)` replaces `Index.load` (tests)."""
     import json, os
-    from .engine import Index
+    if index_loader is None:
+        from .engine import Index
+        index_loader = lambda path, capacity, device: Index.load(path, capacity=capacity, device=device)   # noqa: E731
     with open(os.path.join(directory, name + ".columns.json")) as f:
         meta = json.load(f)
     fields = [FieldSchema(x["name"], DataType(x["dtype"]), is_primary=x["is_primary"], **x["params"]) for x in meta["fields"]]
@@ -226,12 +235,16 @@ def load_collection(name: str, directory: str, device: int = 0, using: str = "de
     st.scalar_index = {}
     st.n_inserted = int(meta["n"])
     st.metric = meta["metric"]
+    st.dead = set(int(r) for r in meta.get("deleted", []))
     pk = st.schema.primary_field.name
-    st.pk_to_row = {v: i for i, v in enumerate(st.columns[pk])}
+    st.pk_to_row = {v: i for i, v in enumerate(st.columns[pk]) if i not in st.dead}
     mpath = os.path.join(directory, name + ".ragfin")
     if st.n_inserted and os.path.exists(mpath):
-        st.index = Index.load(mpath, capacity=max(st.capacity, st.n_inserted), device=device)
+        st.index = index_loader(mpath, max(st.capacity, st.n_inserted), device)
         st.capacity = st.index.capacity
+        dead_in_file = set(np.flatnonzero(~np.asarray(st.index.live_mask(), dtype=bool)).tolist())
+        if dead_in_file != st.dead:
+            raise MilvusException(message=f"{mpath}: its deleted rows ({len(dead_in_file)}) disagree with {name}.columns.json ({len(st.dead)})")
     return col
 
 
@@ -319,9 +332,22 @@ class SearchResult(list):
 
 
 class MutationResult:
-    def __init__(self, primary_keys):
+    def __init__(self, primary_keys, insert_count: Optional[int] = None, delete_count: int = 0, upsert_count: int = 0):
         self.primary_keys = list(primary_keys)
-        self.insert_count = len(self.primary_keys)
+        self.insert_count = len(self.primary_keys) if insert_count is None else insert_count
+        self.delete_count = delete_count
+        self.upsert_count = upsert_count
+
+
+class CompactionState:
+    """What get_compaction_state() reports: compaction here is synchronous, so it has always completed."""
+
+    def __init__(self, completed: int):
+        self.state = "Completed"
+        self.executing_plan_no, self.timeout_plan_no, self.completed_plan_no = 0, 0, completed
+
+    def __repr__(self):
+        return f"CompactionState(state={self.state}, completed_plan_no={self.completed_plan_no})"
 
 
 _STR = r"\"[^\"]*\"|'[^']*'"
@@ -385,6 +411,81 @@ class Collection:
     # -- ingest -----------------------------------------------------------------------
     def insert(self, data, partition_name=None, timeout=None, **kwargs) -> MutationResult:
         st = self._st
+        emb, pks, cols, n = self._parse(data)
+        with st.lock:
+            # ---- validate every column before anything is touched: a Milvus insert is all-or-nothing
+            staged = self._validate(pks, cols)
+            for pk in pks:
+                if pk in st.pk_to_row:
+                    raise MilvusException(message=f"duplicate primary key {pk!r}")
+            self._commit(staged, pks, emb, n)
+        return MutationResult(pks)
+
+    def upsert(self, data, partition_name=None, timeout=None, **kwargs) -> MutationResult:
+        """Insert rows, replacing the live rows whose primary keys they carry: those rows are deleted (tombstoned) and the
+        new ones appended.  Validated in full first; all-or-nothing like insert()."""
+        st = self._st
+        emb, pks, cols, n = self._parse(data)
+        with st.lock:
+            staged = self._validate(pks, cols)
+            st.flush()                                    # the rows being replaced are on the device
+            old = sorted(st.pk_to_row[pk] for pk in pks if pk in st.pk_to_row)
+            if old:
+                st.index.delete(old)
+                st.dead.update(old)
+            self._commit(staged, pks, emb, n)
+        return MutationResult(pks, delete_count=len(old), upsert_count=n)
+
+    def delete(self, expr: str, partition_name=None, timeout=None, **kwargs) -> MutationResult:
+        """Delete the live rows matching `expr` (`pk in [...]` or `field == literal`): no search or query returns them from
+        now on.  num_entities keeps counting them until compact()."""
+        st = self._st
+        if not isinstance(expr, str) or not expr.strip():
+            raise MilvusException(message="delete needs an expression")
+        with st.lock:
+            st.flush()
+            rows = sorted(set(self._rows_matching(expr.strip(), st.n_inserted)) - st.dead)   # a key listed twice: once
+            if rows:
+                st.index.delete(rows)
+                st.dead.update(rows)
+            pk_col = st.columns[st.schema.primary_field.name]
+            pks = [pk_col[r] for r in rows]
+            for pk in pks:
+                st.pk_to_row.pop(pk, None)
+        return MutationResult(pks, insert_count=0, delete_count=len(rows))
+
+    def compact(self, timeout=None, **kwargs) -> None:
+        """Remove deleted rows for good: the engine compacts its matrix (survivors keep their order), the scalar columns,
+        primary-key map and scalar filter index follow with the same old-to-new row map.  Synchronous."""
+        st = self._st
+        with st.lock:
+            st.flush()
+            st.compactions = getattr(st, "compactions", 0) + 1
+            if not st.dead:
+                return
+            survivors = [int(r) for r in st.index.compact()]
+            if len(survivors) != st.n_inserted - len(st.dead):
+                raise MilvusException(message=f"compaction kept {len(survivors)} rows, expected {st.n_inserted - len(st.dead)}")
+            new_of = {r: i for i, r in enumerate(survivors)}
+            st.columns = {name: [c[r] for r in survivors] for name, c in st.columns.items()}   # earlier hits keep the old lists
+            st.scalar_index = {f: {v: [new_of[r] for r in rows if r in new_of] for v, rows in inv.items()}
+                               for f, inv in st.scalar_index.items()}
+            for inv in st.scalar_index.values():
+                for v in [v for v, rows in inv.items() if not rows]:
+                    del inv[v]
+            st.pk_to_row = {v: i for i, v in enumerate(st.columns[st.schema.primary_field.name])}
+            st.n_inserted = len(survivors)
+            st.dead = set()
+
+    def get_compaction_state(self, timeout=None, **kwargs) -> CompactionState:
+        return CompactionState(getattr(self._st, "compactions", 0))
+
+    def wait_for_compaction_completed(self, timeout=None, **kwargs) -> CompactionState:
+        return self.get_compaction_state()
+
+    def _parse(self, data):
+        """Rows of an insert / upsert -> (embeddings, primary keys, columns in schema order, n); shapes checked."""
+        st = self._st
         fields = st.schema.fields
         if isinstance(data, dict):
             data = [data]
@@ -412,39 +513,39 @@ class Collection:
             emb = np.array(emb, dtype=np.float32, order="C")               # a private copy: pending until flush()
             if n and (emb.ndim != 2 or emb.shape != (n, dim)):
                 raise ParamError(message=f"embedding column must be [{n}, {dim}], got {emb.shape}")
-        pk_name = st.schema.primary_field.name
         pks = list(cols[fields.index(st.schema.primary_field)])
-        with st.lock:
-            # ---- validate every column before anything is touched: a Milvus insert is all-or-nothing
-            if len(set(pks)) != len(pks):
-                raise MilvusException(message="duplicate primary keys inside one insert")
-            for pk in pks:
-                if pk in st.pk_to_row:
-                    raise MilvusException(message=f"duplicate primary key {pk!r}")
-            staged = {}
-            for f, c in zip(fields, cols):
-                if f.dtype == DataType.FLOAT_VECTOR:
-                    continue
-                c = list(c)
-                if f.dtype == DataType.VARCHAR and f.max_length:
-                    for v in c:
-                        if len(str(v)) > f.max_length:
-                            raise MilvusException(message=f"length of varchar field {f.name} exceeds max length {f.max_length}")
-                staged[f.name] = c
-            # ---- commit
-            for name, c in staged.items():
-                st.columns[name].extend(c)
-                inv = st.scalar_index.get(name)
-                if inv is not None:
-                    for j, v in enumerate(c):
-                        inv.setdefault(v, []).append(st.n_inserted + j)
-            for j, pk in enumerate(pks):
-                st.pk_to_row[pk] = st.n_inserted + j
-            if n:
-                st.pending.append(emb)
-            st.n_inserted += n
-        assert pk_name in st.columns
-        return MutationResult(pks)
+        return emb, pks, cols, n
+
+    def _validate(self, pks, cols) -> dict:
+        """Checks that need no collection state beyond the schema; returns the scalar columns to append."""
+        st = self._st
+        if len(set(pks)) != len(pks):
+            raise MilvusException(message="duplicate primary keys inside one insert")
+        staged = {}
+        for f, c in zip(st.schema.fields, cols):
+            if f.dtype == DataType.FLOAT_VECTOR:
+                continue
+            c = list(c)
+            if f.dtype == DataType.VARCHAR and f.max_length:
+                for v in c:
+                    if len(str(v)) > f.max_length:
+                        raise MilvusException(message=f"length of varchar field {f.name} exceeds max length {f.max_length}")
+            staged[f.name] = c
+        return staged
+
+    def _commit(self, staged: dict, pks, emb, n: int) -> None:
+        st = self._st
+        for name, c in staged.items():
+            st.columns[name].extend(c)
+            inv = st.scalar_index.get(name)
+            if inv is not None:
+                for j, v in enumerate(c):
+                    inv.setdefault(v, []).append(st.n_inserted + j)
+        for j, pk in enumerate(pks):
+            st.pk_to_row[pk] = st.n_inserted + j
+        if n:
+            st.pending.append(emb)
+        st.n_inserted += n
 
     def flush(self, timeout=None, **kwargs):
         self._st.flush()
@@ -496,6 +597,7 @@ class Collection:
                 for _ in range(q.shape[0]):
                     res.append(Hits())
                 return res
+            # deleted rows: the engine holds their tombstones and never returns them, filtered or not
             if expr and expr.strip():     # scalar filter -> row bitmask consumed inside the top-k epilogues
                 allow = np.zeros(st.n_inserted, dtype=bool)
                 allow[self._rows_matching(expr.strip(), st.n_inserted)] = True
@@ -554,6 +656,8 @@ class Collection:
                 rows = list(range(n))
             else:
                 rows = self._rows_matching(expr, n)
+            if st.dead:
+                rows = [r for r in rows if r not in st.dead]
             rows = rows[offset:]
             if limit is not None:
                 rows = rows[:int(limit)]
