@@ -47,8 +47,9 @@ enum {
 };
 
 /* ABI version of this header; bumped on any signature change.  Version 4 also carries the row-deletion entry points
- * (ragfin_delete, ragfin_live_count, ragfin_read_live_mask, ragfin_compact): they were added without changing any existing
- * signature, so the version stays 4. */
+ * (ragfin_delete, ragfin_live_count, ragfin_read_live_mask, ragfin_compact) and the range-search entry points
+ * (ragfin_search_range, ragfin_search_range_host): they were added without changing any existing signature, so the version
+ * stays 4. */
 #define RAGFIN_ABI_VERSION 4
 int ragfin_abi_version(void);
 
@@ -143,6 +144,33 @@ int ragfin_search_filtered(ragfin_t* h, const float* q, int32_t nq, int32_t k, c
 int ragfin_search_filtered_host(ragfin_t* h, const float* q_host, int32_t nq, int32_t k,
                                 const uint32_t* allow_bits_host, int64_t n_allowed, int64_t* out_ids_host,
                                 float* out_scores_host);
+
+/* Range search (pymilvus `search(..., {"metric_type": "COSINE", "params": {"radius": r, "range_filter": f}}, limit=k)`):
+ * the k best rows whose score s satisfies  radius < s <= range_filter,  ordered by (score desc, id asc); slots past the
+ * number of rows in the window hold id -1 and score -inf.  s is the exact fp32 score every search returns and the compares
+ * are fp32 compares on it: a row scoring exactly `radius` is excluded, one scoring exactly `range_filter` is included.
+ * radius = -INFINITY is no floor, range_filter = +INFINITY no ceiling; with both open the call IS ragfin_search[_host]
+ * (or _filtered[_host] when allow_bits is given), bit for bit.  allow_bits (may be NULL) and n_allowed mean what they mean for
+ * ragfin_search_filtered[_host]; tombstoned rows are never returned.  RAGFIN_EINVAL for a NULL range, a NaN bound or
+ * range_filter <= radius.
+ * Dispatch (DESIGN.md 7c): the tensor-core append path with the window applied in its bound pass and epilogues when the
+ * batch would take it (k <= 256, no filter, a corpus of >= 4 k tiles), else the large-k pipeline with the window; never the
+ * one-kernel search.  ragfin_last_search_stats reports path 1 (append) or 2 (large-k) and queries_rescanned.  Works on views;
+ * the sharded entry points have no range form.
+ * The window travels by pointer to a ragfin_range in host memory, read before the call returns: every parameter of this
+ * ABI is a pointer or a 32- / 64-bit integer, the rule tests/test_abi_cpu.py checks every ctypes binding against.  FFI
+ * callers pass the address of two consecutive fp32 values {radius, range_filter} (ctypes: (c_float * 2)(r, f)).  A NULL
+ * range is RAGFIN_EINVAL.  The window is validated before the handle, so a bad window fails the same way with any handle.
+ * _range: device buffers and bitmask, asynchronous on `stream` (the large-k route synchronises it); _range_host: host
+ * buffers and bitmask, synchronous. */
+typedef struct {
+    float radius;         /* exclusive floor; -INFINITY = none */
+    float range_filter;   /* inclusive ceiling; +INFINITY = none */
+} ragfin_range;
+int ragfin_search_range(ragfin_t* h, const float* q, int32_t nq, int32_t k, const ragfin_range* range,
+                        const uint32_t* allow_bits_dev, int64_t n_allowed, int64_t* out_ids, float* out_scores, void* stream);
+int ragfin_search_range_host(ragfin_t* h, const float* q_host, int32_t nq, int32_t k, const ragfin_range* range,
+                             const uint32_t* allow_bits_host, int64_t n_allowed, int64_t* out_ids_host, float* out_scores_host);
 
 /* Cross-shard reduce: merge `parts` exact hit lists per query (device memory; -1 ids are
  * padding) into the global top-k, ordered by (score desc, id asc).  Hit j of part p for query q

@@ -13,7 +13,7 @@ namespace rfk {
 template <int DT>
 __global__ void __launch_bounds__(256) score_all_kernel(const void* __restrict__ data, int64_t n_rows, int ld,
                                                         const float* __restrict__ qhat, float* __restrict__ scores,
-                                                        const uint32_t* __restrict__ allow) {
+                                                        const uint32_t* __restrict__ allow, float radius, float range_filter) {
     const int lane = threadIdx.x & 31;
     const typename Store<DT>::T* base = reinterpret_cast<const typename Store<DT>::T*>(data);
     const int64_t stride = (int64_t)gridDim.x * (blockDim.x >> 5);
@@ -23,7 +23,8 @@ __global__ void __launch_bounds__(256) score_all_kernel(const void* __restrict__
             continue;
         }
         const double s = canonical_dot_row<DT>(base + (size_t)r * ld, qhat, ld, lane);
-        if (lane == 0) scores[r] = (float)s + 0.0f;
+        const float s32 = (float)s + 0.0f;
+        if (lane == 0) scores[r] = s32 > radius && s32 <= range_filter ? s32 : -INFINITY;   // outside a range search's window: as filtered
     }
 }
 
@@ -91,9 +92,10 @@ __global__ void __launch_bounds__(256) rank_sort_kernel(const u64* __restrict__ 
         for (int j = 0; j < lim; ++j) rank += tile[j] > mine;
         __syncthreads();
     }
-    if (i < m && rank < k) {
-        out_ids[rank] = id_base + (int64_t)key_row(mine);
-        out_scores[rank] = key_score(mine);
+    if (i < m && rank < k) {   // a -inf key is a row outside a range search's window: padding
+        const bool hit = key_score(mine) > -INFINITY;
+        out_ids[rank] = hit ? id_base + (int64_t)key_row(mine) : -1;
+        out_scores[rank] = hit ? key_score(mine) : -INFINITY;
     }
     if (i >= m && i < k) {   // slots past the number of rows
         out_ids[i] = -1;
@@ -160,7 +162,8 @@ __device__ __forceinline__ void bk_resolve(const BkState* st, int p, int want0, 
 
 // pass p (0..3): histogram of byte (3 - p) of the ordered scores whose higher bytes equal the prefix decided so far
 __global__ void __launch_bounds__(256) bk_hist_kernel(const float* __restrict__ approx, int64_t n, int pass, int keff,
-                                                      BkState* __restrict__ states, const uint32_t* __restrict__ allow) {
+                                                      BkState* __restrict__ states, const uint32_t* __restrict__ allow,
+                                                      const float* __restrict__ wcap) {
     __shared__ uint32_t h[256];
     __shared__ uint32_t s_prefix;
     const int q = blockIdx.y, lane = threadIdx.x & 31;
@@ -178,8 +181,10 @@ __global__ void __launch_bounds__(256) bk_hist_kernel(const float* __restrict__ 
     const uint32_t prefix = pass > 0 ? s_prefix : 0u;
     const int shift = 24 - 8 * pass;
     const float* sc = approx + (size_t)q * n;
+    const float cap = wcap != nullptr ? wcap[q] : INFINITY;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         if (allow != nullptr && !row_allowed(allow, i)) continue;
+        if (sc[i] > cap) continue;   // range search: only rows certainly at or below range_filter count toward T
         const uint32_t o = float_to_ordered(sc[i] + 0.0f);
         if (pass == 0 || (o >> (shift + 8)) == (prefix >> (shift + 8))) atomicAdd(&h[(o >> shift) & 255u], 1u);
     }
@@ -190,8 +195,9 @@ __global__ void __launch_bounds__(256) bk_hist_kernel(const float* __restrict__ 
 // rows whose approximate score reaches T - 2 eps -> cand_rows[q][0 .. n_cand)
 __global__ void __launch_bounds__(256) bk_compact_kernel(const float* __restrict__ approx, int64_t n, int keff, float eps_const,
                                                          const float* __restrict__ eps_q, BkState* __restrict__ states,
-                                                         uint32_t* __restrict__ cand_rows, int cmax, const uint32_t* __restrict__ allow) {
-    __shared__ float s_cut;
+                                                         uint32_t* __restrict__ cand_rows, int cmax, const uint32_t* __restrict__ allow,
+                                                         const float* __restrict__ wlo, const float* __restrict__ whi) {
+    __shared__ float s_cut, s_hi;
     const int q = blockIdx.y, lane = threadIdx.x & 31;
     BkState* st = states + q;
     if (threadIdx.x < 32) {
@@ -199,16 +205,21 @@ __global__ void __launch_bounds__(256) bk_compact_kernel(const float* __restrict
         bk_resolve(st, 3, keff, &t_ord, &rem, lane);
         if (lane == 0) {
             const float e = eps_const + (eps_q ? eps_q[q] : 0.0f);
-            s_cut = keff > 0 ? __fsub_rd(__fsub_rd(ordered_to_float(t_ord), __fmul_ru(2.0f, e)), 2.384185791015625e-07f) : INFINITY;
+            float cut = keff > 0 ? __fsub_rd(__fsub_rd(ordered_to_float(t_ord), __fmul_ru(2.0f, e)), 2.384185791015625e-07f) : INFINITY;
+            // range search: rem == 0 <=> fewer than keff rows lie certainly below the ceiling, so T is no bound and the floor
+            // alone cuts; otherwise the floor may still be the tighter cut
+            if (wlo != nullptr && keff > 0) cut = rem == 0 ? wlo[q] : fmaxf(cut, wlo[q]);
+            s_cut = cut;
+            s_hi = whi != nullptr ? whi[q] : INFINITY;
         }
     }
     __syncthreads();
-    const float cut = s_cut;
+    const float cut = s_cut, hi = s_hi;
     const float* sc = approx + (size_t)q * n;
     uint32_t* out = cand_rows + (size_t)q * cmax;
     for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
         if (allow != nullptr && !row_allowed(allow, i)) continue;
-        if (sc[i] >= cut) {
+        if (sc[i] >= cut && sc[i] <= hi) {
             const uint32_t pos = atomicAdd(&st->n_cand, 1u);
             if (pos < (uint32_t)cmax) out[pos] = (uint32_t)i;
             else st->overflow = 1u;
@@ -220,7 +231,7 @@ __global__ void __launch_bounds__(256) bk_compact_kernel(const float* __restrict
 template <int DT>
 __global__ void __launch_bounds__(256) bk_rescore_kernel(const void* __restrict__ data, int ld, const float* __restrict__ qhat,
                                                          const BkState* __restrict__ states, const uint32_t* __restrict__ cand_rows,
-                                                         int cmax, u64* __restrict__ keys) {
+                                                         int cmax, u64* __restrict__ keys, float radius, float range_filter) {
     const int q = blockIdx.y, lane = threadIdx.x & 31;
     const int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
     if (c >= cmax) return;
@@ -229,7 +240,8 @@ __global__ void __launch_bounds__(256) bk_rescore_kernel(const void* __restrict_
     if ((uint32_t)c < nc) {
         const uint32_t row = cand_rows[(size_t)q * cmax + c];
         const double s = canonical_dot_row<DT>(reinterpret_cast<const typename Store<DT>::T*>(data) + (size_t)row * ld, qhat + (size_t)q * ld, ld, lane);
-        key = make_key((float)s + 0.0f, row);
+        const float s32 = (float)s + 0.0f;
+        key = make_key(s32 > radius && s32 <= range_filter ? s32 : -INFINITY, row);   // outside a range search's window: -inf
     }
     if (lane == 0) keys[(size_t)q * cmax + c] = key;
 }
@@ -253,11 +265,12 @@ __global__ void __launch_bounds__(256) bk_rank_sort_kernel(const u64* __restrict
         for (int j = 0; j < lim; ++j) rank += tile[j] > mine;
         __syncthreads();
     }
-    if (i < m && rank < keff) {
-        oid[rank] = id_base + (int64_t)key_row(mine);
-        osc[rank] = key_score(mine);
+    if (i < m && rank < keff) {   // a -inf key is a row outside a range search's window: padding
+        const bool hit = key_score(mine) > -INFINITY;
+        oid[rank] = hit ? id_base + (int64_t)key_row(mine) : -1;
+        osc[rank] = hit ? key_score(mine) : -INFINITY;
     }
-    if (i >= keff && i < k) {   // slots past the number of rows that exist
+    if (i >= (m < keff ? m : keff) && i < k) {   // slots past the number of rows that exist (a window may hold fewer than keff)
         oid[i] = -1;
         osc[i] = -INFINITY;
     }

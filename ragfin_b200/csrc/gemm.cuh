@@ -189,6 +189,8 @@ struct GemmArgs {
     const float* thr;       // MODE 3: [nq] collection threshold (a row is appended when its score >= thr[q])
     uint32_t* cnt;          // MODE 3: [nq] rows appended so far (may exceed cap: overflow, the query goes to tier 2)
     int cap;                // MODE 3: capacity of one query's append buffer, cand = [nq][cap]
+    const float* wcap;      // range search (window_words_kernel), else null.  MODE 2: [nq] sample rows above it are excluded
+    const float* whi;       //   MODE 3: [nq] a row above it never takes a slot
     int dbg;                // timing experiments only (RAGFIN_GEMM_DEBUG): 1 skip epilogue filter, 2 skip MMAs, 4 skip A loads, 8 skip B loads
 };
 
@@ -375,6 +377,8 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             st.allow = a.allow;
             float tile_mx = -INFINITY;   // MODE 2: maximum over the block's sample tiles
             const float thr3 = (MODE == 3 && q < a.nq) ? __ldg(a.thr + qc) : INFINITY;   // padding lanes never append
+            const float hi3 = (MODE == 3 && a.whi != nullptr) ? __ldg(a.whi + qc) : INFINITY;
+            const float cap2 = (MODE == 2 && a.wcap != nullptr) ? __ldg(a.wcap + qc) : INFINITY;
             uint32_t* const cnt3 = MODE == 3 ? a.cnt + qc : nullptr;
             u64* const buf3 = MODE == 3 ? a.cand + (size_t)qc * a.cap : nullptr;
             uint32_t g_next = MODE != 0 ? 0u : __ldcg(a.gtau + qc);
@@ -420,6 +424,12 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                                 if (!((w >> j) & 1u)) v[j] = 0x7FC00000u;
                         }
                     }
+                    if (MODE == 2 && cap2 < INFINITY) {
+                        // range search: a sample row that may score above range_filter must not raise a block maximum
+#pragma unroll
+                        for (int j = 0; j < 32; ++j)
+                            if (__uint_as_float(v[j]) > cap2) v[j] = 0x7FC00000u;
+                    }
                     // maxima of the four groups of 8 columns, then of the chunk: one compare in the common case
                     float gmx[4];
 #pragma unroll
@@ -441,8 +451,8 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                                         const float sc = __uint_as_float(v[g * 8 + j]);
                                         const long long row = trow + c * 32 + g * 8 + j;
                                         // one atomic per appended row (measured: reserving slots in blocks is no faster); a
-                                        // masked (tombstoned) row never takes a slot
-                                        if (sc >= thr3 && (a.allow == nullptr || row_allowed(a.allow, row))) {
+                                        // masked (tombstoned) row, or one above a range search's ceiling, never takes a slot
+                                        if (sc >= thr3 && sc <= hi3 && (a.allow == nullptr || row_allowed(a.allow, row))) {
                                             const uint32_t pos = atomicAdd(cnt3, 1u);
                                             if (pos < (uint32_t)a.cap) buf3[pos] = make_key(sc + 0.0f, (uint32_t)row);
                                         }
@@ -493,7 +503,7 @@ gemm_topk_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
 __global__ void __launch_bounds__(256) bound_select_kernel(const float* __restrict__ bmax, int nb, int rank,
                                                            uint32_t* __restrict__ gtau, float* __restrict__ thr,
                                                            uint32_t* __restrict__ cnt, float eps_const,
-                                                           const float* __restrict__ eps_q) {
+                                                           const float* __restrict__ eps_q, const float* __restrict__ wlo) {
     __shared__ uint32_t v[1024];
     __shared__ uint32_t hist[256];
     __shared__ uint32_t s3[3];
@@ -506,9 +516,26 @@ __global__ void __launch_bounds__(256) bound_select_kernel(const float* __restri
         if (gtau != nullptr) gtau[q] = mine;
         if (thr != nullptr) {
             const float e = eps_const + (eps_q ? eps_q[q] : 0.0f);
-            thr[q] = __fsub_rd(__fsub_rd(ordered_to_float(mine), __fmul_ru(2.0f, e)), 2.384185791015625e-07f);
+            const float t = __fsub_rd(__fsub_rd(ordered_to_float(mine), __fmul_ru(2.0f, e)), 2.384185791015625e-07f);
+            thr[q] = wlo != nullptr ? fmaxf(t, wlo[q]) : t;   // range search: no row below the floor is worth a slot
         }
     }
+}
+
+// ---- per-query words of a range search (DESIGN.md 7c), radius < score <= range_filter.  e = eps_const + eps_q[q] + 2^-22
+// bounds |approx - exact| with the fp32 rounding of the exact score to spare (directed rounding keeps every word safe):
+//   lo  = radius - e        every row of the window has approx >= lo
+//   hi  = range_filter + e  every row of the window has approx <= hi
+//   cap = range_filter - e  a row with approx <= cap is certainly at or below range_filter
+// Open bounds stay infinite.  Layout: w[0 .. nq) lo, w[nq .. 2 nq) hi, w[2 nq .. 3 nq) cap. ---------------------------------
+__global__ void __launch_bounds__(128) window_words_kernel(int nq, float radius, float range_filter, float eps_const,
+                                                           const float* __restrict__ eps_q, float* __restrict__ w) {
+    const int q = blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= nq) return;
+    const float e = __fadd_ru(__fadd_ru(eps_const, eps_q ? eps_q[q] : 0.0f), 2.384185791015625e-07f);
+    w[q] = __fsub_rd(radius, e);
+    w[nq + q] = __fadd_ru(range_filter, e);
+    w[2 * nq + q] = __fsub_rd(range_filter, e);
 }
 
 // ---- query preparation for the tensor-core path, one launch: normalise (bit-identical to ingest_kernel<0>), zero-pad

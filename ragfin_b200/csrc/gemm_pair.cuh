@@ -198,6 +198,7 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
             const int q = qt * kGM + m;
             const int qc = q < a.nq ? q : a.nq - 1;
             const float thr3 = (MODE == 3 && q < a.nq) ? __ldg(a.thr + qc) : INFINITY;   // padding lanes never append
+            const float hi3 = (MODE == 3 && a.whi != nullptr) ? __ldg(a.whi + qc) : INFINITY;
             uint32_t* const cnt3 = MODE == 3 ? a.cnt + qc : nullptr;
             u64* const buf3 = MODE == 3 ? a.cand + (size_t)qc * a.cap : nullptr;
             for (int t = 0; t < ntiles; ++t) {
@@ -243,7 +244,8 @@ gemm_pair_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant_
                                 for (int j = 0; j < 8; ++j) {
                                     const float sc = __uint_as_float(v[g * 8 + j]);
                                     const long long row = trow + c * 32 + g * 8 + j;
-                                    if (sc >= thr3 && (a.allow == nullptr || row_allowed(a.allow, row))) {   // tombstones never take a slot
+                                    // tombstones, and rows above a range search's ceiling, never take a slot
+                                    if (sc >= thr3 && sc <= hi3 && (a.allow == nullptr || row_allowed(a.allow, row))) {
                                         const uint32_t pos = atomicAdd(cnt3, 1u);
                                         if (pos < (uint32_t)a.cap) buf3[pos] = make_key(sc + 0.0f, (uint32_t)row);
                                     }

@@ -54,6 +54,7 @@ struct RowsArgs {
     uint32_t* cnt;          // [nq]
     int cap;
     const uint32_t* allow;  // row mask (tombstones; bit set = row may be appended), or null
+    const float* whi;       // range search: [nq] a row above it never takes a slot (window_words_kernel), else null
 };
 
 __device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&r)[16]) {
@@ -190,7 +191,8 @@ gemm_rows_kernel(const __grid_constant__ CUtensorMap tmQ, const __grid_constant_
 #pragma unroll
                         for (int j = 0; j < kRN; ++j) {
                             const float sc = (__uint_as_float(v[0][j]) + __uint_as_float(v[1][j])) + (__uint_as_float(v[2][j]) + __uint_as_float(v[3][j]));
-                            if (sc >= thr[j] && (a.allow == nullptr || row_allowed(a.allow, row))) {   // tombstones never take a slot
+                            // tombstones, and rows above a range search's ceiling, never take a slot
+                            if (sc >= thr[j] && (a.whi == nullptr || sc <= __ldg(a.whi + j)) && (a.allow == nullptr || row_allowed(a.allow, row))) {
                                 const uint32_t pos = atomicAdd(a.cnt + j, 1u);
                                 if (pos < (uint32_t)a.cap) a.cand[(size_t)j * a.cap + pos] = make_key(sc + 0.0f, (uint32_t)row);
                             }

@@ -564,6 +564,10 @@ __device__ __forceinline__ uint32_t block_kth_largest(F hi_of, int m, uint32_t w
 //   3. recompute those rows canonically in fp64, order by the exact key, emit k.
 // Unconditionally exact - there is no certificate to fail; only an overflowing buffer (m > cap, or more than
 // kAppendRescore rows above the cut: massive duplication) sends the query to tier 2.
+// Range search (radius < score <= range_filter, DESIGN.md 7c; open bounds are infinite): the buffer holds the rows with
+// approx in [max(thr, lo), hi] and may hold fewer than k.  T is selected among the rows CERTAINLY in the window
+// (radius + e < approx <= range_filter - e); if fewer than k are, every buffer row is rescored.  The exact fp32 window is
+// applied to the rescored scores before the top k are taken.
 // ---------------------------------------------------------------------------------
 constexpr int kAppendRescore = 2048;   // most rows one query may rescore exactly
 constexpr int kFaThreads = 256;
@@ -574,38 +578,72 @@ finalize_append_kernel(const u64* __restrict__ buf, const uint32_t* __restrict__
                        const void* __restrict__ data, int dt, int64_t n_rows, int ld, const float* __restrict__ qhat,
                        float eps_const, const float* __restrict__ eps_q, int k, int64_t id_base,
                        int64_t* __restrict__ out_ids, float* __restrict__ out_scores, int* __restrict__ flags,
-                       int* __restrict__ flag_count) {
+                       int* __restrict__ flag_count, float radius, float range_filter) {
     __shared__ __align__(16) u64 sel[kAppendRescore];
     __shared__ uint32_t hist[256];
     __shared__ uint32_t s3[3];
-    __shared__ int s_c2;
+    __shared__ int s_c2, s_sure;
     const int q = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const bool window = radius > -INFINITY || range_filter < INFINITY;
     const uint32_t m32 = cnt[q];
     const int keff = (int64_t)k < n_rows ? k : (int)n_rows;
-    const bool overflow = m32 > (uint32_t)cap || (int)m32 < keff;   // fewer than k rows cannot happen with a valid bound
+    // fewer than k rows cannot happen with a valid bound - except in a range search, whose window may hold fewer
+    const bool overflow = m32 > (uint32_t)cap || (!window && (int)m32 < keff);
     const int m = overflow ? 0 : (int)m32;
     const u64* in = buf + (size_t)q * cap;
-    if (tid == 0) s_c2 = 0;
+    const float eps = eps_const + (eps_q ? eps_q[q] : 0.0f);
+    if (tid == 0) { s_c2 = 0; s_sure = 0; }
     __syncthreads();
+    if (window && !overflow && m > 0) {   // block-uniform
+        const float ew = __fadd_ru(eps, 2.384185791015625e-07f);
+        const float sure_lo = __fadd_ru(radius, ew), sure_hi = __fsub_rd(range_filter, ew);
+        int c = 0;
+        for (int i = tid; i < m; i += kFaThreads) { const float s = key_score(in[i]); c += s > sure_lo && s <= sure_hi; }
+        c = __reduce_add_sync(kFull, c);
+        if (lane == 0 && c) atomicAdd(&s_sure, c);
+        __syncthreads();
+        if (s_sure < keff) {   // T would not be a bound: every buffer row goes to the exact rescore
+            for (int i = tid; i < m; i += kFaThreads) {
+                const int pos = atomicAdd(&s_c2, 1);
+                if (pos < kAppendRescore) sel[pos] = in[i];
+            }
+            __syncthreads();
+        } else {
+            const uint32_t t_ord = block_kth_largest([&](int i) {
+                const float s = key_score(in[i]);
+                return s > sure_lo && s <= sure_hi ? (uint32_t)(in[i] >> 32) : 0u;
+            }, m, (uint32_t)keff, hist, s3);
+            const float cut = __fsub_rd(__fsub_rd(ordered_to_float(t_ord), __fmul_ru(2.0f, eps)), 2.384185791015625e-07f);
+            for (int i = tid; i < m; i += kFaThreads) {
+                const u64 key = in[i];
+                if (key_score(key) >= cut) {
+                    const int pos = atomicAdd(&s_c2, 1);
+                    if (pos < kAppendRescore) sel[pos] = key;
+                }
+            }
+            __syncthreads();
+        }
+    }
     if (overflow || keff == 0) {   // block-uniform
         if (tid == 0) { flags[q] = overflow ? 1 : 0; if (overflow) atomicAdd(flag_count, 1); }
         if (!overflow)
             for (int i = tid; i < k; i += kFaThreads) { out_ids[(size_t)q * k + i] = -1; out_scores[(size_t)q * k + i] = -INFINITY; }
         return;
     }
-    // ---- 1. T = keff-th largest approximate score, as an ordered uint ----
-    const uint32_t t_ord = block_kth_largest([&](int i) { return (uint32_t)(in[i] >> 32); }, m, (uint32_t)keff, hist, s3);
-    // ---- 2. gather the rows above the cut ----
-    const float eps = eps_const + (eps_q ? eps_q[q] : 0.0f);
-    const float cut = __fsub_rd(__fsub_rd(ordered_to_float(t_ord), __fmul_ru(2.0f, eps)), 2.384185791015625e-07f);
-    for (int i = tid; i < m; i += kFaThreads) {
-        const u64 key = in[i];
-        if (key_score(key) >= cut) {
-            const int pos = atomicAdd(&s_c2, 1);
-            if (pos < kAppendRescore) sel[pos] = key;
+    if (!window) {
+        // ---- 1. T = keff-th largest approximate score, as an ordered uint ----
+        const uint32_t t_ord = block_kth_largest([&](int i) { return (uint32_t)(in[i] >> 32); }, m, (uint32_t)keff, hist, s3);
+        // ---- 2. gather the rows above the cut ----
+        const float cut = __fsub_rd(__fsub_rd(ordered_to_float(t_ord), __fmul_ru(2.0f, eps)), 2.384185791015625e-07f);
+        for (int i = tid; i < m; i += kFaThreads) {
+            const u64 key = in[i];
+            if (key_score(key) >= cut) {
+                const int pos = atomicAdd(&s_c2, 1);
+                if (pos < kAppendRescore) sel[pos] = key;
+            }
         }
+        __syncthreads();
     }
-    __syncthreads();
     const int c2 = s_c2;
     if (c2 > kAppendRescore) {   // block-uniform
         if (tid == 0) { flags[q] = 1; atomicAdd(flag_count, 1); }
@@ -620,7 +658,8 @@ finalize_append_kernel(const u64* __restrict__ buf, const uint32_t* __restrict__
         else if (dt == 1) sc = rescore_row<1>(data, row, ld, qv, lane);
         else sc = rescore_row<2>(data, row, ld, qv, lane);
         __syncwarp();
-        if (lane == 0) sel[c] = make_key((float)sc + 0.0f, row);
+        const float s = (float)sc + 0.0f;
+        if (lane == 0) sel[c] = s > radius && s <= range_filter ? make_key(s, row) : 0ull;   // the exact window
     }
     int P2 = 32;
     while (P2 < c2) P2 <<= 1;
@@ -644,7 +683,7 @@ template <int DT>
 __global__ void __launch_bounds__(kScanThreads)
 exact_scan_kernel(const void* __restrict__ data, int64_t n_rows, int ld, const float* __restrict__ qhat,
                   int nq, const int* __restrict__ flags, const int* __restrict__ flag_count, int kpe,
-                  u64* __restrict__ cand_e, const uint32_t* __restrict__ allow) {
+                  u64* __restrict__ cand_e, const uint32_t* __restrict__ allow, float radius, float range_filter) {
     if (*flag_count == 0) return;
     extern __shared__ __align__(16) u64 lists[];  // [kScanWarps][kpe]
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -659,7 +698,9 @@ exact_scan_kernel(const void* __restrict__ data, int64_t n_rows, int ld, const f
         for (int64_t r = (int64_t)blockIdx.x * kScanWarps + warp; r < n_rows; r += stride) {
             if (allow != nullptr && !row_allowed(allow, r)) continue;
             const double s = canonical_dot_row<DT>(base + (size_t)r * ld, qv, ld, lane);
-            const u64 key = make_key((float)s + 0.0f, (uint32_t)r);
+            const float s32 = (float)s + 0.0f;
+            if (!(s32 > radius && s32 <= range_filter)) continue;   // outside a range search's window (open bounds are infinite)
+            const u64 key = make_key(s32, (uint32_t)r);
             if (key > mine[kpe - 1]) warp_list_insert(mine, kpe, key, lane);
         }
         __syncthreads();

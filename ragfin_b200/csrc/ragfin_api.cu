@@ -70,7 +70,7 @@ struct ragfin {
     bool is_view = false;  // ragfin_create_view: `data` and `sweep_data` belong to another handle (read-only here, never freed here)
     std::mutex mu;
     // workspace (grow-only)
-    Buf qhat, q16, eps_q, gtau, bmax, acnt, athr, allow, bk_scores, bk_state, bk_keys, bk_rows, cand, cand_e, flags, stage_q, stage_ids, stage_scores, add_stage;
+    Buf qhat, q16, eps_q, gtau, bmax, acnt, athr, awin, allow, bk_scores, bk_state, bk_keys, bk_rows, cand, cand_e, flags, stage_q, stage_ids, stage_scores, add_stage;
     int gemm_min_nq = 3;      // query batches of at least this many rows take the tcgen05 path (1-2: HBM-bound scan) ...
     int gemm_min_nq_large = 1;   // ... except on corpora of >= kSweepBytes, where the TMA-fed sweep wins from 1 query
     int gemm_cluster = 0;     // 0 = choose by batch size; 1, 2 or 4 = force
@@ -79,6 +79,8 @@ struct ragfin {
     const uint32_t* cur_allow = nullptr;   // row mask of the search in flight (device bitmask: filter, tombstones or both), else null
     int64_t cur_allowed = 0;               // rows it allows
     bool cur_user_filter = false;          // the caller passed a filter: filtered dispatch (no bound pass, no append mode)
+    bool cur_window = false;               // the search in flight is a range search (ragfin_search_range): hits must satisfy
+    float cur_radius = -INFINITY, cur_range_filter = INFINITY;   //   cur_radius < score <= cur_range_filter (DESIGN.md 7c)
     // Tombstones (ragfin_delete).  live_host mirrors the device mask live_dev bit for bit: ceil(capacity / 32) words in the
     // allow_bits layout, bit set = row live; rows at or past `count` are live (rows added later are).  Both stay empty until
     // the first delete, and a handle with n_dead == 0 passes a null mask to every kernel.
@@ -305,7 +307,7 @@ extern "C" void ragfin_destroy(ragfin_t* h) {
     if (!h) return;
     DeviceGuard g(h->device);
     (void)cudaDeviceSynchronize();
-    Buf* bufs[] = {&h->qhat, &h->q16, &h->eps_q, &h->gtau, &h->bmax, &h->acnt, &h->athr, &h->allow, &h->bk_scores, &h->bk_state, &h->bk_keys, &h->bk_rows, &h->cand, &h->cand_e, &h->flags, &h->stage_q, &h->stage_ids, &h->stage_scores, &h->add_stage, &h->fctl, &h->fcand, &h->fqn, &h->fflags};
+    Buf* bufs[] = {&h->qhat, &h->q16, &h->eps_q, &h->gtau, &h->bmax, &h->acnt, &h->athr, &h->awin, &h->allow, &h->bk_scores, &h->bk_state, &h->bk_keys, &h->bk_rows, &h->cand, &h->cand_e, &h->flags, &h->stage_q, &h->stage_ids, &h->stage_scores, &h->add_stage, &h->fctl, &h->fcand, &h->fqn, &h->fflags};
     for (Buf* b : bufs)
         if (b->p) cudaFree(b->p);
     if (h->sweep_data && has_copy(h) && !h->is_view) cudaFree(h->sweep_data);
@@ -1163,6 +1165,7 @@ static int run_gemm(ragfin* h, int nb, int k, int kp, int* G, bool* appended, fl
     a.dump = dump;
     a.bound_tps = 0; a.bound_tiles = 0; a.bound_stride = 0;
     a.thr = (const float*)h->athr.p; a.cnt = (uint32_t*)h->acnt.p; a.cap = kAppendCap;
+    a.wcap = nullptr; a.whi = nullptr;
     a.dbg = 0;
 #ifdef RAGFIN_TIMING_EXPERIMENTS   // scripts/gemm_dbg_sweep.py: switch pipeline stages off (INVALID results, timing only)
     { const char* e = getenv("RAGFIN_GEMM_DEBUG"); a.dbg = e ? atoi(e) : 0; }
@@ -1176,6 +1179,16 @@ static int run_gemm(ragfin* h, int nb, int k, int kp, int* G, bool* appended, fl
     at[0].val.clusterDim.x = C; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
     cfg.attrs = at; cfg.numAttrs = 1;
 
+    const float* wlo = nullptr;
+    if (append && h->cur_window) {   // range search: per-query window words (window_words_kernel) for the three passes below
+        if ((rc = ensure(h->awin, (size_t)3 * nb * sizeof(float)))) return rc;
+        float* w = (float*)h->awin.p;
+        RF_LAUNCH(window_words_kernel, (nb + 127) / 128, 128, 0, st, nb, h->cur_radius, h->cur_range_filter, eps_approx(h),
+                                                                   (const float*)h->eps_q.p, w);
+        CU_TRY(cudaGetLastError());
+        h->stats.launches++;
+        wlo = w; a.whi = w + nb; a.wcap = w + 2 * nb;
+    }
     if (bound) {
         const int groups = (p.QT + C - 1) / C;
         const int clusters = C > 1 ? resident_clusters : h->num_sms;
@@ -1193,7 +1206,7 @@ static int run_gemm(ragfin* h, int nb, int k, int kp, int* G, bool* appended, fl
         CU_TRY(cudaLaunchKernelEx(&cfg, bfn, tmA, tmB, b));
         RF_LAUNCH(bound_select_kernel, nb, 256, 0, st, (const float*)h->bmax.p, nblk, rank, append ? nullptr : (uint32_t*)h->gtau.p,
                                                  append ? (float*)h->athr.p : nullptr, append ? (uint32_t*)h->acnt.p : nullptr,
-                                                 eps_approx(h), (const float*)h->eps_q.p);
+                                                 eps_approx(h), (const float*)h->eps_q.p, wlo);
         CU_TRY(cudaGetLastError());
         h->stats.launches += 2;
     }
@@ -1203,7 +1216,7 @@ static int run_gemm(ragfin* h, int nb, int k, int kp, int* G, bool* appended, fl
         r.idesc = make_idesc_n(h->sweep_dt == 0 ? 2 : h->sweep_dt == 1 ? 1 : 0, kRN);
         r.num_kblocks = a.num_kblocks; r.k_elems = a.k_elems; r.nq = nb; r.n_rows = n;
         r.S = p.S; r.rows_per_slice = p.rows_per_slice; r.stages = rows_stages(a.num_kblocks);
-        r.cand = a.cand; r.thr = a.thr; r.cnt = a.cnt; r.cap = a.cap; r.allow = a.allow;
+        r.cand = a.cand; r.thr = a.thr; r.cnt = a.cnt; r.cap = a.cap; r.allow = a.allow; r.whi = a.whi;
         CUtensorMap tmQ;
         if ((rc = cached_map(h, &tmQ, h->sweep_dt, a_base, nb_pad, h->ld, kRN))) return rc;
         typedef void (*rows_fn)(const CUtensorMap, const CUtensorMap, const RowsArgs);
@@ -1521,9 +1534,9 @@ static int search_bigk(ragfin* h, const float* q_dev, int nq, int k, int64_t* ou
     for (int q = 0; q < nq; ++q) {
         if ((rc = launch_ingest<false>(0, q_dev + (size_t)q * h->dim, 0, 0, 0, 0, 1, h->dim, h->ld, qhat, h->num_sms, st))) return rc;
         switch (h->dtype) {
-            case 0: score_all_kernel<0><<<blocks, 256, 0, st>>>(h->data, n, h->ld, qhat, scores, h->cur_allow); break;
-            case 1: score_all_kernel<1><<<blocks, 256, 0, st>>>(h->data, n, h->ld, qhat, scores, h->cur_allow); break;
-            default: score_all_kernel<2><<<blocks, 256, 0, st>>>(h->data, n, h->ld, qhat, scores, h->cur_allow); break;
+            case 0: score_all_kernel<0><<<blocks, 256, 0, st>>>(h->data, n, h->ld, qhat, scores, h->cur_allow, h->cur_radius, h->cur_range_filter); break;
+            case 1: score_all_kernel<1><<<blocks, 256, 0, st>>>(h->data, n, h->ld, qhat, scores, h->cur_allow, h->cur_radius, h->cur_range_filter); break;
+            default: score_all_kernel<2><<<blocks, 256, 0, st>>>(h->data, n, h->ld, qhat, scores, h->cur_allow, h->cur_radius, h->cur_range_filter); break;
         }
         CU_TRY(cudaGetLastError());
         RadixState init;
@@ -1569,6 +1582,7 @@ static int search_bigk_batched(ragfin* h, const float* q_dev, int nq, int k, int
     if ((rc = ensure(h->bk_state, (size_t)nq * sizeof(BkState)))) return rc;
     if ((rc = ensure(h->bk_rows, (size_t)kBigChunk * cmax * sizeof(uint32_t)))) return rc;
     if ((rc = ensure(h->bk_keys, (size_t)kBigChunk * cmax * sizeof(u64)))) return rc;
+    if (h->cur_window && (rc = ensure(h->awin, (size_t)3 * kBigChunk * sizeof(float)))) return rc;
     float* qhat = (float*)h->qhat.p;
     float* scores = (float*)h->bk_scores.p;
     BkState* states = (BkState*)h->bk_state.p;
@@ -1589,15 +1603,24 @@ static int search_bigk_batched(ragfin* h, const float* q_dev, int nq, int k, int
         int G = 0;
         bool ap = false;
         if ((rc = run_gemm(h, nb, 10, 32, &G, &ap, scores, st, true))) return rc;        // MODE 1: approx[q][row]
+        const float* w = nullptr;   // range search: per-query window words {lo, hi, cap}
+        if (h->cur_window) {
+            w = (const float*)h->awin.p;
+            RF_LAUNCH(window_words_kernel, (nb + 127) / 128, 128, 0, st, nb, h->cur_radius, h->cur_range_filter, eps,
+                                                                       (const float*)h->eps_q.p, (float*)h->awin.p);
+            CU_TRY(cudaGetLastError());
+            h->stats.launches++;
+        }
         BkState* stq = states + q0;
         for (int pass = 0; pass < 4; ++pass)
-            bk_hist_kernel<<<dim3(blocks, nb), 256, 0, st>>>(scores, n, pass, keff, stq, h->cur_allow);
-        bk_compact_kernel<<<dim3(blocks, nb), 256, 0, st>>>(scores, n, keff, eps, (const float*)h->eps_q.p, stq, (uint32_t*)h->bk_rows.p, cmax, h->cur_allow);
+            bk_hist_kernel<<<dim3(blocks, nb), 256, 0, st>>>(scores, n, pass, keff, stq, h->cur_allow, w ? w + 2 * nb : nullptr);
+        bk_compact_kernel<<<dim3(blocks, nb), 256, 0, st>>>(scores, n, keff, eps, (const float*)h->eps_q.p, stq, (uint32_t*)h->bk_rows.p, cmax, h->cur_allow,
+                                                            w, w ? w + nb : nullptr);
         const dim3 rg((cmax + 7) / 8, nb);
         switch (h->dtype) {
-            case 0: bk_rescore_kernel<0><<<rg, 256, 0, st>>>(h->data, h->ld, qhat, stq, (const uint32_t*)h->bk_rows.p, cmax, (u64*)h->bk_keys.p); break;
-            case 1: bk_rescore_kernel<1><<<rg, 256, 0, st>>>(h->data, h->ld, qhat, stq, (const uint32_t*)h->bk_rows.p, cmax, (u64*)h->bk_keys.p); break;
-            default: bk_rescore_kernel<2><<<rg, 256, 0, st>>>(h->data, h->ld, qhat, stq, (const uint32_t*)h->bk_rows.p, cmax, (u64*)h->bk_keys.p); break;
+            case 0: bk_rescore_kernel<0><<<rg, 256, 0, st>>>(h->data, h->ld, qhat, stq, (const uint32_t*)h->bk_rows.p, cmax, (u64*)h->bk_keys.p, h->cur_radius, h->cur_range_filter); break;
+            case 1: bk_rescore_kernel<1><<<rg, 256, 0, st>>>(h->data, h->ld, qhat, stq, (const uint32_t*)h->bk_rows.p, cmax, (u64*)h->bk_keys.p, h->cur_radius, h->cur_range_filter); break;
+            default: bk_rescore_kernel<2><<<rg, 256, 0, st>>>(h->data, h->ld, qhat, stq, (const uint32_t*)h->bk_rows.p, cmax, (u64*)h->bk_keys.p, h->cur_radius, h->cur_range_filter); break;
         }
         const int span = cmax > k ? cmax : k;
         bk_rank_sort_kernel<<<dim3((span + 255) / 256, nb), 256, 0, st>>>((const u64*)h->bk_keys.p, stq, cmax, k, keff, h->id_base,
@@ -1635,13 +1658,19 @@ static int search_locked(ragfin* h, const float* q_dev, int nq, int k, int64_t* 
     const int steps = round_steps((nvec + 31) / 32);
     const int64_t n_eff = h->cur_allow ? h->cur_allowed : n;   // rows a hit may come from
     if ((rc = ensure(h->flags, (size_t)(kMaxQueryBatch + 1) * sizeof(int)))) return rc;
-    if (nq <= h->fused_max_nq && fused_eligible(h, nq, k)) {   // the one-kernel search (sweep_fused.cuh): prep, sweep, finalize, exact fallback
+    const int min_nq_all = (size_t)n * h->ld * esize(h->dtype) >= kSweepBytes ? h->gemm_min_nq_large : h->gemm_min_nq;
+    const bool ap = append_eligible(h, k) && nq >= min_nq_all;   // tensor-core append mode: no K' lists needed
+    if (h->cur_window && !ap) {
+        // Range search (DESIGN.md 7c): the append path when the batch would take it, else the large-k pipeline with the
+        // window, which serves every k, filter and corpus size.  Never the one-kernel search.
+        if (h->use_bigk_batched && n >= 4096 && gemm_rows_ok(h)) return search_bigk_batched(h, q_dev, nq, k, out_ids, out_scores, st);
+        return search_bigk(h, q_dev, nq, k, out_ids, out_scores, st);
+    }
+    if (!h->cur_window && nq <= h->fused_max_nq && fused_eligible(h, nq, k)) {   // the one-kernel search (sweep_fused.cuh): prep, sweep, finalize, exact fallback
         return run_fused(h, q_dev, nq, k, n_eff, out_ids, out_scores, st, h->cur_pipelined);
     }
     int kp = cand_per_query(k);
     if (kp == 0 && n <= 256) kp = 256;   // every row is a candidate: any k (graph_cons.py:279 asks limit=1000 of 16 rows)
-    const int min_nq_all = (size_t)n * h->ld * esize(h->dtype) >= kSweepBytes ? h->gemm_min_nq_large : h->gemm_min_nq;
-    const bool ap = append_eligible(h, k) && nq >= min_nq_all;   // tensor-core append mode: no K' lists needed
     if (kp == 0 && !ap) {
         // k beyond the list / append modes: batched dump + select on corpora worth a tensor-core sweep, else one query at a time
         if (h->use_bigk_batched && n >= 4096 && gemm_rows_ok(h)) return search_bigk_batched(h, q_dev, nq, k, out_ids, out_scores, st);
@@ -1660,7 +1689,8 @@ static int search_locked(ragfin* h, const float* q_dev, int nq, int k, int64_t* 
         const int nb4 = (nb + 3) / 4 * 4;
         const size_t corpus_bytes = (size_t)h->count * h->ld * esize(h->dtype);
         const int min_nq = corpus_bytes >= kSweepBytes ? h->gemm_min_nq_large : h->gemm_min_nq;
-        const bool via_gemm = nb >= min_nq && (gemm_supported(h, kp) || (ap && h->count > 0));
+        // a range search's last chunk takes the append path whatever its size (its window is not applied elsewhere)
+        const bool via_gemm = (h->cur_window || nb >= min_nq) && (gemm_supported(h, kp) || (ap && h->count > 0));
         const int nbq = via_gemm ? (nb + kGM - 1) / kGM * kGM : nb4;   // tensor-core path: whole 128-query tiles
         // 1. normalise the queries (same kernel as ingest, fp32 out, stride ld); pad with zero rows
         if ((rc = ensure(h->qhat, (size_t)nbq * h->ld * sizeof(float)))) return rc;
@@ -1755,7 +1785,7 @@ static int search_locked(ragfin* h, const float* q_dev, int nq, int k, int64_t* 
         if (appended) {
             RF_LAUNCH(finalize_append_kernel, nb, kFaThreads, 0, st,
                 (const u64*)h->cand.p, (const uint32_t*)h->acnt.p, kAppendCap, h->data, h->dtype, n_eff, h->ld, qhat, eps, eps_q, k,
-                h->id_base, out_ids + (size_t)q0 * k, out_scores + (size_t)q0 * k, flags, flag_count);
+                h->id_base, out_ids + (size_t)q0 * k, out_scores + (size_t)q0 * k, flags, flag_count, h->cur_radius, h->cur_range_filter);
             CU_TRY(cudaGetLastError());
             h->stats.launches++;
         } else {
@@ -1771,9 +1801,12 @@ static int search_locked(ragfin* h, const float* q_dev, int nq, int k, int64_t* 
             if ((rc = ensure(h->cand_e, (size_t)nb * Ge * kpe * sizeof(u64)))) return rc;
             const size_t smem = (size_t)kScanWarps * kpe * sizeof(u64);
             switch (h->dtype) {
-                case 0: RF_LAUNCH(exact_scan_kernel<0>, Ge, kScanThreads, smem, st, h->data, n, h->ld, qhat, nb, flags, flag_count, kpe, (u64*)h->cand_e.p, h->cur_allow); break;
-                case 1: RF_LAUNCH(exact_scan_kernel<1>, Ge, kScanThreads, smem, st, h->data, n, h->ld, qhat, nb, flags, flag_count, kpe, (u64*)h->cand_e.p, h->cur_allow); break;
-                default: RF_LAUNCH(exact_scan_kernel<2>, Ge, kScanThreads, smem, st, h->data, n, h->ld, qhat, nb, flags, flag_count, kpe, (u64*)h->cand_e.p, h->cur_allow); break;
+                case 0: RF_LAUNCH(exact_scan_kernel<0>, Ge, kScanThreads, smem, st, h->data, n, h->ld, qhat, nb, flags, flag_count, kpe, (u64*)h->cand_e.p, h->cur_allow,
+                                          h->cur_radius, h->cur_range_filter); break;
+                case 1: RF_LAUNCH(exact_scan_kernel<1>, Ge, kScanThreads, smem, st, h->data, n, h->ld, qhat, nb, flags, flag_count, kpe, (u64*)h->cand_e.p, h->cur_allow,
+                                          h->cur_radius, h->cur_range_filter); break;
+                default: RF_LAUNCH(exact_scan_kernel<2>, Ge, kScanThreads, smem, st, h->data, n, h->ld, qhat, nb, flags, flag_count, kpe, (u64*)h->cand_e.p, h->cur_allow,
+                                          h->cur_radius, h->cur_range_filter); break;
             }
             CU_TRY(cudaGetLastError());
             RF_LAUNCH(finalize_kernel<true>, nb, kFinThreads, 0, st, (const u64*)h->cand_e.p, Ge, kpe, h->data, h->dtype, n_eff, 1, 1, nullptr,
@@ -2186,7 +2219,7 @@ static int search_host_locked(ragfin* h, const float* q_host, int nq, int k, int
         }
         void* dptr = nullptr;
         if (h->hstage && cudaHostGetDevicePointer(&dptr, h->hstage, 0) == cudaSuccess) {
-            if (nq <= h->fused_max_nq && fused_eligible(h, nq, k)) {
+            if (!h->cur_window && nq <= h->fused_max_nq && fused_eligible(h, nq, k)) {
                 if ((rc = fused_host_call(h, nullptr, q_host, nq, k, out_ids_host, out_scores_host, st))) return rc;
                 return mark_done(h, st);
             }
@@ -2316,6 +2349,73 @@ extern "C" int ragfin_search_filtered_host(ragfin_t* h, const float* q_host, int
     CU_TRY(cudaMemcpyAsync(out_scores_host, h->stage_scores.p, sb, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaStreamSynchronize(st));
     return mark_done(h, st);
+}
+
+// Range search (DESIGN.md 7c): the k best rows with radius < score <= range_filter.  Both bounds open: the plain entry
+// points themselves.  Otherwise the window is installed next to the row mask for the one dispatch (search_locked).
+// The window is checked first: it needs neither a handle nor a device.
+static int check_range_args(const ragfin* h, const float* q, int nq, int k, const ragfin_range* range,
+                            const void* out_ids, const void* out_scores) {
+    if (!range) return fail(RAGFIN_EINVAL, "NULL range");
+    const float radius = range->radius, range_filter = range->range_filter;
+    if (radius != radius || range_filter != range_filter) return fail(RAGFIN_EINVAL, "radius and range_filter must not be NaN");
+    if (!(range_filter > radius)) return fail(RAGFIN_EINVAL, "range_filter (%g) must be greater than radius (%g)", (double)range_filter, (double)radius);
+    if (!h) return fail(RAGFIN_EINVAL, "NULL handle");
+    if (nq < 0 || (nq > 0 && (!q || !out_ids || !out_scores))) return fail(RAGFIN_EINVAL, "NULL buffer");
+    if (k < 1 || k > 16384) return fail(RAGFIN_EINVAL, "k = %d outside [1, 16384]", k);
+    return 0;
+}
+static bool range_open(float radius, float range_filter) { return radius == -INFINITY && range_filter == INFINITY; }
+static void set_window(ragfin* h, float radius, float range_filter) {
+    h->cur_window = true; h->cur_radius = radius; h->cur_range_filter = range_filter;
+}
+static void clear_window(ragfin* h) {
+    h->cur_window = false; h->cur_radius = -INFINITY; h->cur_range_filter = INFINITY;
+}
+
+extern "C" int ragfin_search_range(ragfin_t* h, const float* q, int32_t nq, int32_t k, const ragfin_range* range,
+                                   const uint32_t* allow_bits_dev, int64_t n_allowed, int64_t* out_ids, float* out_scores,
+                                   void* stream) {
+    int rc;
+    if ((rc = check_range_args(h, q, nq, k, range, out_ids, out_scores))) return rc;
+    const float radius = range->radius, range_filter = range->range_filter;
+    if (range_open(radius, range_filter))
+        return allow_bits_dev ? ragfin_search_filtered(h, q, nq, k, allow_bits_dev, n_allowed, out_ids, out_scores, stream)
+                              : ragfin_search(h, q, nq, k, out_ids, out_scores, stream);
+    if (nq == 0) return RAGFIN_OK;
+    std::lock_guard<std::mutex> lk(h->mu);
+    DeviceGuard g(h->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    if ((rc = wait_prev(h, st))) return rc;
+    if ((rc = set_filter(h, allow_bits_dev, n_allowed, 1, st))) return rc;
+    set_window(h, radius, range_filter);
+    rc = search_locked(h, q, nq, k, out_ids, out_scores, st);
+    clear_window(h);
+    clear_filter(h);
+    if (rc) return rc;
+    return mark_done(h, st);
+}
+
+extern "C" int ragfin_search_range_host(ragfin_t* h, const float* q_host, int32_t nq, int32_t k, const ragfin_range* range,
+                                        const uint32_t* allow_bits_host, int64_t n_allowed, int64_t* out_ids_host,
+                                        float* out_scores_host) {
+    int rc;
+    if ((rc = check_range_args(h, q_host, nq, k, range, out_ids_host, out_scores_host))) return rc;
+    const float radius = range->radius, range_filter = range->range_filter;
+    if (range_open(radius, range_filter))
+        return allow_bits_host ? ragfin_search_filtered_host(h, q_host, nq, k, allow_bits_host, n_allowed, out_ids_host, out_scores_host)
+                               : ragfin_search_host(h, q_host, nq, k, out_ids_host, out_scores_host);
+    if (nq == 0) return RAGFIN_OK;
+    std::lock_guard<std::mutex> lk(h->mu);
+    DeviceGuard g(h->device);
+    cudaStream_t st = 0;
+    if ((rc = wait_prev(h, st))) return rc;
+    if ((rc = set_filter(h, allow_bits_host, n_allowed, 0, st))) return rc;
+    set_window(h, radius, range_filter);
+    rc = search_host_locked(h, q_host, nq, k, out_ids_host, out_scores_host, st);
+    clear_window(h);
+    clear_filter(h);
+    return rc;
 }
 
 extern "C" int ragfin_last_search_stats(ragfin_t* h, ragfin_search_stats* out) {

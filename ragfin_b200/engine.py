@@ -46,6 +46,14 @@ def _host_queries(queries, dim: int):
     return q, q.ctypes.data, q.shape[0]
 
 
+def _window(radius, range_filter):
+    """Range-search bounds as the C ABI takes them (a ragfin_range): fp32 (round to nearest even), None = open (-inf / +inf).
+    The library rejects a NaN bound and range_filter <= radius."""
+    lo = -np.inf if radius is None else float(np.float32(radius))
+    hi = np.inf if range_filter is None else float(np.float32(range_filter))
+    return (ctypes.c_float * 2)(lo, hi)
+
+
 def _host_out(out, nq: int, k: int, np_dtype, what: str):
     """Caller-owned result buffer (numpy array or torch CPU tensor, C-contiguous [nq, k]) or a fresh numpy one -> (obj, address)."""
     if out is None:
@@ -237,32 +245,47 @@ class Index:
         return k
 
     def search(self, queries, k: int, out_ids: Optional[np.ndarray] = None,
-               out_scores: Optional[np.ndarray] = None, allow: Optional[np.ndarray] = None) -> Tuple[np.ndarray, np.ndarray]:
+               out_scores: Optional[np.ndarray] = None, allow: Optional[np.ndarray] = None,
+               radius: Optional[float] = None, range_filter: Optional[float] = None) -> Tuple[np.ndarray, np.ndarray]:
         """Host path: queries numpy / list / torch CPU tensor [nq, dim] -> (ids int64 [nq, k], scores fp32 [nq, k]).
         Hits are in descending score, ties to the lower id; slots past min(k, N) hold (-1, -inf).
         `out_ids` / `out_scores` may be caller-owned (e.g. pinned) C-contiguous numpy arrays or torch CPU tensors; they are
         returned as passed, fresh numpy arrays otherwise.
-        `allow`: optional bool array [N]; only rows with allow[r] may be returned (scalar-filtered search)."""
+        `allow`: optional bool array [N]; only rows with allow[r] may be returned (scalar-filtered search).
+        `radius` / `range_filter`: range search, only rows with radius < score <= range_filter (both rounded to fp32 with
+        np.float32; None = open) may be returned, and slots past the rows in the window hold (-1, -inf)."""
         k = self._check_k(k)
         q, qp, nq = _host_queries(queries, self.dim)
         ids, ip = _host_out(out_ids, nq, k, np.int64, "out_ids")
         scores, sp = _host_out(out_scores, nq, k, np.float32, "out_scores")
+        if radius is not None or range_filter is not None:
+            window = _window(radius, range_filter)
+            packed, n_allowed = self._pack_allow(allow) if allow is not None else (None, 0)
+            _lib.check(self._L.ragfin_search_range_host(self._h, qp, nq, k, window,
+                                                        packed.ctypes.data if packed is not None else None, n_allowed, ip, sp))
+            return ids, scores
         if allow is not None:
-            mask = np.ascontiguousarray(allow, dtype=bool)
-            if mask.shape != (len(self),):
-                raise ValueError(f"allow must be a bool array of shape [{len(self)}], got {mask.shape}")
-            packed = np.packbits(mask, bitorder="little")
-            packed = np.concatenate([packed, np.zeros((-len(packed)) % 4, np.uint8)]).view(np.uint32)
-            if packed.size == 0:
-                packed = np.zeros(1, np.uint32)
-            _lib.check(self._L.ragfin_search_filtered_host(self._h, qp, nq, k, packed.ctypes.data, int(mask.sum()), ip, sp))
+            packed, n_allowed = self._pack_allow(allow)
+            _lib.check(self._L.ragfin_search_filtered_host(self._h, qp, nq, k, packed.ctypes.data, n_allowed, ip, sp))
             return ids, scores
         _lib.check(self._L.ragfin_search_host(self._h, qp, nq, k, ip, sp))
         return ids, scores
 
-    def search_device(self, queries, k: int, out_ids=None, out_scores=None, stream=None):
+    def _pack_allow(self, allow):
+        """bool [N] -> (ceil(N / 32) little-endian uint32 words, number of set bits), the allow_bits layout."""
+        mask = np.ascontiguousarray(allow, dtype=bool)
+        if mask.shape != (len(self),):
+            raise ValueError(f"allow must be a bool array of shape [{len(self)}], got {mask.shape}")
+        packed = np.packbits(mask, bitorder="little")
+        packed = np.concatenate([packed, np.zeros((-len(packed)) % 4, np.uint8)]).view(np.uint32)
+        if packed.size == 0:
+            packed = np.zeros(1, np.uint32)
+        return packed, int(mask.sum())
+
+    def search_device(self, queries, k: int, out_ids=None, out_scores=None, stream=None,
+                      radius: Optional[float] = None, range_filter: Optional[float] = None):
         """Device path: `queries` is a torch CUDA fp32 tensor [nq, dim]; returns torch CUDA tensors.
-        Asynchronous on the given (default: current) stream."""
+        Asynchronous on the given (default: current) stream.  `radius` / `range_filter`: range search, as in search()."""
         import torch
         k = self._check_k(k)
         if not queries.is_cuda or queries.dtype != torch.float32 or queries.dim() != 2 or queries.shape[1] != self.dim:
@@ -274,6 +297,10 @@ class Index:
         if out_scores is None:
             out_scores = torch.empty((nq, k), dtype=torch.float32, device=queries.device)
         with torch.cuda.device(self.device):
+            if radius is not None or range_filter is not None:
+                _lib.check(self._L.ragfin_search_range(self._h, queries.data_ptr(), nq, k, _window(radius, range_filter), None, 0,
+                                                       out_ids.data_ptr(), out_scores.data_ptr(), _stream_ptr(stream)))
+                return out_ids, out_scores
             _lib.check(self._L.ragfin_search(self._h, queries.data_ptr(), nq, k, out_ids.data_ptr(),
                                              out_scores.data_ptr(), _stream_ptr(stream)))
         return out_ids, out_scores

@@ -16,6 +16,9 @@ object the reference uses, so a maintainer switches with
   .num_entities                            vector_rag_mcp/main.py:113,120,164, test_vector.py:29
   .search(data, anns_field, param, limit, output_fields=)   retrieve.py:28-34, vector_rag_mcp/main.py:51-57,
                                            "chunking_storing (1).py":411-417, graph_cons.py:275-281
+  .search(..., {"metric_type": "COSINE", "params": {"radius": r, "range_filter": f}}, limit)   range search: at most
+                                           `limit` hits with r < score <= f, best first (pymilvus 2.3; both bounds are
+                                           rounded to fp32 and compared with the fp32 scores; range_filter needs radius)
   .query(expr, output_fields=, limit=)     test_vector.py:35-39, graph_cons.py:308-311
   .delete(expr) / .upsert(data) / .compact()   keeping a corpus current: restated filings, re-cut chunks, withdrawn
                                            documents (pymilvus 2.3 names; not called by the reference itself)
@@ -26,7 +29,8 @@ host; only the embedding column goes to the GPU.  Row id = insertion ordinal; eq
 resolve to the earlier-inserted row (SURVEY.md 8c).  delete() tombstones rows (the engine's search never returns them);
 num_entities keeps counting them, as Milvus does, until compact() removes them and renumbers the survivors.
 
-The engine is exact: index_type / nlist / nprobe are accepted and ignored.
+The engine is exact: index_type / nlist / nprobe (and the other keys of a search's "params" but radius and range_filter)
+are accepted and ignored.
 """
 from __future__ import annotations
 
@@ -371,6 +375,39 @@ def _parse_literal(tok: str):
             raise MilvusException(message=f"cannot parse expression: invalid literal {tok!r}") from None
 
 
+def _range_window(params: dict) -> Dict[str, float]:
+    """radius / range_filter of a search's "params" as Index.search keywords ({} for a plain search).  Both must be real
+    numbers (bool is refused), neither NaN, and range_filter > radius after rounding to fp32, the precision the engine
+    compares in; a radius of +inf or a range_filter of -inf after that rounding leaves no score to return and is refused;
+    range_filter without radius is refused rather than dropped, as Milvus would."""
+    if not isinstance(params, dict):
+        raise MilvusException(message=f"search params must be a dict, got {type(params).__name__}")
+    if "radius" not in params:
+        if "range_filter" in params:
+            raise MilvusException(message="range_filter needs radius: a range search is radius < score <= range_filter")
+        return {}
+    out = {}
+    for key in ("radius", "range_filter"):
+        if key not in params:
+            continue
+        v = params[key]
+        if isinstance(v, (bool, np.bool_)) or not isinstance(v, (int, float, np.integer, np.floating)):
+            raise MilvusException(message=f"{key} must be a number, got {v!r}")
+        with np.errstate(over="ignore"):      # a finite value beyond the fp32 range rounds to +-inf, checked below
+            v32 = np.float32(v)
+        if np.isnan(v32):
+            raise MilvusException(message=f"{key} must not be NaN")
+        out[key] = float(v32)
+    if out["radius"] == np.inf:
+        raise MilvusException(message=f"radius must be below +inf in fp32, got {params['radius']!r}: no score exceeds it")
+    if out.get("range_filter", 0.0) == -np.inf:
+        raise MilvusException(message=f"range_filter must be above -inf in fp32, got {params['range_filter']!r}")
+    if "range_filter" in out and not out["range_filter"] > out["radius"]:
+        raise MilvusException(message=f"range_filter must be greater than radius for COSINE: radius {params['radius']!r}, "
+                                      f"range_filter {params['range_filter']!r}")
+    return out
+
+
 class Collection:
     def __init__(self, name: str, schema: Optional[CollectionSchema] = None, using: str = "default", **kwargs):
         self.name, self._using = name, using
@@ -585,6 +622,7 @@ class Collection:
         for f in out_fields:
             if f not in st.columns:
                 raise MilvusException(message=f"field {f} not exist")
+        window = _range_window((param or {}).get("params") or {})
         q = np.ascontiguousarray(data, dtype=np.float32)
         if q.ndim == 1:
             q = q[None, :]
@@ -601,14 +639,14 @@ class Collection:
             if expr and expr.strip():     # scalar filter -> row bitmask consumed inside the top-k epilogues
                 allow = np.zeros(st.n_inserted, dtype=bool)
                 allow[self._rows_matching(expr.strip(), st.n_inserted)] = True
-                ids, scores = st.index.search(q, int(limit), allow=allow)
+                ids, scores = st.index.search(q, int(limit), allow=allow, **window)
             else:
-                ids, scores = st.index.search(q, int(limit))
+                ids, scores = st.index.search(q, int(limit), **window)
             pk_col = st.columns[st.schema.primary_field.name]
             cols, names = st.columns, tuple(out_fields)
             for qi in range(q.shape[0]):
                 rows_q, sc_q = ids[qi].tolist(), scores[qi].tolist()      # Python ints / floats (fp32 scores widened exactly)
-                if rows_q and rows_q[-1] < 0:                            # padded: fewer than `limit` rows (or allowed rows)
+                if rows_q and rows_q[-1] < 0:                            # padded: fewer than `limit` rows (allowed, in the window)
                     rows_q = rows_q[:next(i for i, r in enumerate(rows_q) if r < 0)]
                 if round_decimal >= 0:
                     sc_q = [round(s_, round_decimal) for s_ in sc_q]
