@@ -68,6 +68,8 @@ int ragfin_create(ragfin_t** out, int32_t dim, int32_t dtype, int64_t capacity_r
 /* Append n fp32 rows ([n, dim] row-major; host memory, or device memory when
  * src_is_device != 0).  Each row is L2-normalised (fp64 canonical sum, see DESIGN.md) and
  * rounded once to the storage type by the ingest kernel.  Row ids are insertion ordinals.
+ * A row with any NaN or +-Inf component is stored as the zero row (every element 0: it scores exactly 0 against every query);
+ * nothing is validated or reported, so a device source stays asynchronous.
  * Replaces: collection.insert([... embeddings ...]); flush(); load()
  * - "chunking_storing (1).py":383-396. */
 int ragfin_add(ragfin_t* h, const float* rows, int64_t n, int32_t src_is_device, void* stream);
@@ -124,6 +126,8 @@ int ragfin_set_id_base(ragfin_t* h, int64_t id_base);
  * in descending score, ties broken by lower id; slots beyond min(k, N) hold id -1 and
  * score -inf.  Asynchronous on `stream` for k <= 224; larger k (up to 16384, the Milvus limit) takes
  * an exact radix-select path that synchronises the stream once per query.
+ * A query with any NaN or +-Inf component is searched as the zero query: every row scores exactly 0 (this holds for every
+ * search entry point).
  * Replaces: Collection.search(q, "embedding", {"metric_type":"COSINE"}, k)
  * - vector_rag_mcp/main.py:51-57 (and the three other call sites listed above). */
 int ragfin_search(ragfin_t* h, const float* q, int32_t nq, int32_t k, int64_t* out_ids,

@@ -15,6 +15,7 @@
  * Canonical arithmetic: 32 strided fp64 partial sums, butterfly fold 16/8/4/2/1,
  * one rounding to fp32, "+ 0.0f" to canonicalise -0.  Build WITHOUT -ffast-math.
  */
+#include <float.h>
 #include <math.h>
 #include <pthread.h>
 #include <stdint.h>
@@ -117,9 +118,12 @@ static void norm_range(int64_t lo, int64_t hi, void* p) {
     for (int64_t r = lo; r < hi; ++r) {
         const float* xr = c->x + r * c->dim;
         double n2 = canonical_dot(xr, xr, c->dim);
-        double inv = n2 > 0.0 ? 1.0 / sqrt(n2) : 0.0;
-        for (int32_t j = 0; j < c->dim; ++j)
-            c->out[r * c->dim + j] = round_storage((float)((double)xr[j] * inv), c->dtype);
+        /* a zero row and a non-finite one (n2 NaN or +inf) get inv = 0; the NaN of Inf * 0 or NaN * 0 is stored as +0 */
+        double inv = n2 > 0.0 && n2 <= DBL_MAX ? 1.0 / sqrt(n2) : 0.0;
+        for (int32_t j = 0; j < c->dim; ++j) {
+            float y = (float)((double)xr[j] * inv);
+            c->out[r * c->dim + j] = round_storage(y == y ? y : 0.0f, c->dtype);
+        }
     }
 }
 void oracle_normalize_rows(const float* x, int64_t n, int32_t dim, int32_t dtype, float* out) {

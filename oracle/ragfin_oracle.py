@@ -38,6 +38,8 @@ the CUDA rescore kernel) so that "bit-exact" is a property and not luck:
     holds the same value.
   * Row normalisation: n2 = canonical sum of squares; stored = RNE_storage(
     RNE_fp32(double(x) * (1 / sqrt(n2)))); a zero row stays zero (score 0).
+    A row with any NaN or +-Inf component (n2 NaN or +inf) is stored as a zero
+    row: inv = 0, and the NaN of Inf * 0 or NaN * 0 becomes +0.
     bf16 / fp16 storage rounds the fp32 value once more (RNE).
   * Query normalisation: same, to fp32.
   * score = RNE_fp32(canonical_dot(stored_row, q_hat)) + 0.0f   (kills -0).
@@ -178,9 +180,10 @@ def normalize_rows(x32: np.ndarray, dtype: str = "f32") -> np.ndarray:
     if x32.ndim == 1:
         x32 = x32[None, :]
     n2 = canonical_sumsq(x32)
-    with np.errstate(divide="ignore", invalid="ignore"):
-        inv = np.where(n2 > 0.0, 1.0 / np.sqrt(n2), 0.0)
-    y = (x32.astype(np.float64) * inv[:, None]).astype(np.float32)
+    with np.errstate(divide="ignore", invalid="ignore", over="ignore"):
+        inv = np.where((n2 > 0.0) & np.isfinite(n2), 1.0 / np.sqrt(n2), 0.0)
+        y = (x32.astype(np.float64) * inv[:, None]).astype(np.float32)
+    y[np.isnan(y)] = 0.0                     # Inf * 0 and NaN * 0 in a non-finite row: stored as +0
     return round_to_storage(y, dtype)
 
 

@@ -103,6 +103,18 @@ __device__ __forceinline__ double warp_butterfly_f64(double v) {
     return v;
 }
 
+// Normalisation of one stored row or query from its canonical sum of squares n2 (DESIGN.md 2): inv = 1 / sqrt(n2), and
+// inv = 0 for a zero vector and for a non-finite one (any NaN or +-Inf component makes n2 NaN or +inf; a finite fp32 row
+// cannot overflow n2 in fp64).  norm_elem maps the NaN that an Inf or NaN element times inv = 0 gives to +0, so a
+// non-finite vector is stored as a zero vector and scores exactly 0 against everything.  Every normaliser uses these two.
+__device__ __forceinline__ double inv_norm(double n2) {
+    return n2 > 0.0 && n2 <= 1.7976931348623157e308 ? 1.0 / sqrt(n2) : 0.0;
+}
+__device__ __forceinline__ float norm_elem(float x, double inv) {
+    const float y = (float)((double)x * inv);
+    return y == y ? y : 0.0f;
+}
+
 template <int DT>
 __device__ __forceinline__ double canonical_dot_row(const typename Store<DT>::T* __restrict__ row,
                                                     const float* __restrict__ q, int dim, int lane) {

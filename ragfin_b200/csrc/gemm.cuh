@@ -565,10 +565,10 @@ __global__ void __launch_bounds__(256) prep_queries_kernel(const float* __restri
         acc = acc + v * v;
     }
     const double n2 = warp_butterfly_f64(acc);
-    const double inv = n2 > 0.0 ? 1.0 / sqrt(n2) : 0.0;
+    const double inv = inv_norm(n2);
     double d2 = 0.0;
     for (int i = lane; i < ld; i += kWarp) {
-        const float y = i < dim ? (float)((double)x[i] * inv) : 0.0f;
+        const float y = i < dim ? norm_elem(x[i], inv) : 0.0f;
         out[i] = y;
         if (DT != 0) {
             const typename Store<DT>::T r = Store<DT>::from_f32(y);

@@ -64,11 +64,11 @@ __global__ void __launch_bounds__(256) ingest_kernel(const float* __restrict__ s
             acc = acc + v * v;
         }
         const double n2 = warp_butterfly_f64(acc);
-        const double inv = n2 > 0.0 ? 1.0 / sqrt(n2) : 0.0;
+        const double inv = inv_norm(n2);
         T* out = dst + r * (int64_t)ld;
         for (int i = lane * 2; i < ld; i += 2 * kWarp) {
-            const float y0 = i < dim ? (float)((double)elem(i) * inv) : 0.0f;
-            const float y1 = i + 1 < dim ? (float)((double)elem(i + 1) * inv) : 0.0f;
+            const float y0 = i < dim ? norm_elem(elem(i), inv) : 0.0f;
+            const float y1 = i + 1 < dim ? norm_elem(elem(i + 1), inv) : 0.0f;
             if (DT == 0 || DT == 3) {
                 *reinterpret_cast<float2*>(out + i) = make_float2(y0, y1);
                 if (DT == 3) *reinterpret_cast<__half2*>(dst16 + r * (int64_t)ld + i) = __halves2half2(__float2half_rn(y0), __float2half_rn(y1));
@@ -122,14 +122,14 @@ __global__ void __launch_bounds__(kIngestThreads) ingest_vec_kernel(const float*
         }
         __syncwarp();                               // the staging row is free for the next iteration
         const double n2 = warp_butterfly_f64(acc);
-        const double inv = n2 > 0.0 ? 1.0 / sqrt(n2) : 0.0;
+        const double inv = inv_norm(n2);
         T* out = dst + r * (int64_t)ld;
 #pragma unroll
         for (int j = 0; j < NV; ++j) {
             const int vi = j * kWarp + lane;
             if (vi < nvec_out) {                    // vectors in [nvec, nvec_out) are the zero padding of the stored row
-                const float y0 = (float)((double)v[j].x * inv), y1 = (float)((double)v[j].y * inv);
-                const float y2 = (float)((double)v[j].z * inv), y3 = (float)((double)v[j].w * inv);
+                const float y0 = norm_elem(v[j].x, inv), y1 = norm_elem(v[j].y, inv);
+                const float y2 = norm_elem(v[j].z, inv), y3 = norm_elem(v[j].w, inv);
                 if (DT == 0 || DT == 3) {
                     __stcs(reinterpret_cast<float4*>(out) + vi, make_float4(y0, y1, y2, y3));
                     if (DT == 3) {

@@ -327,7 +327,7 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
                 for (int u = 0; u < 24; ++u) { const double v = (double)xv[u]; acc = acc + v * v; }   // + 0 for the tail: exact
             }
             const double n2 = warp_butterfly_f64(acc);
-            if (lane == 0) inv_s[j] = n2 > 0.0 ? 1.0 / sqrt(n2) : 0.0;
+            if (lane == 0) inv_s[j] = inv_norm(n2);
         }
         __syncthreads();
         if (blockIdx.x == 0 && tid == 0) a.ctl->t[9] = global_ns();
@@ -364,7 +364,7 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
                         uint8_t* p_hi = fsm + (size_t)kb * QTILE + (size_t)(row_hi >> 3) * 1024 + (size_t)(row_hi & 7) * 128 + ((cc ^ (row_hi & 7)) << 4);
                         float y[VE];
 #pragma unroll
-                        for (int e = 0; e < VE; ++e) y[e] = (float)((double)xv[u][e] * inv);
+                        for (int e = 0; e < VE; ++e) y[e] = norm_elem(xv[u][e], inv);
                         if (blockIdx.x == 0) {
 #pragma unroll
                             for (int e = 0; e < VE; e += 4) *reinterpret_cast<float4*>(a.qn + (size_t)j * a.ld + i + e) = make_float4(y[e], y[e + 1], y[e + 2], y[e + 3]);
@@ -418,7 +418,7 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
                     if (un >= units) break;                         // block-uniform
                     const int j = un / upq, i = (un - j * upq) * kFThreads + tid;
                     if (i < a.dim) {
-                        const float y = (float)((double)xv[u] * inv_s[j]);
+                        const float y = norm_elem(xv[u], inv_s[j]);
                         if (blockIdx.x == 0) a.qn[(size_t)j * a.ld + i] = y;
                         const int row_hi = SPLIT ? (j >> 3) * 16 + (j & 7) : j;
                         const int kb = i / KE, c = (i % KE) * esz;

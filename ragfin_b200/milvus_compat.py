@@ -60,6 +60,16 @@ class ParamError(MilvusException):
     pass
 
 
+def _refuse_non_finite(vectors: np.ndarray, what: str) -> None:
+    """Milvus refuses float vectors holding NaN or +-Inf.  The engine would treat such a vector as the zero vector
+    (include/ragfin.h), a silent answer for what is almost always a broken embedding, so the shim refuses host data.
+    CUDA tensors are not checked: that would cost a pass and a synchronisation, and the engine's rule holds for them."""
+    bad = ~np.isfinite(vectors)
+    if bad.any():
+        row = int(np.argwhere(bad)[0][0])
+        raise MilvusException(message=f"{what}: vector {row} holds NaN or Inf; float vectors must be finite")
+
+
 class DataType(IntEnum):
     NONE = 0
     BOOL = 1
@@ -550,6 +560,7 @@ class Collection:
             emb = np.array(emb, dtype=np.float32, order="C")               # a private copy: pending until flush()
             if n and (emb.ndim != 2 or emb.shape != (n, dim)):
                 raise ParamError(message=f"embedding column must be [{n}, {dim}], got {emb.shape}")
+            _refuse_non_finite(emb, "insert")
         pks = list(cols[fields.index(st.schema.primary_field)])
         return emb, pks, cols, n
 
@@ -628,6 +639,7 @@ class Collection:
             q = q[None, :]
         if q.ndim != 2 or q.shape[1] != st.schema.vector_field.dim:
             raise MilvusException(message=f"vector dimension mismatch: expected {st.schema.vector_field.dim}, got {q.shape}")
+        _refuse_non_finite(q, "search")
         with st.lock:
             st.flush()
             res = SearchResult()
