@@ -234,6 +234,26 @@ int ragfin_read_rows(ragfin_t* h, int64_t row0, int64_t n, void* out_host, int32
  * rows otherwise (test hook). */
 int ragfin_read_sweep_rows(ragfin_t* h, int64_t row0, int64_t n, void* out_host, int32_t* ld_out);
 
+/* Grouping search (Milvus' group_by_field, DESIGN.md 7d): the k best GROUPS, one hit per group.  Row r belongs to the
+ * group group_of_row[r]: `count` int32 codes, one per stored row, passed per search like allow_bits (the handle keeps no
+ * codes; ragfin_add, ragfin_compact and the file format are unchanged).
+ *  - A group's score is the exact fp32 score of its best row: the largest (score desc, row asc) among its allowed, live
+ *    rows.  The hit of a group is that row; hits are ordered (score desc, id asc) and slots past the number of non-empty
+ *    groups hold (-1, -inf).
+ *  - A row whose code lies outside [0, n_groups) is never returned (as if filtered out): codes need no validation pass.
+ *  - allow_bits (NULL = every row) and tombstones compose as with ragfin_search_filtered.
+ *  - codes[r] = r with n_groups = count is the plain search, bit for bit; a single group is the plain top-1.
+ * Codes: ragfin_search_grouped takes device memory; ragfin_search_grouped_host takes host memory (copied in) or, with
+ * groups_on_device = 1, device memory, so that a caller keeping the codes resident uploads nothing per search.  A NULL code
+ * pointer or n_groups < 1 gives RAGFIN_EINVAL, checked before the handle.  ragfin_last_search_stats reports path 2, and
+ * queries_rescanned counts queries that overflowed the batched route into the exact path.  No sharded form; grouping is
+ * not combined with a range window.  Workspace: 16 * n_groups * 4 bytes next to the large-k route's score dump. */
+int ragfin_search_grouped(ragfin_t* h, const float* q, int32_t nq, int32_t k, const int32_t* group_of_row_dev, int32_t n_groups,
+                          const uint32_t* allow_bits_dev, int64_t n_allowed, int64_t* out_ids, float* out_scores, void* stream);
+int ragfin_search_grouped_host(ragfin_t* h, const float* q_host, int32_t nq, int32_t k, const int32_t* group_of_row,
+                               int32_t groups_on_device, int32_t n_groups, const uint32_t* allow_bits_host, int64_t n_allowed,
+                               int64_t* out_ids_host, float* out_scores_host);
+
 /* Counters of the most recent search on this handle: kernel launches issued, queries that
  * took the exact-rescan tier (certificate failed), which scoring path ran
  * (0 = small-batch scan, 1 = tcgen05 GEMM, 2 = large-k radix select).  Reading queries_rescanned synchronises. */

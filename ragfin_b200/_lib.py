@@ -18,7 +18,7 @@ SO_PATH = os.environ.get("RAGFIN_LIB") or os.path.join(CSRC, "libragfin.so")
 SYMBOLS = (
     "ragfin_abi_version", "ragfin_create", "ragfin_create_view", "ragfin_add", "ragfin_add_synthetic", "ragfin_add_synthetic_topics", "ragfin_count", "ragfin_reserve",
     "ragfin_delete", "ragfin_live_count", "ragfin_read_live_mask", "ragfin_compact",
-    "ragfin_set_id_base", "ragfin_search", "ragfin_search_host", "ragfin_search_filtered", "ragfin_search_filtered_host", "ragfin_search_range", "ragfin_search_range_host", "ragfin_merge_topk", "ragfin_read_rows", "ragfin_read_sweep_rows",
+    "ragfin_set_id_base", "ragfin_search", "ragfin_search_host", "ragfin_search_filtered", "ragfin_search_filtered_host", "ragfin_search_range", "ragfin_search_range_host", "ragfin_search_grouped", "ragfin_search_grouped_host", "ragfin_merge_topk", "ragfin_read_rows", "ragfin_read_sweep_rows",
     "ragfin_last_search_stats", "ragfin_profile", "ragfin_profile_read", "ragfin_save", "ragfin_load", "ragfin_set_gemm_min_batch", "ragfin_set_gemm_cluster", "ragfin_set_gemm_variant", "ragfin_set_bound_pass", "ragfin_set_scan_variant", "ragfin_set_append_mode", "ragfin_set_fused", "ragfin_set_pipelined", "ragfin_debug_fused_counts", "ragfin_debug_fused_times", "ragfin_debug_fused_ctas", "ragfin_debug_fused_tile_order", "ragfin_debug_gemm_scores", "ragfin_debug_plan", "ragfin_destroy", "ragfin_last_error",
     "ragfin_exchange_create", "ragfin_exchange_handle", "ragfin_exchange_connect", "ragfin_exchange_allgather_merge", "ragfin_fused_eligible", "ragfin_search_sharded", "ragfin_search_sharded_host", "ragfin_exchange_destroy",
 )
@@ -69,6 +69,8 @@ def load() -> ctypes.CDLL:
     L.ragfin_search_filtered_host.argtypes = [vp, vp, i32, i32, vp, i64, vp, vp]
     L.ragfin_search_range.argtypes = [vp, vp, i32, i32, vp, vp, i64, vp, vp, vp]   # range: ctypes.c_float * 2 {radius, range_filter}
     L.ragfin_search_range_host.argtypes = [vp, vp, i32, i32, vp, vp, i64, vp, vp]
+    L.ragfin_search_grouped.argtypes = [vp, vp, i32, i32, vp, i32, vp, i64, vp, vp, vp]
+    L.ragfin_search_grouped_host.argtypes = [vp, vp, i32, i32, vp, i32, i32, vp, i64, vp, vp]
     L.ragfin_merge_topk.argtypes = [vp, vp, i32, i32, i32, i64, i64, i64, vp, vp, i32, vp]
     L.ragfin_profile.argtypes = [vp, i32]
     L.ragfin_save.argtypes = [vp, ctypes.c_char_p]

@@ -70,7 +70,7 @@ struct ragfin {
     bool is_view = false;  // ragfin_create_view: `data` and `sweep_data` belong to another handle (read-only here, never freed here)
     std::mutex mu;
     // workspace (grow-only)
-    Buf qhat, q16, eps_q, gtau, bmax, acnt, athr, awin, allow, bk_scores, bk_state, bk_keys, bk_rows, cand, cand_e, flags, stage_q, stage_ids, stage_scores, add_stage;
+    Buf qhat, q16, eps_q, gtau, bmax, acnt, athr, awin, allow, bk_scores, bk_state, bk_keys, bk_rows, grp, grp_codes, cand, cand_e, flags, stage_q, stage_ids, stage_scores, add_stage;
     int gemm_min_nq = 3;      // query batches of at least this many rows take the tcgen05 path (1-2: HBM-bound scan) ...
     int gemm_min_nq_large = 1;   // ... except on corpora of >= kSweepBytes, where the TMA-fed sweep wins from 1 query
     int gemm_cluster = 0;     // 0 = choose by batch size; 1, 2 or 4 = force
@@ -81,6 +81,8 @@ struct ragfin {
     bool cur_user_filter = false;          // the caller passed a filter: filtered dispatch (no bound pass, no append mode)
     bool cur_window = false;               // the search in flight is a range search (ragfin_search_range): hits must satisfy
     float cur_radius = -INFINITY, cur_range_filter = INFINITY;   //   cur_radius < score <= cur_range_filter (DESIGN.md 7c)
+    const int32_t* cur_groups = nullptr;   // the search in flight is a grouping search (ragfin_search_grouped): device codes
+    int32_t cur_n_groups = 0;              //   [count], one hit per code in [0, cur_n_groups) (DESIGN.md 7d)
     // Tombstones (ragfin_delete).  live_host mirrors the device mask live_dev bit for bit: ceil(capacity / 32) words in the
     // allow_bits layout, bit set = row live; rows at or past `count` are live (rows added later are).  Both stay empty until
     // the first delete, and a handle with n_dead == 0 passes a null mask to every kernel.
@@ -307,7 +309,7 @@ extern "C" void ragfin_destroy(ragfin_t* h) {
     if (!h) return;
     DeviceGuard g(h->device);
     (void)cudaDeviceSynchronize();
-    Buf* bufs[] = {&h->qhat, &h->q16, &h->eps_q, &h->gtau, &h->bmax, &h->acnt, &h->athr, &h->awin, &h->allow, &h->bk_scores, &h->bk_state, &h->bk_keys, &h->bk_rows, &h->cand, &h->cand_e, &h->flags, &h->stage_q, &h->stage_ids, &h->stage_scores, &h->add_stage, &h->fctl, &h->fcand, &h->fqn, &h->fflags};
+    Buf* bufs[] = {&h->qhat, &h->q16, &h->eps_q, &h->gtau, &h->bmax, &h->acnt, &h->athr, &h->awin, &h->allow, &h->bk_scores, &h->bk_state, &h->bk_keys, &h->bk_rows, &h->grp, &h->grp_codes, &h->cand, &h->cand_e, &h->flags, &h->stage_q, &h->stage_ids, &h->stage_scores, &h->add_stage, &h->fctl, &h->fcand, &h->fqn, &h->fflags};
     for (Buf* b : bufs)
         if (b->p) cudaFree(b->p);
     if (h->sweep_data && has_copy(h) && !h->is_view) cudaFree(h->sweep_data);
@@ -1557,9 +1559,61 @@ static int search_bigk(ragfin* h, const float* q_dev, int nq, int k, int64_t* ou
     return 0;
 }
 
+// Grouping search, exact path (DESIGN.md 7d): exact scores of every row, the best key of every group, radix select of the
+// m-th largest group key, rank sort.  One query at a time; serves small corpora, RAGFIN_NO_BIGK_BATCHED=1 and the batched
+// route's overflow.
+static int search_grouped(ragfin* h, const float* q_dev, int nq, int k, int64_t* out_ids, float* out_scores, cudaStream_t st) {
+    int rc;
+    const int64_t n = h->count, ng = h->cur_n_groups;
+    const int m = (int64_t)k < ng ? k : (int)ng;   // hits that may exist
+    h->stats.path = 2;
+    h->stats.cand_per_query = m;
+    h->stats.queries_rescanned = 0;
+    if ((rc = ensure(h->qhat, (size_t)h->ld * sizeof(float)))) return rc;
+    if ((rc = ensure(h->bk_scores, (size_t)n * sizeof(float)))) return rc;
+    if ((rc = ensure(h->bk_state, sizeof(RadixState)))) return rc;
+    if ((rc = ensure(h->bk_keys, (size_t)m * sizeof(u64)))) return rc;
+    if ((rc = ensure(h->grp, (size_t)ng * sizeof(u64)))) return rc;
+    float* qhat = (float*)h->qhat.p;
+    float* scores = (float*)h->bk_scores.p;
+    RadixState* state = (RadixState*)h->bk_state.p;
+    u64* keys = (u64*)h->bk_keys.p;
+    u64* gbest = (u64*)h->grp.p;
+    const int blocks = h->num_sms * 8;
+    for (int q = 0; q < nq; ++q) {
+        if ((rc = launch_ingest<false>(0, q_dev + (size_t)q * h->dim, 0, 0, 0, 0, 1, h->dim, h->ld, qhat, h->num_sms, st))) return rc;
+        switch (h->dtype) {
+            case 0: score_all_kernel<0><<<blocks, 256, 0, st>>>(h->data, n, h->ld, qhat, scores, h->cur_allow, -INFINITY, INFINITY); break;
+            case 1: score_all_kernel<1><<<blocks, 256, 0, st>>>(h->data, n, h->ld, qhat, scores, h->cur_allow, -INFINITY, INFINITY); break;
+            default: score_all_kernel<2><<<blocks, 256, 0, st>>>(h->data, n, h->ld, qhat, scores, h->cur_allow, -INFINITY, INFINITY); break;
+        }
+        CU_TRY(cudaMemsetAsync(gbest, 0, (size_t)ng * sizeof(u64), st));
+        group_best_kernel<<<blocks, 256, 0, st>>>(scores, n, h->cur_groups, (int)ng, gbest);
+        CU_TRY(cudaGetLastError());
+        RadixState init;
+        memset(&init, 0, sizeof(init));
+        init.remaining = m;
+        CU_TRY(cudaMemcpyAsync(state, &init, sizeof(init), cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaStreamSynchronize(st));   // `init` lives on this stack frame
+        for (int shift = 56; shift >= 0; shift -= 8) {
+            radix_hist_keys_kernel<<<blocks, 256, 0, st>>>(gbest, ng, shift, state);
+            radix_pick_kernel<<<1, 32, 0, st>>>(shift, state);
+        }
+        pad_keys_kernel<<<(m + 255) / 256, 256, 0, st>>>(keys, m);
+        group_compact_kernel<<<blocks, 256, 0, st>>>(gbest, ng, state, keys, m);
+        const int span = m > k ? m : k;
+        rank_sort_kernel<<<(span + 255) / 256, 256, 0, st>>>(keys, m, k, h->id_base, out_ids + (size_t)q * k, out_scores + (size_t)q * k);
+        CU_TRY(cudaGetLastError());
+        h->stats.launches += 23;
+    }
+    return 0;
+}
+
 // Batched large-k path (bigk.cuh, second half): up to 16 queries per tensor-core sweep, approximate scores dumped, radix
 // select + compaction + exact rescore + rank sort per query with grid.y = query; ONE stream synchronisation at the end to
 // read the overflow flags (flagged queries - thousands of rows within 2 eps of the k-th score - take the exact one-query path).
+// A grouping search (h->cur_groups, DESIGN.md 7d) adds the group maxima, selects T among them, cuts each row at its group's
+// maximum too, keeps one candidate per group, and sends flagged queries to search_grouped.
 static const int kBigChunk = 16;
 static int search_bigk_batched(ragfin* h, const float* q_dev, int nq, int k, int64_t* out_ids, float* out_scores, cudaStream_t st) {
     int rc;
@@ -1583,6 +1637,9 @@ static int search_bigk_batched(ragfin* h, const float* q_dev, int nq, int k, int
     if ((rc = ensure(h->bk_rows, (size_t)kBigChunk * cmax * sizeof(uint32_t)))) return rc;
     if ((rc = ensure(h->bk_keys, (size_t)kBigChunk * cmax * sizeof(u64)))) return rc;
     if (h->cur_window && (rc = ensure(h->awin, (size_t)3 * kBigChunk * sizeof(float)))) return rc;
+    const int ng = h->cur_n_groups;
+    if (h->cur_groups && (rc = ensure(h->grp, (size_t)kBigChunk * ng * sizeof(uint32_t)))) return rc;
+    uint32_t* gmax = (uint32_t*)h->grp.p;
     float* qhat = (float*)h->qhat.p;
     float* scores = (float*)h->bk_scores.p;
     BkState* states = (BkState*)h->bk_state.p;
@@ -1612,15 +1669,29 @@ static int search_bigk_batched(ragfin* h, const float* q_dev, int nq, int k, int
             h->stats.launches++;
         }
         BkState* stq = states + q0;
-        for (int pass = 0; pass < 4; ++pass)
-            bk_hist_kernel<<<dim3(blocks, nb), 256, 0, st>>>(scores, n, pass, keff, stq, h->cur_allow, w ? w + 2 * nb : nullptr);
-        bk_compact_kernel<<<dim3(blocks, nb), 256, 0, st>>>(scores, n, keff, eps, (const float*)h->eps_q.p, stq, (uint32_t*)h->bk_rows.p, cmax, h->cur_allow,
-                                                            w, w ? w + nb : nullptr);
+        if (h->cur_groups) {
+            CU_TRY(cudaMemsetAsync(gmax, 0, (size_t)nb * ng * sizeof(uint32_t), st));
+            bk_group_max_kernel<<<blocks, 256, 0, st>>>(scores, n, nb, h->cur_groups, ng, h->cur_allow, gmax);
+            for (int pass = 0; pass < 4; ++pass)
+                bk_hist_kernel<true><<<dim3(blocks, nb), 256, 0, st>>>((const float*)gmax, ng, pass, keff, stq, nullptr, nullptr);
+            bk_group_compact_kernel<<<dim3(blocks, nb), 256, 0, st>>>(scores, n, keff, eps, (const float*)h->eps_q.p, stq, (uint32_t*)h->bk_rows.p,
+                                                                      cmax, h->cur_allow, h->cur_groups, ng, gmax);
+            h->stats.launches += 2;
+        } else {
+            for (int pass = 0; pass < 4; ++pass)
+                bk_hist_kernel<<<dim3(blocks, nb), 256, 0, st>>>(scores, n, pass, keff, stq, h->cur_allow, w ? w + 2 * nb : nullptr);
+            bk_compact_kernel<<<dim3(blocks, nb), 256, 0, st>>>(scores, n, keff, eps, (const float*)h->eps_q.p, stq, (uint32_t*)h->bk_rows.p, cmax, h->cur_allow,
+                                                                w, w ? w + nb : nullptr);
+        }
         const dim3 rg((cmax + 7) / 8, nb);
         switch (h->dtype) {
             case 0: bk_rescore_kernel<0><<<rg, 256, 0, st>>>(h->data, h->ld, qhat, stq, (const uint32_t*)h->bk_rows.p, cmax, (u64*)h->bk_keys.p, h->cur_radius, h->cur_range_filter); break;
             case 1: bk_rescore_kernel<1><<<rg, 256, 0, st>>>(h->data, h->ld, qhat, stq, (const uint32_t*)h->bk_rows.p, cmax, (u64*)h->bk_keys.p, h->cur_radius, h->cur_range_filter); break;
             default: bk_rescore_kernel<2><<<rg, 256, 0, st>>>(h->data, h->ld, qhat, stq, (const uint32_t*)h->bk_rows.p, cmax, (u64*)h->bk_keys.p, h->cur_radius, h->cur_range_filter); break;
+        }
+        if (h->cur_groups) {
+            bk_group_rep_kernel<<<dim3((cmax + 255) / 256, nb), 256, 0, st>>>((u64*)h->bk_keys.p, stq, cmax, h->cur_groups);
+            h->stats.launches++;
         }
         const int span = cmax > k ? cmax : k;
         bk_rank_sort_kernel<<<dim3((span + 255) / 256, nb), 256, 0, st>>>((const u64*)h->bk_keys.p, stq, cmax, k, keff, h->id_base,
@@ -1637,7 +1708,8 @@ static int search_bigk_batched(ragfin* h, const float* q_dev, int nq, int k, int
     for (int q = 0; q < nq; ++q) {
         if (!host[q].overflow) continue;
         ++redone;
-        if ((rc = search_bigk(h, q_dev + (size_t)q * h->dim, 1, k, out_ids + (size_t)q * k, out_scores + (size_t)q * k, st))) return rc;
+        if ((rc = (h->cur_groups ? search_grouped : search_bigk)(h, q_dev + (size_t)q * h->dim, 1, k, out_ids + (size_t)q * k,
+                                                                 out_scores + (size_t)q * k, st))) return rc;
     }
     h->stats.path = 2;
     h->stats.cand_per_query = cmax;
@@ -1658,6 +1730,10 @@ static int search_locked(ragfin* h, const float* q_dev, int nq, int k, int64_t* 
     const int steps = round_steps((nvec + 31) / 32);
     const int64_t n_eff = h->cur_allow ? h->cur_allowed : n;   // rows a hit may come from
     if ((rc = ensure(h->flags, (size_t)(kMaxQueryBatch + 1) * sizeof(int)))) return rc;
+    if (h->cur_groups) {   // grouping search (DESIGN.md 7d): the large-k route on corpora worth a sweep, else the exact path
+        if (h->use_bigk_batched && n >= 4096 && gemm_rows_ok(h)) return search_bigk_batched(h, q_dev, nq, k, out_ids, out_scores, st);
+        return search_grouped(h, q_dev, nq, k, out_ids, out_scores, st);
+    }
     const int min_nq_all = (size_t)n * h->ld * esize(h->dtype) >= kSweepBytes ? h->gemm_min_nq_large : h->gemm_min_nq;
     const bool ap = append_eligible(h, k) && nq >= min_nq_all;   // tensor-core append mode: no K' lists needed
     if (h->cur_window && !ap) {
@@ -2219,7 +2295,7 @@ static int search_host_locked(ragfin* h, const float* q_host, int nq, int k, int
         }
         void* dptr = nullptr;
         if (h->hstage && cudaHostGetDevicePointer(&dptr, h->hstage, 0) == cudaSuccess) {
-            if (!h->cur_window && nq <= h->fused_max_nq && fused_eligible(h, nq, k)) {
+            if (!h->cur_window && !h->cur_groups && nq <= h->fused_max_nq && fused_eligible(h, nq, k)) {
                 if ((rc = fused_host_call(h, nullptr, q_host, nq, k, out_ids_host, out_scores_host, st))) return rc;
                 return mark_done(h, st);
             }
@@ -2414,6 +2490,63 @@ extern "C" int ragfin_search_range_host(ragfin_t* h, const float* q_host, int32_
     set_window(h, radius, range_filter);
     rc = search_host_locked(h, q_host, nq, k, out_ids_host, out_scores_host, st);
     clear_window(h);
+    clear_filter(h);
+    return rc;
+}
+
+// Grouping search (DESIGN.md 7d): the k best groups, each represented by its best row.  The codes are installed next to the
+// row mask for the one dispatch (search_locked).  The codes are checked first: that needs neither a handle nor a device.
+static int check_group_args(const ragfin* h, const float* q, int nq, int k, const int32_t* groups, int n_groups,
+                            const void* out_ids, const void* out_scores) {
+    if (!groups) return fail(RAGFIN_EINVAL, "NULL group codes");
+    if (n_groups < 1) return fail(RAGFIN_EINVAL, "n_groups = %d must be at least 1", n_groups);
+    if (!h) return fail(RAGFIN_EINVAL, "NULL handle");
+    if (nq < 0 || (nq > 0 && (!q || !out_ids || !out_scores))) return fail(RAGFIN_EINVAL, "NULL buffer");
+    if (k < 1 || k > 16384) return fail(RAGFIN_EINVAL, "k = %d outside [1, 16384]", k);
+    return 0;
+}
+static void set_groups(ragfin* h, const int32_t* groups_dev, int n_groups) { h->cur_groups = groups_dev; h->cur_n_groups = n_groups; }
+static void clear_groups(ragfin* h) { h->cur_groups = nullptr; h->cur_n_groups = 0; }
+
+extern "C" int ragfin_search_grouped(ragfin_t* h, const float* q, int32_t nq, int32_t k, const int32_t* group_of_row_dev,
+                                     int32_t n_groups, const uint32_t* allow_bits_dev, int64_t n_allowed, int64_t* out_ids,
+                                     float* out_scores, void* stream) {
+    int rc;
+    if ((rc = check_group_args(h, q, nq, k, group_of_row_dev, n_groups, out_ids, out_scores))) return rc;
+    if (nq == 0) return RAGFIN_OK;
+    std::lock_guard<std::mutex> lk(h->mu);
+    DeviceGuard g(h->device);
+    cudaStream_t st = (cudaStream_t)stream;
+    if ((rc = wait_prev(h, st))) return rc;
+    if ((rc = set_filter(h, allow_bits_dev, n_allowed, 1, st))) return rc;
+    set_groups(h, group_of_row_dev, n_groups);
+    rc = search_locked(h, q, nq, k, out_ids, out_scores, st);
+    clear_groups(h);
+    clear_filter(h);
+    if (rc) return rc;
+    return mark_done(h, st);
+}
+
+extern "C" int ragfin_search_grouped_host(ragfin_t* h, const float* q_host, int32_t nq, int32_t k, const int32_t* group_of_row,
+                                          int32_t groups_on_device, int32_t n_groups, const uint32_t* allow_bits_host,
+                                          int64_t n_allowed, int64_t* out_ids_host, float* out_scores_host) {
+    int rc;
+    if ((rc = check_group_args(h, q_host, nq, k, group_of_row, n_groups, out_ids_host, out_scores_host))) return rc;
+    if (nq == 0) return RAGFIN_OK;
+    std::lock_guard<std::mutex> lk(h->mu);
+    DeviceGuard g(h->device);
+    cudaStream_t st = 0;
+    if ((rc = wait_prev(h, st))) return rc;
+    const int32_t* codes = group_of_row;
+    if (!groups_on_device && h->count > 0) {
+        if ((rc = ensure(h->grp_codes, (size_t)h->count * sizeof(int32_t)))) return rc;
+        CU_TRY(cudaMemcpyAsync(h->grp_codes.p, group_of_row, (size_t)h->count * sizeof(int32_t), cudaMemcpyHostToDevice, st));
+        codes = (const int32_t*)h->grp_codes.p;
+    }
+    if ((rc = set_filter(h, allow_bits_host, n_allowed, 0, st))) return rc;
+    set_groups(h, codes, n_groups);
+    rc = search_host_locked(h, q_host, nq, k, out_ids_host, out_scores_host, st);
+    clear_groups(h);
     clear_filter(h);
     return rc;
 }

@@ -246,18 +246,30 @@ class Index:
 
     def search(self, queries, k: int, out_ids: Optional[np.ndarray] = None,
                out_scores: Optional[np.ndarray] = None, allow: Optional[np.ndarray] = None,
-               radius: Optional[float] = None, range_filter: Optional[float] = None) -> Tuple[np.ndarray, np.ndarray]:
+               radius: Optional[float] = None, range_filter: Optional[float] = None,
+               group_by=None, n_groups: Optional[int] = None) -> Tuple[np.ndarray, np.ndarray]:
         """Host path: queries numpy / list / torch CPU tensor [nq, dim] -> (ids int64 [nq, k], scores fp32 [nq, k]).
         Hits are in descending score, ties to the lower id; slots past min(k, N) hold (-1, -inf).
         `out_ids` / `out_scores` may be caller-owned (e.g. pinned) C-contiguous numpy arrays or torch CPU tensors; they are
         returned as passed, fresh numpy arrays otherwise.
         `allow`: optional bool array [N]; only rows with allow[r] may be returned (scalar-filtered search).
         `radius` / `range_filter`: range search, only rows with radius < score <= range_filter (both rounded to fp32 with
-        np.float32; None = open) may be returned, and slots past the rows in the window hold (-1, -inf)."""
+        np.float32; None = open) may be returned, and slots past the rows in the window hold (-1, -inf).
+        `group_by` / `n_groups`: grouping search, the k best groups with one hit each (the group's best row); `group_by` is
+        row r's group code, int32 [N] as a numpy array (copied in) or a CUDA tensor (read in place).  Rows whose code lies
+        outside [0, n_groups) are never returned; slots past the non-empty groups hold (-1, -inf).  Composes with `allow`,
+        not with a range window."""
         k = self._check_k(k)
+        grouped = self._check_groups(group_by, n_groups, radius, range_filter)
         q, qp, nq = _host_queries(queries, self.dim)
         ids, ip = _host_out(out_ids, nq, k, np.int64, "out_ids")
         scores, sp = _host_out(out_scores, nq, k, np.float32, "out_scores")
+        if grouped is not None:
+            codes, cp, on_device = grouped
+            packed, n_allowed = self._pack_allow(allow) if allow is not None else (None, 0)
+            _lib.check(self._L.ragfin_search_grouped_host(self._h, qp, nq, k, cp, on_device, int(n_groups),
+                                                          packed.ctypes.data if packed is not None else None, n_allowed, ip, sp))
+            return ids, scores
         if radius is not None or range_filter is not None:
             window = _window(radius, range_filter)
             packed, n_allowed = self._pack_allow(allow) if allow is not None else (None, 0)
@@ -271,6 +283,33 @@ class Index:
         _lib.check(self._L.ragfin_search_host(self._h, qp, nq, k, ip, sp))
         return ids, scores
 
+    def _check_groups(self, group_by, n_groups, radius, range_filter):
+        """Grouping arguments -> None (plain search) or (object keeping the codes alive, address, on_device)."""
+        if group_by is None:
+            if n_groups is not None:
+                raise ValueError("n_groups needs group_by")
+            return None
+        if radius is not None or range_filter is not None:
+            raise ValueError("group_by cannot be combined with radius / range_filter")
+        if n_groups is None or not 1 <= int(n_groups) <= np.iinfo(np.int32).max:
+            raise ValueError(f"n_groups must be in [1, 2^31 - 1], got {n_groups!r}")
+        n = len(self)
+        if hasattr(group_by, "is_cuda") and group_by.is_cuda:
+            import torch
+            if group_by.dtype != torch.int32 or tuple(group_by.shape) != (n,):
+                raise ValueError(f"group_by must be an int32 tensor of shape [{n}], got {group_by.dtype} {tuple(group_by.shape)}")
+            if group_by.device.index != self.device:
+                raise ValueError(f"group_by lives on cuda:{group_by.device.index}, index on cuda:{self.device}")
+            g = group_by.contiguous()
+            return g, g.data_ptr(), 1
+        g = np.asarray(group_by.numpy() if hasattr(group_by, "numpy") else group_by)
+        if g.dtype != np.int32 or g.shape != (n,):
+            raise ValueError(f"group_by must be an int32 array of shape [{n}], got {g.dtype} {g.shape}")
+        g = np.ascontiguousarray(g)
+        if n == 0:
+            g = np.zeros(1, np.int32)   # the library wants a non-NULL pointer; nothing is read
+        return g, g.ctypes.data, 0
+
     def _pack_allow(self, allow):
         """bool [N] -> (ceil(N / 32) little-endian uint32 words, number of set bits), the allow_bits layout."""
         mask = np.ascontiguousarray(allow, dtype=bool)
@@ -283,11 +322,16 @@ class Index:
         return packed, int(mask.sum())
 
     def search_device(self, queries, k: int, out_ids=None, out_scores=None, stream=None,
-                      radius: Optional[float] = None, range_filter: Optional[float] = None):
+                      radius: Optional[float] = None, range_filter: Optional[float] = None,
+                      group_by=None, n_groups: Optional[int] = None):
         """Device path: `queries` is a torch CUDA fp32 tensor [nq, dim]; returns torch CUDA tensors.
-        Asynchronous on the given (default: current) stream.  `radius` / `range_filter`: range search, as in search()."""
+        Asynchronous on the given (default: current) stream.  `radius` / `range_filter`: range search, as in search().
+        `group_by` (CUDA int32 tensor [N]) / `n_groups`: grouping search, as in search()."""
         import torch
         k = self._check_k(k)
+        if group_by is not None and not (hasattr(group_by, "is_cuda") and group_by.is_cuda):
+            raise ValueError("search_device takes group_by as a CUDA int32 tensor")
+        grouped = self._check_groups(group_by, n_groups, radius, range_filter)
         if not queries.is_cuda or queries.dtype != torch.float32 or queries.dim() != 2 or queries.shape[1] != self.dim:
             raise ValueError(f"queries must be a CUDA fp32 tensor [nq, {self.dim}]")
         queries = queries.contiguous()
@@ -297,6 +341,10 @@ class Index:
         if out_scores is None:
             out_scores = torch.empty((nq, k), dtype=torch.float32, device=queries.device)
         with torch.cuda.device(self.device):
+            if grouped is not None:
+                _lib.check(self._L.ragfin_search_grouped(self._h, queries.data_ptr(), nq, k, grouped[1], int(n_groups), None, 0,
+                                                         out_ids.data_ptr(), out_scores.data_ptr(), _stream_ptr(stream)))
+                return out_ids, out_scores
             if radius is not None or range_filter is not None:
                 _lib.check(self._L.ragfin_search_range(self._h, queries.data_ptr(), nq, k, _window(radius, range_filter), None, 0,
                                                        out_ids.data_ptr(), out_scores.data_ptr(), _stream_ptr(stream)))

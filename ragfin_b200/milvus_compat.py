@@ -19,6 +19,9 @@ object the reference uses, so a maintainer switches with
   .search(..., {"metric_type": "COSINE", "params": {"radius": r, "range_filter": f}}, limit)   range search: at most
                                            `limit` hits with r < score <= f, best first (pymilvus 2.3; both bounds are
                                            rounded to fp32 and compared with the fp32 scores; range_filter needs radius)
+  .search(..., group_by_field=name)        grouping search (pymilvus 2.4): the `limit` best groups of rows sharing a value
+                                           of the scalar field `name`, one hit per group (its best row), best first; composes
+                                           with expr, output_fields and round_decimal; not with a range search
   .query(expr, output_fields=, limit=)     test_vector.py:35-39, graph_cons.py:308-311
   .delete(expr) / .upsert(data) / .compact()   keeping a corpus current: restated filings, re-cut chunks, withdrawn
                                            documents (pymilvus 2.3 names; not called by the reference itself)
@@ -30,7 +33,7 @@ resolve to the earlier-inserted row (SURVEY.md 8c).  delete() tombstones rows (t
 num_entities keeps counting them, as Milvus does, until compact() removes them and renumbers the survivors.
 
 The engine is exact: index_type / nlist / nprobe (and the other keys of a search's "params" but radius and range_filter)
-are accepted and ignored.
+are accepted and ignored, and so are search keywords other than group_by_field.
 """
 from __future__ import annotations
 
@@ -167,6 +170,10 @@ class _Store:
         # value -> ascending rows, per scalar field, built on the first filter over that field and kept current by
         # insert(): a filtered search costs the matching rows, not a pass over every row of the column
         self.scalar_index: Dict[str, Dict[Any, List[int]]] = {}
+        # field -> [value -> group code (first-seen order), int32 codes of the first n rows on the collection's device],
+        # built on the first grouping search over that field, extended to new rows by the next one, dropped by compact();
+        # delete() leaves it alone (the engine's tombstones keep deleted rows out)
+        self.group_codes: Dict[str, list] = {}
         self.lock = threading.RLock()
 
     def rows_with(self, field: str, wanted, n: int) -> List[int]:
@@ -193,6 +200,21 @@ class _Store:
                 import bisect
                 out = out[:bisect.bisect_left(out, n)]
             return list(out)
+
+    def codes_for(self, field: str):
+        """(int32 codes [n_inserted] of `field` on the collection's device, number of codes) for a grouping search."""
+        import torch
+        with self.lock:
+            entry = self.group_codes.get(field)
+            if entry is None:
+                dev = torch.device("cuda", self.device) if torch.cuda.is_available() else torch.device("cpu")
+                entry = self.group_codes[field] = [{}, torch.zeros(0, dtype=torch.int32, device=dev)]
+            code_of, codes = entry
+            n = codes.shape[0]
+            if n < self.n_inserted:
+                new = [code_of.setdefault(v, len(code_of)) for v in self.columns[field][n:self.n_inserted]]
+                entry[1] = torch.cat([codes, torch.tensor(new, dtype=torch.int32).to(codes.device)])
+            return entry[1], len(code_of)
 
     def flush(self):
         """Upload the pending blocks through K1.  The collection keeps NO host copy of the embeddings: when the rows
@@ -523,6 +545,7 @@ class Collection:
             st.pk_to_row = {v: i for i, v in enumerate(st.columns[st.schema.primary_field.name])}
             st.n_inserted = len(survivors)
             st.dead = set()
+            st.group_codes = {}   # rebuilt from the compacted columns by the next grouping search
 
     def get_compaction_state(self, timeout=None, **kwargs) -> CompactionState:
         return CompactionState(getattr(self._st, "compactions", 0))
@@ -634,6 +657,9 @@ class Collection:
             if f not in st.columns:
                 raise MilvusException(message=f"field {f} not exist")
         window = _range_window((param or {}).get("params") or {})
+        group_field = kwargs.get("group_by_field")
+        if group_field is not None:
+            self._check_group_field(group_field, window)
         q = np.ascontiguousarray(data, dtype=np.float32)
         if q.ndim == 1:
             q = q[None, :]
@@ -648,12 +674,15 @@ class Collection:
                     res.append(Hits())
                 return res
             # deleted rows: the engine holds their tombstones and never returns them, filtered or not
+            extra = dict(window)
+            if group_field is not None:
+                extra["group_by"], extra["n_groups"] = st.codes_for(group_field)
             if expr and expr.strip():     # scalar filter -> row bitmask consumed inside the top-k epilogues
                 allow = np.zeros(st.n_inserted, dtype=bool)
                 allow[self._rows_matching(expr.strip(), st.n_inserted)] = True
-                ids, scores = st.index.search(q, int(limit), allow=allow, **window)
+                ids, scores = st.index.search(q, int(limit), allow=allow, **extra)
             else:
-                ids, scores = st.index.search(q, int(limit), **window)
+                ids, scores = st.index.search(q, int(limit), **extra)
             pk_col = st.columns[st.schema.primary_field.name]
             cols, names = st.columns, tuple(out_fields)
             for qi in range(q.shape[0]):
@@ -664,6 +693,19 @@ class Collection:
                     sc_q = [round(s_, round_decimal) for s_ in sc_q]
                 res.append(Hits([Hit(pk_col[row], sc, Entity(cols, row, names)) for row, sc in zip(rows_q, sc_q)]))
             return res
+
+    def _check_group_field(self, name, window) -> None:
+        """group_by_field must name a scalar field Milvus can group by, and cannot be combined with a range search."""
+        st = self._st
+        if not isinstance(name, str):
+            raise MilvusException(message=f"group_by_field must be a field name, got {name!r}")
+        field = next((f for f in st.schema.fields if f.name == name), None)
+        if field is None:
+            raise MilvusException(message=f"group_by_field {name} not exist")
+        if field.dtype in (DataType.FLOAT_VECTOR, DataType.BINARY_VECTOR, DataType.FLOAT, DataType.DOUBLE, DataType.JSON):
+            raise MilvusException(message=f"group by is not supported on field {name} of type {field.dtype.name}")
+        if window:
+            raise MilvusException(message="group_by_field cannot be combined with a range search (radius / range_filter)")
 
     def _rows_matching(self, expr: str, n: int) -> List[int]:
         """Rows (ascending) among the first n that satisfy `field in [...]` or `field == literal`."""
