@@ -362,6 +362,15 @@ int ragfin_debug_gemm_scores(ragfin_t* h, const float* q_dev, int32_t nq, float*
  * The CPU suite checks the invariants exactness rests on: slices cover every row once, sample tiles are distinct and
  * never the last (partial) tile, at least 2 x rank sample blocks. */
 int ragfin_debug_plan(int32_t nq, int64_t n_rows, int32_t num_sms, int32_t k, int32_t cluster, int64_t* out);
+/* Test hook, pure host arithmetic (needs no device): the one-kernel search's plan for nq queries and top-k on a collection of
+ * `dtype` (RAGFIN_F32 .. RAGFIN_F32_F16) and `dim`, under the query limits max_nq and max_nqk (0: the defaults, 16 queries and
+ * queries x k <= 400; RAGFIN_FUSED_MAX_NQ / _NQK set them per handle) and the default ring depth.
+ * out[5] = {ncol (0: the search takes another path), split (1: the query enters as hi + lo), stages, pend, cap};
+ * out_eps[4] = {rel, sub, query term, eps_approx}: the per-element query-rounding bound |y - hi (- lo)| <= rel |y| + sub of the
+ * planned variant (plain when none), the query term of eps it gives, and the rest of eps (accumulation allowance, tf32
+ * truncation, fp16-copy rounding).  The kernel's eps is their sum, rounded up. */
+int ragfin_debug_fused_plan(int32_t dtype, int32_t dim, int32_t nq, int32_t k, int32_t max_nq, int32_t max_nqk, int64_t* out,
+                            double* out_eps);
 
 /* A second handle over the SAME device matrix (no copy) with its own workspace: searches through the parent and the
  * view (or two views) may be in flight at once on different streams, so the latency-bound head and tail of one call

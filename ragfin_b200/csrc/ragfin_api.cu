@@ -57,6 +57,8 @@ struct Buf {
     size_t bytes = 0;
 };
 
+static const int kFusedMaxNq = 16, kFusedMaxNqk = 400;   // default query limits of the one-kernel search (plan_fused)
+
 struct ragfin {
     int dim = 0, ld = 0, dtype = 0, device = 0, num_sms = 0;
     int64_t capacity = 0, count = 0, id_base = 0;
@@ -107,8 +109,8 @@ struct ragfin {
     bool use_fused = true;    // <= 64 queries, k <= 128: the one-kernel search (sweep_fused.cuh); RAGFIN_NO_FUSED=1 disables
     int fused_min_rows = 8192;
     int fused_refresh_every = 4, fused_stage_cap = kRMaxStages;   // experiment knobs (RAGFIN_FUSED_REFRESH_EVERY / _STAGES)
-    int fused_max_nq = 16;    // see plan_fused; RAGFIN_FUSED_MAX_NQ overrides (<= 64)
-    int fused_max_nqk = 400;  // queries x k; RAGFIN_FUSED_MAX_NQK overrides
+    int fused_max_nq = kFusedMaxNq;     // see plan_fused; RAGFIN_FUSED_MAX_NQ overrides (<= 64)
+    int fused_max_nqk = kFusedMaxNqk;   // queries x k; RAGFIN_FUSED_MAX_NQK overrides
     struct MapSlot { const void* base = nullptr; int64_t rows = 0; int ld = 0, dtype = 0, box_rows = 0; CUtensorMap map; };
     MapSlot map_cache[8];     // tensor maps are pure functions of (base, rows, ld, dtype, box): encode once
     int map_next = 0;
@@ -840,7 +842,7 @@ static int cand_per_query(int k) {
 
 // |fp32-accumulated dot - exact dot| for unit-norm operands (any summation order), plus the
 // fp32 rounding of the exact score and one ulp so that a tie after rounding cannot hide a row.
-static float eps_fp32_accumulate(int ld) { return (float)((ld + 64) * 5.9604644775390625e-08 * 1.0625 + 4.76837158203125e-07); }
+static float eps_fp32_accumulate(int ld) { return (float)((ld + 64) * 0x1p-24 * 1.0625 + 4.76837158203125e-07); }
 
 static const size_t kHostStageQ = 64 << 10, kHostStageOut = 64 << 10;   // mapped staging of ragfin_search_host (small requests)
 static const size_t kHostStageFlag = 64;                                // ... + the completion word the one-kernel search sets
@@ -988,11 +990,12 @@ static float eps_gemm_const(int dtype, int ld) {
 }
 // |approximate score - exact score| beyond the query rounding term, for the rows the sweeps read: + eps_sweep when they are
 // the fp16 copy of fp32 rows (the exact score is the fp32 row's)
-static float eps_approx(const ragfin* h) {
-    const float e = eps_gemm_const(h->sweep_dt, h->ld);
-    if (h->eps_sweep == 0.f) return e;
-    return nextafterf((float)((double)e + (double)h->eps_sweep), INFINITY);
+static float eps_approx(int sweep_dt, int ld, float eps_sweep) {
+    const float e = eps_gemm_const(sweep_dt, ld);
+    if (eps_sweep == 0.f) return e;
+    return nextafterf((float)((double)e + (double)eps_sweep), INFINITY);
 }
+static float eps_approx(const ragfin* h) { return eps_approx(h->sweep_dt, h->ld, h->eps_sweep); }
 
 // TMA coordinates are signed 32-bit: shards of 2^31 rows or more stay on the scan path (int64 row arithmetic)
 static bool gemm_rows_ok(const ragfin* h) { return h->count > 0 && h->count < ((int64_t)1 << 31) - kGN; }
@@ -1383,14 +1386,14 @@ struct FusedPlan {
 // that its per-query bookkeeping in the first tile and the finalize outweigh the launches it saves (32 queries: 0.383 vs 0.343;
 // 16 queries at k = 100: 0.504 vs 0.416).  Default limits: <= 16 queries and queries x k <= 400; RAGFIN_FUSED_MAX_NQ /
 // RAGFIN_FUSED_MAX_NQK override them (the wider configurations stay compiled in and tested).
-static FusedPlan plan_fused(const ragfin* h, int nb, int k) {
+static FusedPlan plan_fused(int sweep_dt, int ld, int max_nq, int max_nqk, int stage_cap, int nb, int k) {
     FusedPlan best;
-    if (nb < 1 || nb > (h->fused_max_nq < kFMaxQ ? h->fused_max_nq : kFMaxQ) || k > kFMaxK || (int64_t)nb * k > h->fused_max_nqk) return best;
-    const int es = (int)esize(h->sweep_dt);
+    if (nb < 1 || nb > (max_nq < kFMaxQ ? max_nq : kFMaxQ) || k > kFMaxK || (int64_t)nb * k > max_nqk) return best;
+    const int es = (int)esize(sweep_dt);
     const int k_elems = kGKBytes / es;
-    const int nkb = (h->ld + k_elems - 1) / k_elems;
+    const int nkb = (ld + k_elems - 1) / k_elems;
     const int pend = nb <= 16 ? 64 : 32;
-    const bool can_split = h->sweep_dt != 0;
+    const bool can_split = sweep_dt != 0;
     // candidates in order of preference: split (tight error bound) first, then plain
     const int cols_split[3] = {16, 32, 64}, cols_plain[3] = {16, 32, 64};
     for (int pass = 0; pass < 2; ++pass) {
@@ -1399,11 +1402,11 @@ static FusedPlan plan_fused(const ragfin* h, int nb, int k) {
         for (int ci = 0; ci < 3; ++ci) {
             const int ncol = split ? cols_split[ci] : cols_plain[ci];
             if ((split ? ncol / 2 : ncol) < nb) continue;
-            for (int stages = h->fused_stage_cap; stages >= 2; --stages) {
+            for (int stages = stage_cap; stages >= 2; --stages) {
                 const size_t smem = fused_smem_bytes(nkb, ncol, stages, nb, k, pend);
                 if (smem > (size_t)227 * 1024) continue;
                 const size_t region = (size_t)nkb * ncol * kGKBytes + (size_t)stages * kBBytes;
-                const size_t hdr = (((size_t)((h->ld + 3) / 4 * 4) * 4 + 256 * 4 + 16 + 15) / 16) * 16;
+                const size_t hdr = (((size_t)((ld + 3) / 4 * 4) * 4 + 256 * 4 + 16 + 15) / 16) * 16;
                 if (region < hdr + 4096 * sizeof(u64)) continue;      // the finalize's scratch (rows within 2 eps of the k-th score)
                 // every CTA appends ~k rows of its first tile, so the buffer scales with k (148 CTAs x 128 = 19 k rows)
                 const int cap = k <= 16 ? kAppendCap : 4 * kAppendCap;
@@ -1415,6 +1418,29 @@ static FusedPlan plan_fused(const ragfin* h, int nb, int k) {
         }
     }
     return best;
+}
+static FusedPlan plan_fused(const ragfin* h, int nb, int k) {
+    return plan_fused(h->sweep_dt, h->ld, h->fused_max_nq, h->fused_max_nqk, h->fused_stage_cap, nb, k);
+}
+
+// Query term of the one-kernel search's eps: |approx - exact| <= |q - hi - lo|_2 * max |stored row|_2 + the accumulation
+// allowance, where the query enters the MMA as hi = RNE(q) (plain) or hi + lo with lo = RNE(q - hi) (split; q - hi is exact
+// in fp32).  Round to nearest with p significant bits is off by at most half an ulp, 2^-p |y| (bf16 p = 8, fp16 p = 11).
+// Split: with 2^e <= |y|, |q - hi| <= 2^(e-p); either it equals 2^(e-p) (then lo = q - hi exactly) or it lies at least one
+// binade lower, where lo is off by at most 2^(e-2p-1) <= 2^-(2p+1) |y|.  Subnormal results lose relative accuracy: at most
+// half the subnormal spacing more per element, absolute (fp16 2^-25, bf16 2^-134).
+// Per element |q_i - hi_i (- lo_i)| <= rel |q_i| + sub, so |q - hi (- lo)|_2 <= rel |q|_2 + sub sqrt(ld); |q|_2 <= 1 + 2^-22
+// and |row|_2 <= 1 + 2^-8: factor 1.0078125.  fp32 sweeps (kind::tf32) have no query term here: eps_gemm_const charges the
+// operand truncation.  tests/test_query_rounding_cpu.py checks rel and sub on every fp32 value of the binades that matter.
+static void fused_query_rounding(int sweep_dt, bool split, double* rel, double* sub) {
+    *rel = sweep_dt == 0 ? 0.0 : sweep_dt == 1 ? (split ? 0x1p-17 : 0x1p-8) : (split ? 0x1p-23 : 0x1p-11);
+    *sub = sweep_dt == 0 ? 0.0 : sweep_dt == 1 ? 0x1p-134 : 0x1p-25;
+}
+static float eps_fused_query(int sweep_dt, bool split, int ld) {
+    double rel, sub;
+    fused_query_rounding(sweep_dt, split, &rel, &sub);
+    if (rel == 0.0) return 0.f;
+    return nextafterf((float)((rel + sub * sqrt((double)ld)) * 1.0078125), INFINITY);
 }
 
 static bool fused_eligible(const ragfin* h, int nb, int k) {
@@ -1483,6 +1509,7 @@ static int run_fused(ragfin* h, const float* q_dev, int nb, int k, int64_t n_eff
     a.cand = (u64*)((char*)h->fcand.p + half * cand_half); a.cap = f.cap;
     a.ctl = (FusedCtl*)h->fctl.p + half;
     a.eps_const = eps_approx(h);
+    a.eps_query = eps_fused_query(h->sweep_dt, f.split, h->ld);
     a.id_base = h->id_base;
     a.out_ids = (long long*)out_ids; a.out_scores = out_scores;
     a.flags = (int*)h->fflags.p + half * (kFMaxQ + 1); a.flag_count = a.flags + kFMaxQ;
@@ -2040,6 +2067,25 @@ extern "C" int ragfin_debug_plan(int32_t nq, int64_t n_rows, int32_t num_sms, in
     if (bound) bound_geometry(n_tiles, append ? k : kp, append, QT0, k, &nblk, &g, &bstride);
     const int64_t v[10] = {C, p.QT, p.S, p.rows_per_slice, p.grid, append, bound, nblk, g, bstride};
     for (int i = 0; i < 10; ++i) out[i] = v[i];
+    return RAGFIN_OK;
+}
+
+// Test hook, pure host arithmetic (no device needed): what the one-kernel search does for nq queries, top-k, on a collection
+// of `dtype` (public code) and `dim`, with the query limits max_nq / max_nqk (0: the defaults, 16 and 400) and the default
+// ring depth.  out[5] = {ncol (0: the shape does not take it), split, stages, pend, cap}; out_eps[4] = {rel, sub (the
+// per-element query-rounding bound rel |y| + sub), query term, eps_approx} for the variant planned (the plain one if none is).
+extern "C" int ragfin_debug_fused_plan(int32_t dtype, int32_t dim, int32_t nq, int32_t k, int32_t max_nq, int32_t max_nqk,
+                                       int64_t* out, double* out_eps) {
+    if (!out || !out_eps || dtype < 0 || dtype > 3 || dim < 1 || dim > 65536 || nq < 1 || k < 1 || max_nq < 0 || max_nq > kFMaxQ || max_nqk < 0)
+        return fail(RAGFIN_EINVAL, "bad argument");
+    const int ld = (dim + 7) / 8 * 8;
+    const int sweep_dt = dtype == RAGFIN_F32_F16 ? RAGFIN_F16 : dtype;
+    const FusedPlan f = plan_fused(sweep_dt, ld, max_nq ? max_nq : kFusedMaxNq, max_nqk ? max_nqk : kFusedMaxNqk, kRMaxStages, nq, k);
+    const int64_t v[5] = {f.ncol, f.split, f.stages, f.pend, f.cap};
+    for (int i = 0; i < 5; ++i) out[i] = v[i];
+    fused_query_rounding(sweep_dt, f.split, &out_eps[0], &out_eps[1]);
+    out_eps[2] = eps_fused_query(sweep_dt, f.split, ld);
+    out_eps[3] = eps_approx(sweep_dt, ld, dtype == RAGFIN_F32_F16 ? eps_sweep_const(ld) : 0.f);
     return RAGFIN_OK;
 }
 

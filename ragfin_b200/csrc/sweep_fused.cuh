@@ -10,7 +10,8 @@
 //              then all threads scale 16-byte chunks exactly as ingest does and store them straight into shared memory in the
 //              tensor core's K-major SWIZZLE_128B layout, while the TMA producer already has a ring-full of corpus bytes in
 //              flight.  16-bit storage: every query enters as TWO columns, hi = round(q) and lo = round(q - hi), summed in
-//              the epilogue, so the query term of the error bound drops from ~1.6e-3 to an a-priori 2^-18 (SPLIT).
+//              the epilogue, so the query term of the error bound drops from 2^-8 (hi alone) to an a-priori 2^-17 (SPLIT,
+//              bf16; fp16: 2^-11 and 2^-23), computed on the host (eps_fused_query) and passed in FusedArgs::eps_query.
 //   sweep      as gemm_rows.cuh: corpus rows are the MMA's M (two 128-row halves per 256-row tile), the query block its
 //              N = 16 / 32 / 64, P partial accumulators per half so that no MMA waits on its predecessor.  Tiles of a slice are
 //              visited in a strided permutation starting mid-slice, so a corpus sorted by similarity cannot make every row
@@ -104,6 +105,7 @@ struct FusedArgs {
     int cap;
     FusedCtl* ctl;
     float eps_const;            // accumulation allowance (+ tf32 truncation, + the fp16 copy's rounding), see eps_approx
+    float eps_query;            // query-rounding term of this variant (plain or split), see eps_fused_query
     long long id_base;
     long long* out_ids;         // [nq][k]
     float* out_scores;          // [nq][k]
@@ -448,18 +450,9 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
         }
         __syncthreads();
         // |approx - exact| <= |q - hi - lo|_2 * max |stored row|_2 + the accumulation allowance.  The residual is bounded a
-        // priori, element by element (round to nearest: half an ulp): bf16 keeps 8 significant bits, so |q - hi| <= 2^-9 |q|
-        // and |q - hi - lo| <= 2^-18 |q|; fp16 keeps 11 (2^-12, 2^-24) but loses relative accuracy below 2^-14, where the
-        // spacing is 2^-24: at most 2^-25 more per element.  |q|_2 <= 1 + 2^-22 and |row|_2 <= 1 + 2^-8: factor 1.0078125.
-        {
-            float eq = 0.f;
-            if (KIND != 1) {
-                const float rel = a.sdt == 1 ? (SPLIT ? 3.814697265625e-06f : 1.953125e-03f) : (SPLIT ? 5.9604644775390625e-08f : 2.44140625e-04f);
-                const float sub = a.sdt == 1 ? 0.f : __fmul_ru(__fsqrt_ru((float)a.ld), 2.98023223876953125e-08f);
-                eq = __fmul_ru(__fadd_ru(rel, sub), 1.0078125f);
-            }
-            for (int j = tid; j < nq; j += kFThreads) eps_s[j] = __fadd_ru(a.eps_const, eq);
-        }
+        // priori, element by element, on the host (eps_fused_query: half an ulp of each rounding, 2^-8 |q| for bf16 hi alone,
+        // 2^-17 |q| for hi + lo; fp16 2^-11 and 2^-23, plus half the subnormal spacing).
+        for (int j = tid; j < nq; j += kFThreads) eps_s[j] = __fadd_ru(a.eps_const, a.eps_query);
         __syncthreads();
         for (int i = tid; i < 2 * kFMaxQ + 2; i += kFThreads) pend[i] = 0u;   // the parking area goes back to the pending lists
         fence_proxy_async_smem();   // generic-proxy writes above -> visible to the tensor core's async-proxy reads

@@ -445,6 +445,19 @@ class Index:
                 "cand_per_query": s.cand_per_query}
 
 
+def fused_plan(dtype: str, dim: int, nq: int, k: int, max_nq: int = 0, max_nqk: int = 0) -> dict:
+    """What the one-kernel search does for nq queries and top-k on a `dtype` collection of `dim` (no device needed; include/
+    ragfin.h, ragfin_debug_fused_plan): ncol (0: another path serves the shape), split (the query enters as hi + lo), stages,
+    pend, cap, and its eps split into the per-element query-rounding bound rel |y| + sub, the query term and eps_approx.
+    max_nq / max_nqk: the handle's query limits (0: the defaults)."""
+    L = _lib.load()
+    out, eps = (ctypes.c_int64 * 5)(), (ctypes.c_double * 4)()
+    _lib.check(L.ragfin_debug_fused_plan(DTYPE_CODE[dtype], int(dim), int(nq), int(k), int(max_nq), int(max_nqk), out, eps))
+    plan = dict(zip(("ncol", "split", "stages", "pend", "cap"), (int(v) for v in out)))
+    plan.update(zip(("rel", "sub", "eps_query", "eps_approx"), (float(v) for v in eps)))
+    return plan
+
+
 def merge_topk(ids, scores, parts: int, k: int, stream=None, out_ids=None, out_scores=None):
     """Cross-shard reduce of exact hit lists (torch CUDA tensors, ids int64 / scores fp32).
 

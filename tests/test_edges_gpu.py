@@ -8,7 +8,8 @@ magnitudes, and NaN / Inf components (stored and searched as zero vectors).
 
 Fallbacks are predicted per query from the oracle's exact scores S and each path's own eps, computed as the library computes
 it (eps_gemm_const / eps_sweep_const / eps_fp32_accumulate in csrc/ragfin_api.cu; eps_q of prep_queries_kernel from the
-oracle's normalised query; the one-kernel search's a-priori query term).  The approximate error is taken as at most eps / 2:
+oracle's normalised query; the one-kernel search's a-priori query term of the variant the cell runs, from
+ragfin_debug_fused_plan).  The approximate error is taken as at most eps / 2:
 test_tensor_core_error_stays_inside_the_allowance holds it below eps / 4.  With S_k the k-th exact score:
   * a cut T - 2 eps keeps every row with S >= S_k - eps for certain and no row below S_k - 3 eps;
   * the bound pass is simulated on the exact scores (bound_geometry: 256-row tiles, the rank-th largest sampled block maximum),
@@ -173,15 +174,13 @@ def _eps_q(qh, dtype):
     return np.sqrt((d * d).sum(axis=1)) * 1.0078125 + 1e-9
 
 
-def _eps_fused(dtype, ld):
-    """(smallest, largest) eps of the one-kernel search: the query enters as hi + lo (split) or hi alone (plain)."""
-    base = _eps_approx(dtype, ld)
-    if dtype == "f32":
-        return base, base
-    if dtype == "bf16":
-        return base + 3.814697265625e-06 * 1.0078125, base + 1.953125e-03 * 1.0078125
-    sub = np.sqrt(ld) * 2.98023223876953125e-08
-    return base + (5.9604644775390625e-08 + sub) * 1.0078125, base + (2.44140625e-04 + sub) * 1.0078125
+def _eps_fused(dtype, dim, nq, k):
+    """eps of the one-kernel search for the variant this shape takes (split: the query enters as hi + lo; plain: hi alone),
+    as the library plans it (ragfin_debug_fused_plan)."""
+    from ragfin_b200.engine import fused_plan
+    p = fused_plan(dtype, dim, nq, k)
+    assert p["ncol"], p
+    return p["eps_approx"] + p["eps_query"]
 
 
 def _bound_threshold(S, k, nq):
@@ -212,8 +211,8 @@ def _predict(c, nq, k, rule, S=None):
     u = 2.5e-7
     count = lambda t: (S >= t[:, None]).sum(axis=1)                 # noqa: E731
     if rule == "fused":
-        lo, hi = _eps_fused(c.dtype, ld)
-        c_in, c_poss = count(Sk - lo), count(Sk - 3 * hi - u)
+        eps = _eps_fused(c.dtype, c.dim, nq, k)
+        c_in, c_poss = count(Sk - eps), count(Sk - 3 * eps - u)
         return [True if a > 16384 else False if b <= 8192 else None for a, b in zip(c_in, c_poss)], c_in
     eps = _eps_approx(c.dtype, ld) + c.eps_q[:nq] if rule != "scan" else np.full(nq, (ld + 64) * 2.0 ** -24 * 1.0625 + 2.0 ** -21)
     c_in, c_poss = count(Sk - eps), count(Sk - 3 * eps - u)
