@@ -338,6 +338,21 @@ int ragfin_set_fused(ragfin_t* h, int32_t enable, int64_t min_rows);
  * Replaces: nothing in the reference (its searches are sequential gRPC calls - vector_rag_mcp/main.py:51-57). */
 int ragfin_set_pipelined(ragfin_t* h, int32_t enable);
 
+/* The one-kernel search's int8 tile filter on bf16 / fp16 collections (csrc/sweep_fused.cuh, DESIGN.md 2.5): tiles are first
+ * swept from an int8 copy of the rows (half the bytes) with a rigorous bound on each row's 16-bit score, and read in 16 bits
+ * only where some row can reach a query's threshold.  The copy ([capacity] x ceil16(dim) int8 + 8 bytes per row) is made
+ * by the first one-kernel search that uses it and kept current by the searches after ragfin_add / ragfin_reserve /
+ * ragfin_compact; files do not change.  mode 1 = on, 0 = off, RAGFIN_SWEEP_COPY_AUTO (default) = on from 2^20 rows.
+ * Results are identical either way; a copy that cannot be allocated leaves the search on the 16-bit rows. */
+#define RAGFIN_SWEEP_COPY_AUTO (-1)
+int ragfin_set_sweep_copy(ragfin_t* h, int32_t mode);
+/* Test hook: rows [row0, row0 + n) of the int8 copy, out_rows_host [n][*ld8_out] int8, and their {scale, residual bound},
+ * out_side_host [n][2] float.  RAGFIN_EUNSUPPORTED when the collection has no copy.  Synchronises. */
+int ragfin_debug_sweep_copy(ragfin_t* h, int64_t row0, int64_t n, int8_t* out_rows_host, float* out_side_host, int32_t* ld8_out);
+/* Diagnostics of the last one-kernel search, out[2]: 256-row tiles read in 16 bits (every CTA's first tile and the refined
+ * ones; without the int8 filter, all) and tiles screened from the int8 copy.  Synchronises. */
+int ragfin_debug_fused_tiles(ragfin_t* h, int64_t* out);
+
 /* Test / bench hook: per-query diagnostics of the last one-kernel search on this handle - rows appended to the query's
  * buffer during the sweep and rows rescored exactly by the finalize (-1: the buffer overflowed and the query was answered
  * by the in-kernel exact scan).  Synchronises. */

@@ -19,7 +19,7 @@ SYMBOLS = (
     "ragfin_abi_version", "ragfin_create", "ragfin_create_view", "ragfin_add", "ragfin_add_synthetic", "ragfin_add_synthetic_topics", "ragfin_count", "ragfin_reserve",
     "ragfin_delete", "ragfin_live_count", "ragfin_read_live_mask", "ragfin_compact",
     "ragfin_set_id_base", "ragfin_search", "ragfin_search_host", "ragfin_search_filtered", "ragfin_search_filtered_host", "ragfin_search_range", "ragfin_search_range_host", "ragfin_search_grouped", "ragfin_search_grouped_host", "ragfin_merge_topk", "ragfin_read_rows", "ragfin_read_sweep_rows",
-    "ragfin_last_search_stats", "ragfin_profile", "ragfin_profile_read", "ragfin_save", "ragfin_load", "ragfin_set_gemm_min_batch", "ragfin_set_gemm_cluster", "ragfin_set_gemm_variant", "ragfin_set_bound_pass", "ragfin_set_scan_variant", "ragfin_set_append_mode", "ragfin_set_fused", "ragfin_set_pipelined", "ragfin_debug_fused_counts", "ragfin_debug_fused_times", "ragfin_debug_fused_ctas", "ragfin_debug_fused_tile_order", "ragfin_debug_gemm_scores", "ragfin_debug_plan", "ragfin_debug_fused_plan", "ragfin_destroy", "ragfin_last_error",
+    "ragfin_last_search_stats", "ragfin_profile", "ragfin_profile_read", "ragfin_save", "ragfin_load", "ragfin_set_gemm_min_batch", "ragfin_set_gemm_cluster", "ragfin_set_gemm_variant", "ragfin_set_bound_pass", "ragfin_set_scan_variant", "ragfin_set_append_mode", "ragfin_set_fused", "ragfin_set_pipelined", "ragfin_set_sweep_copy", "ragfin_debug_sweep_copy", "ragfin_debug_fused_tiles", "ragfin_debug_fused_counts", "ragfin_debug_fused_times", "ragfin_debug_fused_ctas", "ragfin_debug_fused_tile_order", "ragfin_debug_gemm_scores", "ragfin_debug_plan", "ragfin_debug_fused_plan", "ragfin_destroy", "ragfin_last_error",
     "ragfin_exchange_create", "ragfin_exchange_handle", "ragfin_exchange_connect", "ragfin_exchange_allgather_merge", "ragfin_fused_eligible", "ragfin_search_sharded", "ragfin_search_sharded_host", "ragfin_exchange_destroy",
 )
 
@@ -92,6 +92,9 @@ def load() -> ctypes.CDLL:
     L.ragfin_set_append_mode.argtypes = [vp, i32]
     L.ragfin_set_fused.argtypes = [vp, i32, i64]
     L.ragfin_set_pipelined.argtypes = [vp, i32]
+    L.ragfin_set_sweep_copy.argtypes = [vp, i32]
+    L.ragfin_debug_sweep_copy.argtypes = [vp, i64, i64, vp, vp, ctypes.POINTER(i32)]
+    L.ragfin_debug_fused_tiles.argtypes = [vp, vp]
     L.ragfin_debug_fused_counts.argtypes = [vp, i32, vp, vp]
     L.ragfin_debug_fused_times.argtypes = [vp, vp]
     L.ragfin_debug_fused_ctas.argtypes = [vp, vp, vp]

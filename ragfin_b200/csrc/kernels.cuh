@@ -828,4 +828,51 @@ __global__ void exchange_merge_kernel(const char* area, const uint32_t* flags, i
                     (int64_t)(record_bytes / 8), (int64_t)(record_bytes / 4), (int64_t)k, out_ids, out_scores);
 }
 
+// int8 screen copy of 16-bit rows for the one-kernel search's tile filter (sweep_fused.cuh, DESIGN.md 2.5), one warp per
+// row: x ~ s * x8 with s = max |x_i| / 127, x8_i = clamp(rint(x_i / s), -127, 127), and e >= |x - s x8|_2 (fp64, every step
+// rounded up; x_i - s x8_i itself is exact in fp64: both terms are multiples of 2^-33 s unless x8_i = 0, and span < 53 bits).
+// Components far below the maximum become 0 and their whole value is charged to e.  A zero row and a row with a non-finite
+// component (never appended by the 16-bit sweep either) get x8 = 0, s = e = 0.  Padding columns [ld, ld8) are written 0.
+template <int DT>
+__global__ void quantize_i8_kernel(const typename Store<DT>::T* __restrict__ data, int ld, long long row0, long long n,
+                                   int8_t* __restrict__ q8, int ld8, float2* __restrict__ side) {
+    const int lane = threadIdx.x & 31;
+    const long long w0 = ((long long)blockIdx.x * blockDim.x + threadIdx.x) >> 5, nw = ((long long)gridDim.x * blockDim.x) >> 5;
+    const int nv = ld / 8;                                   // 16-byte vectors of a stored row
+    for (long long r = row0 + w0; r < row0 + n; r += nw) {
+        const uint4* src = reinterpret_cast<const uint4*>(data + (size_t)r * ld);
+        float mx = 0.f;
+        bool fin = true;
+        for (int v = lane; v < nv; v += kWarp) {
+            float f[8];
+            Store<DT>::unpack(ldg_stream(src + v), f);
+#pragma unroll
+            for (int e = 0; e < 8; ++e) { fin = fin && isfinite(f[e]); mx = fmaxf(mx, fabsf(f[e])); }
+        }
+#pragma unroll
+        for (int off = 16; off >= 1; off >>= 1) mx = fmaxf(mx, __shfl_xor_sync(kFull, mx, off));
+        const bool live = __all_sync(kFull, fin) && mx > 0.f;
+        const float s = live ? mx / 127.0f : 0.f, rs = live ? 127.0f / mx : 0.f;
+        double d2 = 0.0;
+        uint2* dst = reinterpret_cast<uint2*>(q8 + (size_t)r * ld8);
+        for (int v = lane; v < nv; v += kWarp) {
+            float f[8];
+            Store<DT>::unpack(src[v], f);
+            uint32_t w[2] = {0u, 0u};
+#pragma unroll
+            for (int e = 0; e < 8; ++e) {
+                const float qf = live ? fminf(fmaxf(rintf(f[e] * rs), -127.f), 127.f) : 0.f;
+                const double d = (double)f[e] - (double)s * (double)qf;
+                if (live) d2 = __dadd_ru(d2, __dmul_ru(d, d));
+                w[e >> 2] |= ((uint32_t)(uint8_t)(int8_t)qf) << (8 * (e & 3));
+            }
+            dst[v] = make_uint2(w[0], w[1]);
+        }
+        if (lane == 0 && ld8 > ld) dst[nv] = make_uint2(0u, 0u);   // ld8 - ld is 0 or 8
+#pragma unroll
+        for (int off = 16; off >= 1; off >>= 1) d2 = __dadd_ru(d2, __shfl_xor_sync(kFull, d2, off));
+        if (lane == 0) side[r] = make_float2(s, live ? __double2float_ru(__dsqrt_ru(d2)) : 0.f);
+    }
+}
+
 }  // namespace rfk

@@ -123,6 +123,16 @@ struct ragfin {
     bool have_pending = false;            // pipelined searches enqueued on pending_stream since the last event record
     cudaStream_t pending_stream = nullptr;
     ragfin_search_stats stats = {0, 0, 0, 0};
+    // int8 screen copy of the one-kernel search's tile filter (DESIGN.md 2.5), bf16 / fp16 collections: [i8_cap][ld8] int8 rows
+    // and a {scale, residual bound} per row, rows [0, i8_rows) current.  Made at the first one-kernel search that wants it and
+    // brought up to `count` by the next one after rows were added (an ordinary kernel in front of that launch); dropped by
+    // compaction (rows move) and rebuilt when the capacity outgrows it.  A view shares its parent's copy when that covers it.
+    int sweep_copy = RAGFIN_SWEEP_COPY_AUTO;   // ragfin_set_sweep_copy
+    int8_t* i8 = nullptr;
+    float2* i8side = nullptr;
+    int ld8 = 0;
+    int64_t i8_cap = 0, i8_rows = 0;
+    bool i8_owned = false;
     // measurement hook (ragfin_profile): event pairs around the dominant kernel
     bool profiling = false;
     static const int kProfPairs = 512;
@@ -149,6 +159,15 @@ static int public_dtype(const ragfin* h) { return has_copy(h) ? RAGFIN_F32_F16 :
 static float eps_sweep_const(int ld) {
     const double e = (1.0 + 2.384185791015625e-07) * (4.8828125e-04 * (1.0 + 9.5367431640625e-07) + 2.98023223876953125e-08 * sqrt((double)ld));
     return nextafterf((float)e, INFINITY);
+}
+
+static void i8_free(ragfin* h) {
+    if (h->i8_owned) {
+        (void)cudaDeviceSynchronize();   // no search may still be reading it
+        cudaFree(h->i8);
+        cudaFree(h->i8side);
+    }
+    h->i8 = nullptr; h->i8side = nullptr; h->i8_cap = 0; h->i8_rows = 0; h->i8_owned = false;
 }
 
 static int ensure(Buf& b, size_t bytes) {
@@ -281,6 +300,10 @@ extern "C" int ragfin_create_view(ragfin_t* parent, ragfin_t** out) {
     h->use_fused = parent->use_fused; h->use_bigk_batched = parent->use_bigk_batched; h->fused_min_rows = parent->fused_min_rows;
     h->fused_max_nq = parent->fused_max_nq; h->fused_max_nqk = parent->fused_max_nqk; h->allow_pipelined = parent->allow_pipelined;
     h->fused_refresh_every = parent->fused_refresh_every; h->fused_stage_cap = parent->fused_stage_cap;
+    h->sweep_copy = parent->sweep_copy;
+    if (parent->i8 && parent->i8_rows >= h->count) {   // the rows of a view never change: its parent's copy stays valid for them
+        h->i8 = parent->i8; h->i8side = parent->i8side; h->ld8 = parent->ld8; h->i8_cap = parent->i8_cap; h->i8_rows = h->count;
+    }
     read_env_knobs(h);
     cudaError_t e = cudaEventCreateWithFlags(&h->last_done, cudaEventDisableTiming);
     if (e != cudaSuccess) {
@@ -314,6 +337,7 @@ extern "C" void ragfin_destroy(ragfin_t* h) {
     Buf* bufs[] = {&h->qhat, &h->q16, &h->eps_q, &h->gtau, &h->bmax, &h->acnt, &h->athr, &h->awin, &h->allow, &h->bk_scores, &h->bk_state, &h->bk_keys, &h->bk_rows, &h->grp, &h->grp_codes, &h->cand, &h->cand_e, &h->flags, &h->stage_q, &h->stage_ids, &h->stage_scores, &h->add_stage, &h->fctl, &h->fcand, &h->fqn, &h->fflags};
     for (Buf* b : bufs)
         if (b->p) cudaFree(b->p);
+    i8_free(h);
     if (h->sweep_data && has_copy(h) && !h->is_view) cudaFree(h->sweep_data);
     if (h->data && !h->is_view) cudaFree(h->data);
     if (h->live_dev) cudaFree(h->live_dev);
@@ -476,6 +500,7 @@ extern "C" int ragfin_compact(ragfin_t* h) {
     h->live_host.swap(ones);
     h->count = live;
     h->n_dead = 0;
+    i8_free(h);   // rows moved: the next one-kernel search that wants the int8 copy rebuilds it
     for (ragfin::MapSlot& m : h->map_cache) m = ragfin::MapSlot();   // tensor maps of the old matrix are stale
     return RAGFIN_OK;
 }
@@ -882,15 +907,18 @@ static encode_tiled_fn get_encode_tiled() {
     return fn;
 }
 
+static const int kMapI8 = 4;   // make_map dtype of the int8 screen copy
 // [rows, ld] row-major matrix of `dtype`; box = 128 bytes of K x box_rows rows, 128-byte swizzle, zero OOB fill
 static int make_map(CUtensorMap* map, int dtype, const void* base, int64_t rows, int ld, int box_rows) {
     encode_tiled_fn enc = get_encode_tiled();
     if (!enc) return fail(RAGFIN_ECUDA, "cuTensorMapEncodeTiled is not available from the driver");
     const CUtensorMapDataType dt = dtype == 0 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32
-                                   : dtype == 1 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+                                   : dtype == 1 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16
+                                   : dtype == 2 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_UINT8;
+    const size_t es = dtype == kMapI8 ? 1 : esize(dtype);
     const cuuint64_t dims[2] = {(cuuint64_t)ld, (cuuint64_t)rows};
-    const cuuint64_t strides[1] = {(cuuint64_t)ld * esize(dtype)};
-    const cuuint32_t box[2] = {(cuuint32_t)(kGKBytes / esize(dtype)), (cuuint32_t)box_rows};
+    const cuuint64_t strides[1] = {(cuuint64_t)ld * es};
+    const cuuint32_t box[2] = {(cuuint32_t)(kGKBytes / es), (cuuint32_t)box_rows};
     const cuuint32_t estr[2] = {1, 1};
     CUresult r = enc(map, dt, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                      CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -1386,8 +1414,10 @@ struct FusedPlan {
 // that its per-query bookkeeping in the first tile and the finalize outweigh the launches it saves (32 queries: 0.383 vs 0.343;
 // 16 queries at k = 100: 0.504 vs 0.416).  Default limits: <= 16 queries and queries x k <= 400; RAGFIN_FUSED_MAX_NQ /
 // RAGFIN_FUSED_MAX_NQK override them (the wider configurations stay compiled in and tested).
-static FusedPlan plan_fused(int sweep_dt, int ld, int max_nq, int max_nqk, int stage_cap, int nb, int k) {
+// i8: the plan of the int8 tile filter (split only; its query block and state take shared memory too).
+static FusedPlan plan_fused(int sweep_dt, int ld, int max_nq, int max_nqk, int stage_cap, int nb, int k, bool i8 = false) {
     FusedPlan best;
+    const int nkb8 = ((ld + 15) / 16 * 16 + kGKBytes - 1) / kGKBytes;
     if (nb < 1 || nb > (max_nq < kFMaxQ ? max_nq : kFMaxQ) || k > kFMaxK || (int64_t)nb * k > max_nqk) return best;
     const int es = (int)esize(sweep_dt);
     const int k_elems = kGKBytes / es;
@@ -1399,11 +1429,13 @@ static FusedPlan plan_fused(int sweep_dt, int ld, int max_nq, int max_nqk, int s
     for (int pass = 0; pass < 2; ++pass) {
         const bool split = pass == 0;
         if (split && !can_split) continue;
+        if (i8 && !split) continue;
         for (int ci = 0; ci < 3; ++ci) {
             const int ncol = split ? cols_split[ci] : cols_plain[ci];
             if ((split ? ncol / 2 : ncol) < nb) continue;
             for (int stages = stage_cap; stages >= 2; --stages) {
-                const size_t smem = fused_smem_bytes(nkb, ncol, stages, nb, k, pend);
+                const size_t smem = fused_smem_bytes(nkb, ncol, stages, nb, k, pend) +
+                                    (i8 ? (size_t)nkb8 * ncol * kGKBytes + sizeof(FusedI8State) + 16 : 0);
                 if (smem > (size_t)227 * 1024) continue;
                 const size_t region = (size_t)nkb * ncol * kGKBytes + (size_t)stages * kBBytes;
                 const size_t hdr = (((size_t)((ld + 3) / 4 * 4) * 4 + 256 * 4 + 16 + 15) / 16) * 16;
@@ -1443,15 +1475,64 @@ static float eps_fused_query(int sweep_dt, bool split, int ld) {
     return nextafterf((float)((rel + sub * sqrt((double)ld)) * 1.0078125), INFINITY);
 }
 
+// fp32 evaluation of the int8 score w = (s sq) (H + L / 256) in the kernel: five roundings (two int -> float conversions,
+// the add, two products) of 2^-24 each on terms bounded by (sq |hi|_2 + sq |lo|_2 / 256) (s |x8|_2), where s |x8|_2 <=
+// |x|_2 + e <= 1.0078125 (1 + sqrt(ld) / 254) and sq |hi|_2 + sq |lo|_2 / 256 <= 1 + 2^-20 + sqrt(ld) / 127.  Rounded up.
+static float eps_i8_conv(int ld) {
+    const double r = sqrt((double)ld);
+    const double e = 5.01 * 0x1p-24 * 1.0078125 * (1.0 + r / 250.0) * (1.00001 + r / 125.0);
+    return nextafterf((float)e, INFINITY);
+}
+
+// Rows from which a collection's one-kernel search screens tiles with the int8 copy (RAGFIN_SWEEP_COPY_AUTO)
+static const int64_t kI8MinRows = (int64_t)1 << 20;
+static bool i8_wanted(const ragfin* h) {
+    if (h->sweep_copy == 0 || has_copy(h) || (h->dtype != RAGFIN_BF16 && h->dtype != RAGFIN_F16)) return false;
+    return h->sweep_copy == 1 || h->count >= kI8MinRows;
+}
+// Bring the int8 copy up to `count` rows (kernel on st).  Returns false when it cannot be allocated: the search then sweeps
+// the 16-bit rows.  *built: a kernel was enqueued in front of the search.
+static bool i8_prepare(ragfin* h, cudaStream_t st, bool* built) {
+    *built = false;
+    if (h->i8 && h->i8_owned && h->i8_cap < h->capacity) i8_free(h);   // ragfin_reserve grew the collection
+    if (!h->i8) {
+        const int64_t cap = h->capacity;
+        h->ld8 = (h->ld + 15) / 16 * 16;
+        cudaError_t e = cudaMalloc(&h->i8, (size_t)cap * h->ld8);
+        if (e == cudaSuccess) e = cudaMalloc(&h->i8side, (size_t)cap * sizeof(float2));
+        if (e != cudaSuccess) {
+            (void)cudaGetLastError();
+            if (h->i8) cudaFree(h->i8);
+            h->i8 = nullptr; h->i8side = nullptr;
+            return false;
+        }
+        h->i8_cap = cap; h->i8_rows = 0; h->i8_owned = true;
+    }
+    if (h->i8_rows < h->count) {
+        const int64_t n = h->count - h->i8_rows, wpb = 8;
+        const int64_t want = (n + wpb - 1) / wpb, cap_blocks = (int64_t)h->num_sms * 16;
+        const int blocks = (int)(want < cap_blocks ? want : cap_blocks);
+        if (h->dtype == RAGFIN_BF16)
+            quantize_i8_kernel<1><<<blocks, wpb * 32, 0, st>>>((const __nv_bfloat16*)h->data, h->ld, h->i8_rows, n, h->i8, h->ld8, h->i8side);
+        else
+            quantize_i8_kernel<2><<<blocks, wpb * 32, 0, st>>>((const __half*)h->data, h->ld, h->i8_rows, n, h->i8, h->ld8, h->i8side);
+        if (cudaGetLastError() != cudaSuccess) return false;
+        h->i8_rows = h->count;
+        *built = true;
+    }
+    return true;
+}
+
 static bool fused_eligible(const ragfin* h, int nb, int k) {
     return h->use_fused && h->count >= h->fused_min_rows && gemm_rows_ok(h) && plan_fused(h, nb, k).ncol != 0;
 }
 
-typedef void (*fused_fn)(const CUtensorMap, const FusedArgs, const FusedInlineQ);
-static fused_fn pick_fused(int dtype, int ncol, bool split) {
-    if (dtype == 0) return ncol == 16 ? sweep_fused_kernel<1, 16, false> : ncol == 32 ? sweep_fused_kernel<1, 32, false> : sweep_fused_kernel<1, 64, false>;
-    if (split) return ncol == 16 ? sweep_fused_kernel<0, 16, true> : ncol == 32 ? sweep_fused_kernel<0, 32, true> : sweep_fused_kernel<0, 64, true>;
-    return ncol == 16 ? sweep_fused_kernel<0, 16, false> : ncol == 32 ? sweep_fused_kernel<0, 32, false> : sweep_fused_kernel<0, 64, false>;
+typedef void (*fused_fn)(const CUtensorMap, const FusedArgs, const FusedInlineQ, const CUtensorMap);
+static fused_fn pick_fused(int dtype, int ncol, bool split, bool i8) {
+    if (dtype == 0) return ncol == 16 ? sweep_fused_kernel<1, 16, false, false> : ncol == 32 ? sweep_fused_kernel<1, 32, false, false> : sweep_fused_kernel<1, 64, false, false>;
+    if (i8) return ncol == 16 ? sweep_fused_kernel<0, 16, true, true> : ncol == 32 ? sweep_fused_kernel<0, 32, true, true> : sweep_fused_kernel<0, 64, true, true>;
+    if (split) return ncol == 16 ? sweep_fused_kernel<0, 16, true, false> : ncol == 32 ? sweep_fused_kernel<0, 32, true, false> : sweep_fused_kernel<0, 64, true, false>;
+    return ncol == 16 ? sweep_fused_kernel<0, 16, false, false> : ncol == 32 ? sweep_fused_kernel<0, 32, false, false> : sweep_fused_kernel<0, 64, false, false>;
 }
 
 // pipelined: the asynchronous entry points.  The launch carries programmatic stream serialization and the kernel releases its
@@ -1464,9 +1545,20 @@ static int run_fused(ragfin* h, const float* q_dev, int nb, int k, int64_t n_eff
                      cudaStream_t st, bool pipelined, ragfin_exchange* x = nullptr, uint32_t xstep = 0,
                      const float* q_inline_host = nullptr, uint32_t* host_flag_dev = nullptr, uint32_t host_seq = 0) {
     int rc;
-    const FusedPlan f = plan_fused(h, nb, k);
+    FusedPlan f = plan_fused(h, nb, k);
     if (f.ncol == 0) return fail(RAGFIN_EUNSUPPORTED, "no fused sweep for %d queries, k = %d", nb, k);
     const int64_t n = h->count;
+    // int8 tile filter: same eps, same answers, the 16-bit rows read only for tiles within reach of a threshold
+    bool use8 = false;
+    if (i8_wanted(h)) {
+        const FusedPlan f8 = plan_fused(h->sweep_dt, h->ld, h->fused_max_nq, h->fused_max_nqk, h->fused_stage_cap, nb, k, true);
+        bool built = false;
+        if (f8.ncol == f.ncol && f8.split && i8_prepare(h, st, &built)) {
+            f = f8;
+            use8 = true;
+            if (built) pipelined = false;   // the copy's kernel ran in front of this launch: an ordinary launch
+        }
+    }
     const size_t cand_half = (size_t)kFMaxQ * 4 * kAppendCap * sizeof(u64) / 4;   // per half: up to 16 queries x 65 536 keys (= 64 x 16 384)
     const size_t qn_half = (size_t)kFMaxQ * h->ld * sizeof(float);
     if ((size_t)nb * f.cap * sizeof(u64) > cand_half) return fail(RAGFIN_EUNSUPPORTED, "append buffers of %d queries x %d keys exceed the workspace half", nb, f.cap);
@@ -1481,8 +1573,10 @@ static int run_fused(ragfin* h, const float* q_dev, int nb, int k, int64_t n_eff
     const int half = (int)(seq & 1u);
     h->fused_last = half;
     const GemmPlan p = plan_gemm(nb, n, h->num_sms, 32, 1);
-    CUtensorMap tmB;
+    CUtensorMap tmB, tmB8;
     if ((rc = cached_map(h, &tmB, h->sweep_dt, h->sweep_data, n, h->ld, kGN))) return rc;
+    tmB8 = tmB;
+    if (use8 && (rc = cached_map(h, &tmB8, kMapI8, h->i8, n, h->ld8, kGN))) return rc;
     FusedArgs a;
     a.idesc = make_idesc_n(h->sweep_dt == 0 ? 2 : h->sweep_dt == 1 ? 1 : 0, f.ncol);
     a.k_elems = kGKBytes / (int)esize(h->sweep_dt);
@@ -1518,7 +1612,11 @@ static int run_fused(ragfin* h, const float* q_dev, int nb, int k, int64_t n_eff
         a.xworld = x->world; a.xrank = x->rank; a.xstep = xstep; a.xrec_max = x->record_max;
         a.xpeer_area = x->d_peer_area; a.xpeer_qflag = x->d_peer_qflag;
     }
-    fused_fn fn = pick_fused(h->sweep_dt, f.ncol, f.split);
+    a.idesc8 = make_idesc_i8(f.ncol);
+    a.num_kblocks8 = use8 ? (h->ld8 + kGKBytes - 1) / kGKBytes : 0;
+    a.side8 = use8 ? h->i8side : nullptr;
+    a.i8_conv = eps_i8_conv(h->ld);
+    fused_fn fn = pick_fused(h->sweep_dt, f.ncol, f.split, use8);
     if ((rc = set_dyn_smem(h->device, (const void*)fn, f.smem))) return rc;
     h->fctl_dirty = true;          // until the launch is known to have been accepted
     cudaLaunchConfig_t cfg = {};
@@ -1530,7 +1628,7 @@ static int run_fused(ragfin* h, const float* q_dev, int nb, int k, int64_t n_eff
     static thread_local FusedInlineQ qin;          // 12 KB: copied into the launch only up to what the queries occupy matters
     if (q_inline_host) memcpy(qin.v, q_inline_host, (size_t)nb * h->dim * sizeof(float));
     prof_begin(h, st);
-    CU_TRY(cudaLaunchKernelEx(&cfg, fn, tmB, a, qin));
+    CU_TRY(cudaLaunchKernelEx(&cfg, fn, tmB, a, qin, tmB8));
     prof_end(h, st);
     CU_TRY(cudaGetLastError());
     h->fctl_dirty = false;
@@ -2187,6 +2285,43 @@ extern "C" int ragfin_set_fused(ragfin_t* h, int32_t enable, int64_t min_rows) {
 // ordered before that search, or by the host) - a kernel that produces the queries between two searches needs pipelining off
 // (the default), or its own stream synchronisation.  The corpus, filters and workspaces are the library's own business: a
 // search that follows anything but this handle's previous one-kernel search on the same stream is launched normally.
+extern "C" int ragfin_set_sweep_copy(ragfin_t* h, int32_t mode) {
+    if (!h) return fail(RAGFIN_EINVAL, "NULL handle");
+    if (mode != 0 && mode != 1 && mode != RAGFIN_SWEEP_COPY_AUTO)
+        return fail(RAGFIN_EINVAL, "mode %d is not 0 (off), 1 (on) or RAGFIN_SWEEP_COPY_AUTO (%d)", mode, RAGFIN_SWEEP_COPY_AUTO);
+    std::lock_guard<std::mutex> lk(h->mu);
+    h->sweep_copy = mode;
+    return RAGFIN_OK;
+}
+
+extern "C" int ragfin_debug_sweep_copy(ragfin_t* h, int64_t row0, int64_t n, int8_t* out_rows_host, float* out_side_host, int32_t* ld8_out) {
+    if (!h || !ld8_out || row0 < 0 || n < 0 || (n > 0 && (!out_rows_host || !out_side_host))) return fail(RAGFIN_EINVAL, "bad argument");
+    std::lock_guard<std::mutex> lk(h->mu);
+    if (!h->i8) return fail(RAGFIN_EUNSUPPORTED, "this collection has no int8 copy (it is made by the first one-kernel search that uses it)");
+    if (row0 + n > h->i8_rows) return fail(RAGFIN_EINVAL, "rows [%lld, %lld) outside the %lld rows of the int8 copy", (long long)row0, (long long)(row0 + n), (long long)h->i8_rows);
+    *ld8_out = h->ld8;
+    if (n == 0) return RAGFIN_OK;
+    DeviceGuard g(h->device);
+    CU_TRY(cudaDeviceSynchronize());
+    CU_TRY(cudaMemcpy(out_rows_host, h->i8 + (size_t)row0 * h->ld8, (size_t)n * h->ld8, cudaMemcpyDeviceToHost));
+    CU_TRY(cudaMemcpy(out_side_host, h->i8side + row0, (size_t)n * sizeof(float2), cudaMemcpyDeviceToHost));
+    return RAGFIN_OK;
+}
+
+extern "C" int ragfin_debug_fused_tiles(ragfin_t* h, int64_t* out) {
+    if (!h || !out) return fail(RAGFIN_EINVAL, "NULL argument");
+    std::lock_guard<std::mutex> lk(h->mu);
+    out[0] = out[1] = 0;
+    if (!h->fctl.p) return RAGFIN_OK;
+    DeviceGuard g(h->device);
+    CU_TRY(cudaDeviceSynchronize());
+    FusedCtl c;
+    CU_TRY(cudaMemcpy(&c, (FusedCtl*)h->fctl.p + h->fused_last, sizeof(FusedCtl), cudaMemcpyDeviceToHost));
+    out[0] = c.last_refined;
+    out[1] = c.last_screened;
+    return RAGFIN_OK;
+}
+
 extern "C" int ragfin_set_pipelined(ragfin_t* h, int32_t enable) {
     if (!h) return fail(RAGFIN_EINVAL, "NULL handle");
     std::lock_guard<std::mutex> lk(h->mu);

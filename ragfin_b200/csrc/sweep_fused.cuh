@@ -36,6 +36,12 @@
 //              rank's gather area over NVLink (CUDA IPC mappings), publishes a per-(rank, query) flag with st.release.sys,
 //              waits for the W flags of its own area, merges the W x k hits by rank counting and writes the GLOBAL top-k - a
 //              sharded search is this one kernel per GPU, no collective call.
+//   int8 filter (I8 instantiations, 16-bit storage with the split query): every tile but the CTA's first is first swept
+//              from an int8 copy of the rows (kind::i8, exact s32 accumulators, half the bytes).  The epilogue bounds each
+//              row's 16-bit approximate score from above (u, DESIGN.md 2.5); a tile where no row and no query can reach
+//              thr is done, any other tile goes on the refine queue and the producer streams it again in 16 bits between
+//              the int8 tiles - the MMA issuer switches kind per tile and the refined tile takes the ordinary path below.
+//              A skipped tile would have appended nothing, so buffers, lists and bounds are those of a full 16-bit sweep.
 //   pipelining asynchronous entry points launch with programmatic stream serialization and the kernel releases its
 //              dependents when it starts: the next search's CTAs take over SMs as this one's finish, so back-to-back
 //              searches overlap one search's tail with the next one's sweep.  Consecutive searches alternate between two
@@ -51,6 +57,18 @@ constexpr int kFMaxK = 128;       // sorted per-CTA lists live in shared memory
 constexpr int kFGroups = 16;      // CTA groups of the shared bound (see "threshold" above)
 constexpr int kObsQ = 16;         // queries observed at a time in a CTA's first tile ...
 constexpr int kObsStride = kGN + 1;   // ... [kObsQ][256 (+1: bank spread)] ordered scores in the pending area
+constexpr int kFRefineQ = 32;     // refine queue entries: at most the tiles in flight (ring + 2 accumulators) are ever pending
+
+// What a ring stage / an accumulator holds: {kind, slice, tile ordinal t, permuted tile tp}
+enum { kTile16 = 0, kTileI8 = 1, kTileEnd = 2 };
+// int8 filter state (I8 instantiations only), after the pending area
+struct FusedI8State {
+    int4 rq[kFRefineQ];          // refine queue, written by epilogue thread 0, read by the producer
+    int rq_tail, decided;        // entries pushed; int8 tiles decided (pushed or not)
+    int pad[2];
+    float sq[kFMaxQ];            // query scale: q ~ sq * (hi + lo / 256)
+    float c1[kFMaxQ], c0[kFMaxQ];   // u = approx8 + c1 * e_r + c0 (see the prologue)
+};
 
 struct FusedCtl {
     uint32_t cnt[kFMaxQ];     // rows appended per query (may exceed cap: overflow)
@@ -68,6 +86,8 @@ struct FusedCtl {
     unsigned long long t[16];    // globaltimer stamps of the last search (ns): CTA 0: start, prologue done, first tile done,
                                  // sweep done; finalizer of query 0: all CTAs arrived, hits selected, rescored, emitted;
                                  // [8..]: finer stamps (setup done, norms done; count read, keys staged, T found)
+    uint32_t refined, screened;            // tiles swept in 16 bits / from the int8 copy by this search (summed by the CTAs) ...
+    uint32_t last_refined, last_screened;  // ... and by the last search (diagnostics)
 };
 __device__ __forceinline__ unsigned long long global_ns() {
     unsigned long long t;
@@ -120,6 +140,11 @@ struct FusedArgs {
     unsigned long long xrec_max;   // bytes of one rank's record in a gather area
     char* const* xpeer_area;    // [xworld] base of every rank's gather area: [kXSlots][xworld][xrec_max]
     uint32_t* const* xpeer_qflag;  // [xworld] base of every rank's per-query flags: [kXSlots][xworld][kFMaxQ]
+    // int8 filter (I8 instantiations): rows [n_rows][ld8] int8 through tmB8, per row {s, e}: x ~ s * x8, |x - s x8|_2 <= e
+    uint32_t idesc8;
+    int num_kblocks8;           // 128-element k-blocks of an int8 row
+    const float2* side8;
+    float i8_conv;              // fp32 evaluation allowance of the int8 score (see eps_i8_conv)
 };
 
 // pending area: [nq][pend] appended scores per tile in steady state, [kObsQ][kObsStride] observed scores in the first tile
@@ -163,6 +188,18 @@ __device__ __forceinline__ uint32_t ld_acq_gpu(const uint32_t* p) {
     return v;
 }
 __device__ __forceinline__ void fence_proxy_async_smem() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
+// D (s32) += A (s8) * B (s8): M = 128, N from idesc, K = 32
+__device__ __forceinline__ void tc_mma_i8(uint32_t tmem_d, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
+    asm volatile(
+        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
+        "tcgen05.mma.cta_group::1.kind::i8 [%0], %1, %2, %3, p;\n\t}" ::"r"(tmem_d), "l"(adesc), "l"(bdesc), "r"(idesc),
+        "r"(accumulate)
+        : "memory");
+}
+// instruction descriptor of kind::i8: D = s32, A and B signed 8-bit, both K-major, M = 128
+__host__ __device__ constexpr uint32_t make_idesc_i8(int n) {
+    return (2u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(n >> 3) << 17) | ((uint32_t)(128 >> 4) << 24);
+}
 
 // thr = value - 2 eps - 2^-22, every step rounded down (never above the real bound)
 __device__ __forceinline__ float thr_below(float value, float eps) {
@@ -215,9 +252,10 @@ __device__ __forceinline__ void canonical_dot_two_rows(const void* data, uint32_
     out_b = warp_butterfly_f64(acc_b);
 }
 
-template <int KIND, int NCOL, bool SPLIT>
+template <int KIND, int NCOL, bool SPLIT, bool I8>
 __global__ void __launch_bounds__(kFThreads, 1)
-sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, const __grid_constant__ FusedInlineQ qin) {
+sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, const __grid_constant__ FusedInlineQ qin,
+                   const __grid_constant__ CUtensorMap tmB8) {
     const float* const qsrc = a.q != nullptr ? a.q : qin.v;
     constexpr int P = NCOL <= 32 ? 4 : 2;                      // partial accumulators per half tile
     constexpr int kAcc = 2 * P * NCOL;                         // TMEM columns of one tile buffer
@@ -226,15 +264,18 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
     constexpr int QTILE = NCOL * kGKBytes;                     // bytes of one k-block of the query block
     static_assert(2 * kAcc <= 512, "accumulators exceed tensor memory");
     static_assert(!(SPLIT && KIND == 1), "the hi/lo split is for 16-bit storage");
+    static_assert(!I8 || SPLIT, "the int8 filter enters the query as hi / lo columns");
 
     extern __shared__ uint8_t fsm_raw[];
     const uint32_t raw = smem_u32(fsm_raw);
     const uint32_t base = (raw + 1023u) & ~1023u;
     uint8_t* fsm = fsm_raw + (base - raw);
     const int stages = a.stages, nkb = a.num_kblocks, nq = a.nq, k = a.k;
+    const int nkb8 = I8 ? a.num_kblocks8 : 0;
     const uint32_t smQ = base;                                             // [nkb][NCOL x 128 B]
     const uint32_t smB = base + (uint32_t)nkb * QTILE;                     // [stages][32 KB]
-    const size_t region_bytes = (size_t)nkb * QTILE + (size_t)stages * kBBytes;   // reused as scratch by the finalize
+    const uint32_t smQ8 = smB + (uint32_t)stages * kBBytes;                // I8: [nkb8][NCOL x 128 B], int8 query block
+    const size_t region_bytes = (size_t)(nkb + nkb8) * QTILE + (size_t)stages * kBBytes;   // reused as scratch by the finalize
     uint64_t* bars = reinterpret_cast<uint64_t*>(fsm + region_bytes);
     const uint32_t bar0 = smem_u32(bars);
     auto full_bar = [&](int s) { return bar0 + 8u * s; };
@@ -244,6 +285,9 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * kRMaxStages + 4);
     uint32_t* s_ticket = tmem_slot + 1;
     int* s_app = reinterpret_cast<int*>(tmem_slot + 2);    // diagnostics: rows this CTA appended for query 0
+    int4* stage_tag = reinterpret_cast<int4*>(fsm + region_bytes + 112);   // [kRMaxStages] what each ring stage holds ...
+    int4* acc_tag = stage_tag + kRMaxStages;                                // [2] ... and each accumulator
+    static_assert(112 + 16 * (kRMaxStages + 2) <= 256 && 8 * (2 * kRMaxStages + 4) + 12 <= 112, "barrier block layout");
     // per-query threshold state
     float* thr_s = reinterpret_cast<float*>(fsm + region_bytes + 256);     // [kFMaxQ]
     float* eps_s = thr_s + kFMaxQ;                                          // [kFMaxQ]
@@ -253,6 +297,7 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
     uint32_t* pubf_s = pub_s + kFMaxQ;                                      // [kFMaxQ] ... and its last published full bound
     uint32_t* sorted = pubf_s + kFMaxQ;                                     // [nq][k] descending ordered-uint scores
     uint32_t* pend = sorted + (size_t)nq * k;                               // [nq][pend]
+    FusedI8State* i8s = reinterpret_cast<FusedI8State*>((reinterpret_cast<uintptr_t>(pend + fused_pend_words(nq, a.pend)) + 15) & ~(uintptr_t)15);
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
     // Pipelined launches (programmatic stream serialization, see run_fused): the NEXT search's grid may be scheduled as soon as
@@ -272,7 +317,7 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
         for (int ln = tid; ln * 32 < a.nq * a.dim; ln += kFThreads) asm volatile("prefetch.global.L1 [%0];" ::"l"(a.q + (size_t)ln * 32));
     if (tid == 0) {
         for (int s = 0; s < stages; ++s) { mbar_init(full_bar(s), 1); mbar_init(empty_bar(s), 1); }
-        for (int s = 0; s < 2; ++s) { mbar_init(tfull_bar(s), 1); mbar_init(tempty_bar(s), 128); }
+        for (int s = 0; s < 2; ++s) { mbar_init(tfull_bar(s), 2); mbar_init(tempty_bar(s), 128); }   // tfull: tag + commit
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
     if (warp == 1) {
@@ -281,6 +326,10 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
     }
     for (int i = tid; i < kFMaxQ; i += kFThreads) { thr_s[i] = i < nq ? -INFINITY : INFINITY; eps_s[i] = 0.f; scnt[i] = 0; pcnt[i] = 0; pub_s[i] = 0u; pubf_s[i] = 0u; }
     if (tid == 0) *s_app = 0;
+    if (I8) {
+        for (int i = tid; i < kFMaxQ; i += kFThreads) { i8s->sq[i] = 0.f; i8s->c1[i] = 0.f; i8s->c0[i] = 0.f; }
+        if (tid == 0) { i8s->rq_tail = 0; i8s->decided = 0; }
+    }
     if (blockIdx.x == 0 && tid == 0) *a.flag_count = 0;   // ordered before every finalizer's atomicAdd by the arrival counter
     tc_fence_before();
     __syncthreads();
@@ -301,12 +350,16 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
         long long r0, r1;
         const int ntiles = slice_tiles(blockIdx.x, r0, r1);
         const int mult = perm_mult(ntiles);
-        for (int it = 0; it < stages && it < ntiles * nkb; ++it) {
-            const int t = it / nkb, kb = it % nkb;
+        // the same k-blocks, in the same order, as the producer's loop below (I8: the first tile in 16 bits, then int8 tiles)
+        for (int t = 0; t < ntiles && pre_issued < stages; ++t) {
+            const bool i8t = I8 && t > 0;
             const int tp = perm_tile(t, mult, ntiles);
-            mbar_expect_tx(full_bar(it), kBBytes);
-            tma_load_2d(smB + (uint32_t)it * kBBytes, &tmB, kb * a.k_elems, (int)(r0 + (long long)tp * kGN), full_bar(it));
-            ++pre_issued;
+            for (int kb = 0; kb < (i8t ? nkb8 : nkb) && pre_issued < stages; ++kb) {
+                const int it = pre_issued++;
+                stage_tag[it] = make_int4(i8t ? kTileI8 : kTile16, (int)blockIdx.x, t, tp);
+                mbar_expect_tx(full_bar(it), kBBytes);
+                tma_load_2d(smB + (uint32_t)it * kBBytes, i8t ? &tmB8 : &tmB, kb * (i8t ? kGKBytes : a.k_elems), (int)(r0 + (long long)tp * kGN), full_bar(it));
+            }
         }
     }
 
@@ -314,6 +367,10 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
     {
         uint4* qz = reinterpret_cast<uint4*>(fsm);
         for (int i = tid; i < nkb * QTILE / 16; i += kFThreads) qz[i] = make_uint4(0u, 0u, 0u, 0u);
+        if (I8) {
+            uint4* qz8 = reinterpret_cast<uint4*>(fsm + (smQ8 - base));
+            for (int i = tid; i < nkb8 * QTILE / 16; i += kFThreads) qz8[i] = make_uint4(0u, 0u, 0u, 0u);
+        }
         __syncthreads();
         const int esz = KIND == 1 ? 4 : 2;
         // pass 1, one warp per query: canonical sum of squares -> 1 / |q| (fp64), parked in the pending area
@@ -448,11 +505,53 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
                 }
             }
         }
+        if (I8) {
+            // int8 query, one warp per query: y ~ sq * (hi + lo / 256), sq = max |y| / 127, hi and lo in [-127, 127], in the
+            // hi / lo columns of the 16-bit block.  Any hi, lo would do: the bound uses the residual d = y - sq (hi + lo / 256),
+            // computed exactly in fp64 (every term is a multiple of 2^-33 sq or y itself, and spans < 53 bits), |d|_2 rounded up.
+            for (int j = warp; j < nq; j += kFThreads / 32) {
+                const float* x = qsrc + (size_t)j * a.dim;
+                const double inv = inv_s[j];
+                float mx = 0.f;
+                for (int i = lane; i < a.dim; i += kWarp) mx = fmaxf(mx, fabsf(norm_elem(x[i], inv)));
+#pragma unroll
+                for (int off = 16; off >= 1; off >>= 1) mx = fmaxf(mx, __shfl_xor_sync(kFull, mx, off));
+                const float sq = mx / 127.0f;
+                const float rsq = mx > 0.f ? 127.0f / mx : 0.f;
+                const int row_hi = (j >> 3) * 16 + (j & 7);
+                double d2 = 0.0;
+                for (int i = lane; i < a.dim; i += kWarp) {
+                    const float y = norm_elem(x[i], inv);
+                    const float hi = fminf(fmaxf(rintf(y * rsq), -127.f), 127.f);
+                    const float lo = fminf(fmaxf(rintf((y - sq * hi) * rsq * 256.f), -127.f), 127.f);
+                    const double d = ((double)y - (double)sq * (double)hi) - (double)sq * (double)lo * 0.00390625;
+                    d2 = __dadd_ru(d2, __dmul_ru(d, d));
+                    const int kb = i >> 7, c = i & 127;
+                    int8_t* p_hi = reinterpret_cast<int8_t*>(fsm + (smQ8 - base)) + (size_t)kb * QTILE + (size_t)(row_hi >> 3) * 1024 + (size_t)(row_hi & 7) * 128 +
+                                   ((((c >> 4) ^ (row_hi & 7)) << 4) | (c & 15));
+                    p_hi[0] = (int8_t)hi;
+                    p_hi[1024] = (int8_t)lo;      // lo row: 8 MMA columns further
+                }
+#pragma unroll
+                for (int off = 16; off >= 1; off >>= 1) d2 = __dadd_ru(d2, __shfl_xor_sync(kFull, d2, off));
+                if (lane == 0) { i8s->sq[j] = sq; i8s->c1[j] = __double2float_ru(__dsqrt_ru(d2)); }   // c1 holds |d|_2 for now
+            }
+        }
         __syncthreads();
         // |approx - exact| <= |q - hi - lo|_2 * max |stored row|_2 + the accumulation allowance.  The residual is bounded a
         // priori, element by element, on the host (eps_fused_query: half an ulp of each rounding, 2^-8 |q| for bf16 hi alone,
         // 2^-17 |q| for hi + lo; fp16 2^-11 and 2^-23, plus half the subnormal spacing).
-        for (int j = tid; j < nq; j += kFThreads) eps_s[j] = __fadd_ru(a.eps_const, a.eps_query);
+        for (int j = tid; j < nq; j += kFThreads) {
+            eps_s[j] = __fadd_ru(a.eps_const, a.eps_query);
+            if (I8) {
+                // q.x = s sq (H + L / 256) + s d.x8 + q.(x - s x8), so |q.x - approx8| <= |d|_2 (|x|_2 + e) + |q|_2 e with
+                // |x|_2 <= 1 + 2^-7, |q|_2 <= 1 + 2^-20: c1 = |q|_2 + |d|_2, c0 = (1 + 2^-7) |d|_2 + fp32 allowance + eps16,
+                // so that u = approx8 + c1 e + c0 >= approx16 (DESIGN.md 2.5)
+                const float dq = i8s->c1[j];
+                i8s->c1[j] = __fadd_ru(1.00000095367431640625f, dq);
+                i8s->c0[j] = __fadd_ru(__fadd_ru(__fmul_ru(1.0078125f, dq), a.i8_conv), eps_s[j]);
+            }
+        }
         __syncthreads();
         for (int i = tid; i < 2 * kFMaxQ + 2; i += kFThreads) pend[i] = 0u;   // the parking area goes back to the pending lists
         fence_proxy_async_smem();   // generic-proxy writes above -> visible to the tensor core's async-proxy reads
@@ -464,54 +563,95 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
         if (lane == 0) {   // ===== TMA producer =====
             int stage = 0, skip = pre_issued;
             uint32_t phase = 0;
+            // one tile's k-blocks into the ring, each stage tagged with what it holds
+            auto put_tile = [&](int kind, int sl, int t, int tp) {
+                const long long row = (long long)sl * a.rows_per_slice + (long long)tp * kGN;
+                const int nk = kind == kTileI8 ? nkb8 : nkb;
+                for (int kb = 0; kb < nk; ++kb) {
+                    if (skip > 0) {
+                        --skip;                        // issued before the prologue (first round of the ring: slots were free)
+                    } else {
+                        mbar_wait(empty_bar(stage), phase ^ 1u);
+                        stage_tag[stage] = make_int4(kind, sl, t, tp);
+                        mbar_expect_tx(full_bar(stage), kBBytes);
+                        if (I8 && kind == kTileI8) tma_load_2d(smB + (uint32_t)stage * kBBytes, &tmB8, kb * kGKBytes, (int)row, full_bar(stage));
+                        else tma_load_2d(smB + (uint32_t)stage * kBBytes, &tmB, kb * a.k_elems, (int)row, full_bar(stage));
+                    }
+                    if (++stage == stages) { stage = 0; phase ^= 1u; }
+                }
+            };
+            // I8: tiles the epilogue found within reach go back into the ring in 16 bits, between the int8 tiles (never
+            // inside the pre-issued k-blocks, whose order is fixed)
+            int head = 0, n_i8 = 0;
+            auto refine_pending = [&]() {
+                while (skip == 0 && head < *reinterpret_cast<volatile int*>(&i8s->rq_tail)) {
+                    const volatile int4* e = i8s->rq + head % kFRefineQ;   // published before rq_tail
+                    const int esl = e->x, et_ = e->y, etp = e->z;
+                    ++head;
+                    put_tile(kTile16, esl, et_, etp);
+                }
+            };
             for (int sl = blockIdx.x; sl < a.S; sl += gridDim.x) {
                 long long r0, r1;
                 const int ntiles = slice_tiles(sl, r0, r1);
                 const int mult = perm_mult(ntiles);
                 for (int t = 0; t < ntiles; ++t) {
-                    const int tp = perm_tile(t, mult, ntiles);
-                    for (int kb = 0; kb < nkb; ++kb) {
-                        if (skip > 0) {
-                            --skip;                        // issued before the prologue (first round of the ring: slots were free)
-                        } else {
-                            mbar_wait(empty_bar(stage), phase ^ 1u);
-                            mbar_expect_tx(full_bar(stage), kBBytes);
-                            tma_load_2d(smB + (uint32_t)stage * kBBytes, &tmB, kb * a.k_elems, (int)(r0 + (long long)tp * kGN), full_bar(stage));
-                        }
-                        if (++stage == stages) { stage = 0; phase ^= 1u; }
-                    }
+                    const bool i8t = I8 && (sl != (int)blockIdx.x || t > 0);   // the CTA's first tile is observed in 16 bits
+                    put_tile(i8t ? kTileI8 : kTile16, sl, t, perm_tile(t, mult, ntiles));
+                    if (I8) { n_i8 += i8t; refine_pending(); }
                 }
             }
+            if (I8) {   // every int8 tile decided and every refine issued
+                for (;;) {
+                    const int d = *reinterpret_cast<volatile int*>(&i8s->decided);
+                    __threadfence_block();
+                    refine_pending();
+                    if (d == n_i8 && head == *reinterpret_cast<volatile int*>(&i8s->rq_tail)) break;
+                    __nanosleep(64);
+                }
+            }
+            mbar_wait(empty_bar(stage), phase ^ 1u);    // end of the sweep: a tagged stage without bytes
+            stage_tag[stage] = make_int4(kTileEnd, 0, 0, 0);
+            mbar_arrive(full_bar(stage));
         }
     } else if (warp == 1) {
-        if (lane == 0) {   // ===== MMA issuer =====
+        if (lane == 0) {   // ===== MMA issuer: follows the tags of the ring =====
             int stage = 0, acc = 0;
             uint32_t phase = 0, acc_phase = 0;
-            for (int sl = blockIdx.x; sl < a.S; sl += gridDim.x) {
-                long long r0, r1;
-                const int ntiles = slice_tiles(sl, r0, r1);
-                for (int t = 0; t < ntiles; ++t) {
-                    mbar_wait(tempty_bar(acc), acc_phase ^ 1u);
-                    tc_fence_after();
-                    for (int kb = 0; kb < nkb; ++kb) {
-                        mbar_wait(full_bar(stage), phase);
-                        tc_fence_after();
-                        const uint64_t qd = make_smem_desc(smQ + (uint32_t)kb * QTILE);
-#pragma unroll
-                        for (int k4 = 0; k4 < kGKBytes / 32; ++k4) {
-#pragma unroll
-                            for (int h = 0; h < 2; ++h) {
-                                const uint64_t cd = make_smem_desc(smB + (uint32_t)stage * kBBytes + (uint32_t)h * (kBBytes / 2));
-                                const uint32_t d_tmem = tmem_base + (uint32_t)acc * kAcc + (uint32_t)h * (P * NCOL) + (uint32_t)(k4 % P) * NCOL;
-                                tc_mma<KIND>(d_tmem, cd + 2u * k4, qd + 2u * k4, a.idesc, (uint32_t)(kb != 0 || k4 >= P));
-                            }
-                        }
-                        tc_commit(empty_bar(stage));
-                        if (++stage == stages) { stage = 0; phase ^= 1u; }
-                    }
-                    tc_commit(tfull_bar(acc));
-                    if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
+            for (;;) {
+                mbar_wait(tempty_bar(acc), acc_phase ^ 1u);
+                tc_fence_after();
+                mbar_wait(full_bar(stage), phase);
+                const int4 tg = stage_tag[stage];
+                if (tg.x == kTileEnd) {
+                    acc_tag[acc] = tg;
+                    mbar_arrive(tfull_bar(acc));
+                    mbar_arrive(tfull_bar(acc));
+                    break;
                 }
+                const bool i8t = I8 && tg.x == kTileI8;   // K = 32 bytes per MMA either way: the k4 loop is the same
+                const int nk = i8t ? nkb8 : nkb;
+                for (int kb = 0; kb < nk; ++kb) {
+                    if (kb > 0) mbar_wait(full_bar(stage), phase);
+                    tc_fence_after();
+                    const uint64_t qd = make_smem_desc((i8t ? smQ8 : smQ) + (uint32_t)kb * QTILE);
+#pragma unroll
+                    for (int k4 = 0; k4 < kGKBytes / 32; ++k4) {
+#pragma unroll
+                        for (int h = 0; h < 2; ++h) {
+                            const uint64_t cd = make_smem_desc(smB + (uint32_t)stage * kBBytes + (uint32_t)h * (kBBytes / 2));
+                            const uint32_t d_tmem = tmem_base + (uint32_t)acc * kAcc + (uint32_t)h * (P * NCOL) + (uint32_t)(k4 % P) * NCOL;
+                            if (i8t) tc_mma_i8(d_tmem, cd + 2u * k4, qd + 2u * k4, a.idesc8, (uint32_t)(kb != 0 || k4 >= P));
+                            else tc_mma<KIND>(d_tmem, cd + 2u * k4, qd + 2u * k4, a.idesc, (uint32_t)(kb != 0 || k4 >= P));
+                        }
+                    }
+                    tc_commit(empty_bar(stage));
+                    if (++stage == stages) { stage = 0; phase ^= 1u; }
+                }
+                acc_tag[acc] = tg;
+                mbar_arrive(tfull_bar(acc));     // releases the tag ...
+                tc_commit(tfull_bar(acc));       // ... and the accumulator
+                if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
             }
         }
     } else {   // ===== epilogue: thread <-> TMEM lane <-> corpus row of a half tile =====
@@ -670,23 +810,74 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
             }
             __syncwarp();
         };
-        for (int sl = blockIdx.x; sl < a.S; sl += gridDim.x) {
-            long long r0, r1;
-            const int ntiles = slice_tiles(sl, r0, r1);
-            const int mult = perm_mult(ntiles);
-            for (int t = 0; t < ntiles; ++t) {
-                const int tp = perm_tile(t, mult, ntiles);
-                const long long trow = r0 + (long long)tp * kGN;
+        uint32_t n_tiles16 = 0, n_tiles8 = 0;      // diagnostics (thread et = 0)
+        for (;;) {
+            {
                 const bool stamp_tile = blockIdx.x == 0 && et == 0;
                 unsigned long long ts0 = 0, ts1 = 0, ts2 = 0;
                 if (stamp_tile) ts0 = global_ns();
                 mbar_wait(tfull_bar(acc), acc_phase);
                 tc_fence_after();
+                const int4 tg = acc_tag[acc];
+                if (tg.x == kTileEnd) break;
+                const int sl = tg.y, t = tg.z, tp = tg.w;
+                long long r0, r1;
+                (void)slice_tiles(sl, r0, r1);
+                const long long trow = r0 + (long long)tp * kGN;
                 if (stamp_tile) ts1 = global_ns();
                 // rows past the slice / corpus (zero-filled by TMA) and filtered rows never qualify
                 const long long row_h0 = trow + m, row_h1 = trow + 128 + m;
                 const bool ok0 = row_h0 < r1 && (a.allow == nullptr || row_allowed(a.allow, row_h0));
                 const bool ok1 = row_h1 < r1 && (a.allow == nullptr || row_allowed(a.allow, row_h1));
+                if (I8 && tg.x == kTileI8) {
+                    // ---- int8 screen: u >= approx16 for every row and query (prologue); the tile is refined when some
+                    // u reaches the query's threshold, else nothing of it could have been appended ----
+                    const float2 sd0 = ok0 ? __ldg(a.side8 + row_h0) : make_float2(0.f, 0.f);
+                    const float2 sd1 = ok1 ? __ldg(a.side8 + row_h1) : make_float2(0.f, 0.f);
+                    bool need = false;
+#pragma unroll 1
+                    for (int c = 0; c < NCOL / 16; ++c) {
+#pragma unroll 1
+                        for (int h = 0; h < 2; ++h) {
+                            uint32_t v[P][16];
+                            chunk_load(h, c, v);
+                            tmem_ld_wait();
+                            chunk_fence(v);
+                            const float2 sd = h ? sd1 : sd0;
+                            const bool okh = h ? ok1 : ok0;
+#pragma unroll
+                            for (int j = 0; j < QPC; ++j) {
+                                const int qi = c * QPC + j;
+                                int hi = 0, lo = 0;
+#pragma unroll
+                                for (int p = 0; p < P; ++p) { hi += (int)v[p][j]; lo += (int)v[p][j + 8]; }
+                                const float w = __fmul_rn(__fmul_rn(sd.x, i8s->sq[qi]), __fadd_rn(__int2float_rn(hi), __int2float_rn(lo) * 0.00390625f));
+                                const float u = __fadd_ru(w, __fmaf_ru(i8s->c1[qi], sd.y, i8s->c0[qi]));
+                                need |= okh && u >= thr_s[qi];     // padding queries: thr = +inf
+                            }
+                        }
+                    }
+                    tc_fence_before();
+                    mbar_arrive(tempty_bar(acc));
+                    if (++acc == 2) { acc = 0; acc_phase ^= 1u; }
+                    const bool any = named_bar_or(1, 128, need);
+                    if (et == 0) {
+                        volatile int* tail = &i8s->rq_tail;
+                        if (any) {
+                            i8s->rq[*tail % kFRefineQ] = make_int4(sl, t, tp, 0);
+                            __threadfence_block();
+                            *tail = *tail + 1;
+                        }
+                        __threadfence_block();
+                        *reinterpret_cast<volatile int*>(&i8s->decided) = ++n_tiles8;
+                    }
+                    if (t < 8 || t % a.refresh_every == 0) {   // the grid's bounds tighten the screen as they do the appends
+                        warp_refresh();
+                        named_bar_sync(2, 128);
+                    }
+                    continue;
+                }
+                ++n_tiles16;
                 if (warm) {
                     // ---- the CTA's first tile, pass 1 of 2: OBSERVE.  With thr = -inf every CTA would append its whole first
                     // tile (148 x 256 rows per query, all on one counter).  Instead the tile's scores go to shared memory in
@@ -854,6 +1045,7 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
                 warm = false;
             }
         }
+        if (et == 0) { atomicAdd(&a.ctl->refined, n_tiles16); atomicAdd(&a.ctl->screened, n_tiles8); }
         __threadfence();   // this thread's appended keys are visible device-wide before the CTA is counted as done
         if (blockIdx.x == 0 && et == 0) a.ctl->t[3] = global_ns();
         if (et == 0 && blockIdx.x < 160) { a.ctl->cta_thr[blockIdx.x] = thr_s[0]; a.ctl->cta_app[blockIdx.x] = (uint32_t)*s_app; }
@@ -1164,6 +1356,8 @@ sweep_fused_kernel(const __grid_constant__ CUtensorMap tmB, const FusedArgs a, c
             a.ctl->done = 0u;
             a.ctl->obs_done = 0u;
             a.ctl->fin_done = 0u;
+            a.ctl->last_refined = a.ctl->refined; a.ctl->refined = 0u;
+            a.ctl->last_screened = a.ctl->screened; a.ctl->screened = 0u;
             __threadfence();
             a.ctl->n_done = a.seq_on_half + 1u;      // this half is free for the search after the next
             if (a.host_flag != nullptr) { __threadfence_system(); *reinterpret_cast<volatile uint32_t*>(a.host_flag) = a.host_seq; }

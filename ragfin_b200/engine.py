@@ -388,6 +388,27 @@ class Index:
         issued - do not enable it when a kernel enqueued between two searches produces the queries.  Default off."""
         _lib.check(self._L.ragfin_set_pipelined(self._h, 1 if enable else 0))
 
+    def set_sweep_copy(self, mode) -> None:
+        """The one-kernel search's int8 tile filter (bf16 / fp16): True = on, False = off, "auto" (default) = on from 2^20
+        rows.  Results are identical; the int8 copy of the rows is made by the first search that uses it."""
+        m = -1 if mode == "auto" else (1 if mode else 0)
+        _lib.check(self._L.ragfin_set_sweep_copy(self._h, m))
+
+    def sweep_copy_rows(self, row0: int, n: int):
+        """Rows [row0, row0 + n) of the int8 copy: (int8 [n, ld8], float32 [n, 2] = per-row scale and residual bound)."""
+        ld8 = ctypes.c_int32(0)
+        _lib.check(self._L.ragfin_debug_sweep_copy(self._h, int(row0), 0, None, None, ctypes.byref(ld8)))
+        rows = np.zeros((n, ld8.value), np.int8)
+        side = np.zeros((n, 2), np.float32)
+        _lib.check(self._L.ragfin_debug_sweep_copy(self._h, int(row0), int(n), rows.ctypes.data, side.ctypes.data, ctypes.byref(ld8)))
+        return rows, side
+
+    def fused_tiles(self):
+        """Tiles of the last one-kernel search: (read in 16 bits, screened from the int8 copy)."""
+        out = np.zeros(2, np.int64)
+        _lib.check(self._L.ragfin_debug_fused_tiles(self._h, out.ctypes.data))
+        return int(out[0]), int(out[1])
+
     def fused_eligible(self, nq: int, k: int) -> bool:
         """Whether (nq, k) takes the one-kernel search on this handle (csrc/sweep_fused.cuh)."""
         out = ctypes.c_int32()
